@@ -18,6 +18,8 @@ per matrix (SURVEY 8d), value = total flops / device time.
             built from /root/reference with the README's -O3 -mavx) on the host cores, bounded sample.
 
 `--impl reference` times the reference's CPU implementation alone (rank 0 only) on the same metric.
+`--dump-outputs DIR` writes what the last timed step computed as DIR/*.npy (rank 0; see dump_outputs): the inputs are
+seeded, so two builds of the project run with the same arguments can be compared output for output.
 Multi-GPU (torchrun, one rank per GPU): the matrices of the sweep are independent, so each rank
 reduces its own replica of the sweep (weak scaling, no data-path collective).
 """
@@ -161,6 +163,39 @@ def run_reference_arm(args, rank):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line), flush=True)
+
+
+# ------------------------------------------------------------------------------ output dump
+DUMP_BYTES = 48_000_000   # array data of one dump; with the .npy headers the whole dump stays under 64 MB
+
+
+def dump_share(sizes):
+    """Bytes of the whole-matrix sample of each matrix; fails before any GPU work when d, e and the bands alone overflow."""
+    fixed = sum((2 * n - 1 + (BAND + 1) * n) * sum(np.dtype(dt).itemsize for _, dt in DTYPES) for n in sizes)
+    if fixed > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: d, e and the band of {len(sizes) * len(DTYPES)} matrices take {fixed} bytes, "
+                         f"over the {DUMP_BYTES}-byte budget")
+    return (DUMP_BYTES - fixed) // (len(sizes) * len(DTYPES))
+
+
+def dump_outputs(out_dir, torch, cur, dmany, emany, share):
+    """What svdb200_bidiagonalize_many_dev_* handed back in one step, for every matrix of the sweep: d (n), e (n - 1), the
+    diagonals 0..BAND of the overwritten matrix in full (row k = diagonal k, zero-padded to n: the band stage 1 leaves and
+    stage 2 reduces, where builds can differ) and a sample of the whole overwritten matrix, the entries at flat indices drawn
+    without replacement from a generator seeded with n and sorted, as many as DUMP_BYTES leaves after the rest, shared
+    equally over the matrices (dump_share).  Files: DIR/<f64|f32>_n<n>_<d|e|band|a>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    torch.cuda.synchronize()
+    pos = {}
+    for n, suf, a in cur:
+        i = pos[suf] = pos.get(suf, -1) + 1
+        band = torch.zeros(BAND + 1, n, dtype=a.dtype, device=a.device)
+        for k in range(min(BAND, n - 1) + 1):
+            band[k, : n - k] = torch.diagonal(a, k)
+        idx = np.sort(np.random.default_rng(n).choice(n * n, min(n * n, share // a.element_size()), replace=False))
+        sample = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        for name, x in (("d", dmany[suf][i]), ("e", emany[suf][i][: n - 1]), ("band", band), ("a", sample)):
+            np.save(os.path.join(out_dir, f"{suf}_n{n}_{name}.npy"), x.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------ GPU arm
@@ -449,7 +484,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dist-n", type=int, default=65536)  # size of the block-cyclic stage-1 measurement (BASELINE configs[3])
     ap.add_argument("--no-big", action="store_true")      # skip the n=16384 trailing-update measurement
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed (d, e, the band and a seeded sample of each bidiagonalised matrix) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -459,6 +498,7 @@ def main():
     if args.warmup < 3:
         args.warmup = 3
     sizes = [int(s) for s in args.sizes.split(",")] if args.sizes else SIZES
+    dump_sample_bytes = dump_share(sizes) if args.dump_outputs else 0
 
     import torch
     import torch.distributed as dist
@@ -542,6 +582,9 @@ def main():
     sampler.stop_flag = True
     ms = ev0.elapsed_time(ev1)
     launches = sum(h.launch_count() for h in handles.values()) - launches0
+    if args.dump_outputs and rank == 0:
+        # before the breakdown pass below refills sets[0], which may be the set of the last step
+        dump_outputs(args.dump_outputs, torch, sets[idx], dmany, emany, dump_sample_bytes)
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

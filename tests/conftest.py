@@ -125,7 +125,7 @@ def refso():
     """The compiled UNMODIFIED reference (oracle/_ref/libsvdref.so), if it has been built."""
     p = os.path.join(ROOT, "oracle", "_ref", "libsvdref.so")
     if not os.path.exists(p):
-        pytest.skip("oracle/_ref/libsvdref.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libsvdref.so not built (make -C oracle REF=<reference source tree>)")
     return ctypes.CDLL(p)
 
 

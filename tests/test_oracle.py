@@ -149,14 +149,25 @@ def test_band_structure_and_norm_preservation(oracle):
     assert np.abs(s0 - s1).max() < 1e-12 * s0[0]
 
 
-def test_compiled_reference_agrees_when_present(oracle, refso):
+def test_compiled_reference_agrees_when_present(oracle, request):
+    """The oracle == the compiled original reference, bit for bit: parallel::brd_p1<double>(A, 8), then parallel::brd_p2.
+    Compared with the reference's stored outputs for this input (golden_refcheck.npz, tools/make_golden.py --only-refcheck)
+    when they are in the tree, otherwise with the compiled reference itself (refso, which skips without it)."""
     import ctypes
     a = uniform_matrix(80, 80, 11, 0.0, 5.0, np.float64)
-    r = a.copy()
-    refso.svdref_brd_p1_f64(r.ctypes.data_as(ctypes.c_void_p), ctypes.c_size_t(80), ctypes.c_size_t(8))
-    assert np.array_equal(oracle.brd_p1(a, 8), r)
-    refso.svdref_brd_p2_f64(r.ctypes.data_as(ctypes.c_void_p), ctypes.c_size_t(80), ctypes.c_size_t(8), None, None)
-    assert np.array_equal(oracle.brd_p2(oracle.brd_p1(a, 8), 8)[0], r)
+    stored = os.path.join(GOLDEN, "golden_refcheck.npz")
+    if os.path.exists(stored):
+        g = np.load(stored)
+        ref_band, ref_bid = g["band_80_8_f64"], g["bidiag_80_8_f64"]
+    else:
+        refso = request.getfixturevalue("refso")
+        r = a.copy()
+        refso.svdref_brd_p1_f64(r.ctypes.data_as(ctypes.c_void_p), ctypes.c_size_t(80), ctypes.c_size_t(8))
+        ref_band = r.copy()
+        refso.svdref_brd_p2_f64(r.ctypes.data_as(ctypes.c_void_p), ctypes.c_size_t(80), ctypes.c_size_t(8), None, None)
+        ref_bid = r
+    assert np.array_equal(oracle.brd_p1(a, 8), ref_band)
+    assert np.array_equal(oracle.brd_p2(oracle.brd_p1(a, 8), 8)[0], ref_bid)
 
 
 @pytest.mark.parametrize("n,b", [(64, 4), (65, 4), (100, 7), (96, 32), (130, 16), (33, 32)])

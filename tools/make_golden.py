@@ -49,12 +49,24 @@ def onestage():
     np.savez_compressed(os.path.join(OUT, "golden_onestage.npz"), **z)
 
 
+def refcheck():
+    """parallel::brd_p1<double>(A, 8) and then parallel::brd_p2 on the seed-11 80x80 input of
+    tests/test_oracle.py::test_compiled_reference_agrees_when_present: both full output matrices."""
+    a = uniform_matrix(80, 80, 11, 0.0, 5.0, np.float64)
+    band_m, bid_m, _, _ = ref_chain(a, 8, "f64")
+    np.savez_compressed(os.path.join(OUT, "golden_refcheck.npz"), band_80_8_f64=band_m, bidiag_80_8_f64=bid_m)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     if "--only-onestage" in sys.argv:
         onestage()
         return
+    if "--only-refcheck" in sys.argv:
+        refcheck()
+        return
     onestage()
+    refcheck()
     for n in (64, 512):
         for name in ("float", "double"):
             for kind in ("test", "band", "bidiagonal"):
