@@ -126,7 +126,8 @@ int svdb200_bidiagonalize_many_dev_f64(svdb200_handle h, size_t count, double* c
 /* How svdb200_bidiagonalize_many_* schedules a list on `lanes` chains (pure host function, no handle, no device): the matrices
  * are partitioned over the chains longest-processing-time-first (a chain is bound by its stage-2 kernel, whose time is
  * proportional to n), run in ascending size inside a chain and are issued alternating between the chains.  order_out[j] =
- * index of the j-th matrix issued, chain_out[j] = its chain.  The results of the list calls do not depend on the schedule. */
+ * index of the j-th matrix issued, chain_out[j] = its chain.  lanes: 1..4; the list calls use 2.  The results of the list
+ * calls do not depend on the schedule. */
 int svdb200_list_plan(int lanes, size_t count, const size_t* n, size_t* order_out, int* chain_out);
 
 /* ---- Fused chain: singular values of a dense matrix (SURVEY 3.5) ------------------------------

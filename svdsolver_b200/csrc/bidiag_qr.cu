@@ -166,8 +166,8 @@ int bidiag_qr(Ctx* c, T* d, T* e, size_t n, T* sigma) {
     ProfScope ps(c, 5, (double)n);
     // zero-shift QR needs ~n log(1/tol) sweeps: beyond a moderate n the independent-per-value bisection
     // solver (bidiag_bisect.cu) takes over
-    if (c->qr_method == 2 || (c->qr_method == 0 && n > c->qr_auto_limit)) return bidiag_bisect<T>(c, d, e, n, sigma);
-    if (c->qr_method == 3) return bidiag_sqr<T>(c, d, e, n, sigma);          // implicit shifted QR (bidiag_sqr.cu)
+    if (c->cfg.qr_method == 2 || (c->cfg.qr_method == 0 && n > c->cfg.qr_auto_limit)) return bidiag_bisect<T>(c, d, e, n, sigma);
+    if (c->cfg.qr_method == 3) return bidiag_sqr<T>(c, d, e, n, sigma);      // implicit shifted QR (bidiag_sqr.cu)
     int npad = 1;
     while ((size_t)npad < n) npad <<= 1;
     // sort buffer: reuse the stage-2 progress array region is int-sized; use wpart (>= 2*max_n elems)

@@ -1,7 +1,6 @@
 // C ABI of libsvdb200.so (declared in include/svdb200.h).  Thin: argument checks, workspace
 // ownership, host<->device staging and CUDA-event timing; all arithmetic lives in the kernels.
 #include <algorithm>
-#include <cstdlib>
 #include <new>
 #include "common.cuh"
 
@@ -184,19 +183,9 @@ int probe_peak(Ctx* c, int kind, double* tflops) {
 // Shards by matrix across GPUs at the caller's level (one handle per GPU), no collective.
 constexpr int kBatchPool = 16;
 
-// Sub-handles (batch pool, stage-1 chains of the pipelined driver) follow the parent's run-time switches on every call,
+// Sub-handles (batch pool, stage-1 chains of the pipelined driver) follow the parent's settings on every call,
 // not only those set after the sub-handle was created.
-static void inherit_settings(const Ctx* c, Ctx* s) {
-    s->stage2_complete = c->stage2_complete; s->stage2_const_band = c->stage2_const_band; s->stage2_fast = c->stage2_fast;
-    s->qr_method = c->qr_method; s->qr_auto_limit = c->qr_auto_limit;
-    s->use_tc05 = c->use_tc05; s->tc05_min_elems = c->tc05_min_elems;
-    s->lookahead = c->lookahead; s->panel_reg = c->panel_reg; s->panel_reg_min = c->panel_reg_min;
-    s->panel_blk = c->panel_blk;
-    s->panel_chol = c->panel_chol;
-    s->pipe_chol = c->pipe_chol;
-    s->lookahead_reserve = c->lookahead_reserve;
-    s->chol_guard = c->chol_guard;
-}
+static void inherit_settings(const Ctx* c, Ctx* s) { s->cfg = c->cfg; }
 
 // Small matrices (n <= 1024, band <= 64): every kernel of the path runs ONCE PER STEP FOR THE WHOLE BATCH -- a
 // thread-block cluster per matrix for the panels (panel resident in cluster shared memory), one grid slice per
@@ -257,7 +246,7 @@ int batched_small(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma, i
             SVDB_CHECK(c, cudaMemcpyAsync(dall, d_out + z0 * n, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
             SVDB_CHECK(c, cudaMemcpyAsync(eall, e_out + z0 * n, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
         }
-        if (c->qr_method == 1) {                          // the reference's zero-shift QR sweeps, one CTA per matrix
+        if (c->cfg.qr_method == 1) {                      // the reference's zero-shift QR sweeps, one CTA per matrix
             for (int i = 0; i < cnt; ++i) SVDB_TRY(bidiag_qr<T>(c, dall + (size_t)i * n, eall + (size_t)i * n, n, sigma + (z0 + i) * n));
         } else {
             for (int i0 = 0; i0 < cnt; i0 += 32768) {
@@ -371,23 +360,19 @@ static int ensure_s2(Ctx* c) {
 // chains usable for this matrix: their sweep pipelines must be co-resident beside each other
 static int lanes_for(Ctx* c, size_t n, size_t band) {
     const size_t ctas = n / band / 2 + 2;                             // CTAs of one sweep pipeline, all of which must be resident
-    const size_t budget = (size_t)c->num_sms * 5 / 2;                 // 3 light stage-2 CTAs fit an SM; leave room for stage 1
-    const size_t cap = c->pipe_light ? budget : (size_t)c->num_sms - 8;        // the 153-register variant: one CTA per SM
-    return ((size_t)c->lanes * ctas <= cap) ? c->lanes : 1;
+    const size_t cap = (size_t)c->num_sms - 8;                        // the 153-register stage-2 variant: one CTA per SM
+    return ((size_t)Ctx::kLanes * ctas <= cap) ? Ctx::kLanes : 1;
 }
 
 template <typename T>
 static int run_stage2_on_lane(Ctx* c, int lane, T* a, size_t n, size_t band, T* d, T* e) {
     cudaStream_t s0 = c->stream;
     int* p0 = c->prog;
-    const int light0 = c->stage2_light;
     c->stream = c->s2_stream[lane];
     c->prog = c->s2_prog[lane];
-    c->stage2_light = c->pipe_light ? 1 : light0;
     const int st = stage2_chase<T>(c, a, n, band, d, e);
     c->stream = s0;
     c->prog = p0;
-    c->stage2_light = light0;
     return st;
 }
 
@@ -402,12 +387,12 @@ static int drain_into(Ctx* c, cudaStream_t into) {
     return 0;
 }
 
-// One matrix through the pipeline.  Chain k (chosen by plan_list): stage 1 on sub-handle k's streams, stage 2 on lane k -- so `lanes`
-// stage-1 factorizations and `lanes` sweep pipelines are in flight (default 2; 4 measured slower: contention); within a chain stage 1 of the next matrix starts as soon
+// One matrix through the pipeline.  Chain k (chosen by plan_list): stage 1 on sub-handle k's streams, stage 2 on lane k -- so kLanes
+// stage-1 factorizations and kLanes sweep pipelines are in flight; within a chain stage 1 of the next matrix starts as soon
 // as the previous stage 1 is done, beside that matrix's stage 2.  `h2d` (host variant): copy issued on the chain's stream.
 template <typename T>
 static int pipeline_one(Ctx* c, size_t i, T* a_dev, const T* a_host, size_t n, size_t band, int order, T* d, T* e, cudaStream_t* lane_out,
-                        int chain) {
+                        int k) {
     const bool overlap = order == SVDB200_ORDER_PANEL && n <= kOverlapMaxN && !c->profile;
     const int nl = overlap ? lanes_for(c, n, band) : 1;
     if (!overlap || nl == 1) {
@@ -426,7 +411,6 @@ static int pipeline_one(Ctx* c, size_t i, T* a_dev, const T* a_host, size_t n, s
         *lane_out = c->stream;
         return 0;
     }
-    const int k = chain % c->lanes;
     Ctx* s = c->s1ctx[k];
     inherit_settings(c, s);
     if (a_host) SVDB_CHECK(c, cudaMemcpyAsync(a_dev, a_host, sizeof(T) * n * n, cudaMemcpyHostToDevice, s->stream));
@@ -487,7 +471,7 @@ int bidiagonalize_many_dev(Ctx* c, size_t count, T* const* a, const size_t* n, s
         SVDB_CHECK(c, cudaStreamWaitEvent(c->s2_stream[l], c->s2ev[0], 0));
         SVDB_CHECK(c, cudaStreamWaitEvent(c->s1ctx[l]->stream, c->s2ev[0], 0));
     }
-    const ListPlan pl = plan_list(c->lanes, count, n);
+    const ListPlan pl = plan_list(Ctx::kLanes, count, n);
     for (size_t j = 0; j < count; ++j) {
         const size_t i = pl.order[j];
         cudaStream_t lane;
@@ -517,13 +501,12 @@ template <typename T>
 int bidiagonalize_many_host(Ctx* c, size_t count, T* const* a, const size_t* n, size_t band, int order, T* const* d, T* const* e) {
     if (count == 0) return 0;
     SVDB_TRY(ensure_s2(c));
-    constexpr int NBmax = 2 * Ctx::kLanes;
-    const int NB = 2 * c->lanes;
+    constexpr int NB = 2 * Ctx::kLanes;
     if (!c->a_dev) SVDB_CHECK(c, cudaMalloc(&c->a_dev, c->esz * c->max_n * c->max_n));
     c->a_stage[0] = c->a_dev;
     for (int k = 1; k < NB; ++k)
         if (!c->a_stage[k]) SVDB_CHECK(c, cudaMalloc(&c->a_stage[k], c->esz * c->max_n * c->max_n));
-    if (!c->de2) SVDB_CHECK(c, cudaMalloc(&c->de2, c->esz * 2 * NBmax * (c->max_n + 8)));
+    if (!c->de2) SVDB_CHECK(c, cudaMalloc(&c->de2, c->esz * 2 * NB * (c->max_n + 8)));
     cudaStream_t s0 = c->stream;
     SVDB_CHECK(c, cudaEventRecord(c->s2ev[0], s0));
     for (int l = 0; l < Ctx::kLanes; ++l) {
@@ -531,12 +514,12 @@ int bidiagonalize_many_host(Ctx* c, size_t count, T* const* a, const size_t* n, 
         SVDB_CHECK(c, cudaStreamWaitEvent(c->s1ctx[l]->stream, c->s2ev[0], 0));
     }
     struct EvSet {                                                       // buffer k is free again (its D2H copies have finished)
-        cudaEvent_t ev[NBmax] = {};
+        cudaEvent_t ev[NB] = {};
         ~EvSet() { for (auto& x : ev) if (x) cudaEventDestroy(x); }
     } evs;
     cudaEvent_t* ev_free = evs.ev;
     for (auto& ev : evs.ev) SVDB_CHECK(c, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    struct Result { T *a, *d, *e; size_t n; cudaStream_t lane; bool live; } res[NBmax] = {};
+    struct Result { T *a, *d, *e; size_t n; cudaStream_t lane; bool live; } res[NB] = {};
     auto copy_back = [&](int k) -> int {                              // results of the matrix in staging buffer k -> host
         Result& r = res[k];
         if (!r.live) return 0;
@@ -551,13 +534,13 @@ int bidiagonalize_many_host(Ctx* c, size_t count, T* const* a, const size_t* n, 
         return 0;
     };
     int st = 0;
-    const ListPlan pl = plan_list(c->lanes, count, n);
+    const ListPlan pl = plan_list(Ctx::kLanes, count, n);
     size_t per_chain[Ctx::kLanes] = {};
-    bool used[NBmax] = {};
+    bool used[NB] = {};
     for (size_t j = 0; j < count && st == 0; ++j) {
         const size_t i = pl.order[j];
-        const int ch = pl.chain[j] % c->lanes;
-        const int k = ch + c->lanes * (int)(per_chain[ch]++ % 2);     // a chain alternates between its two staging buffers
+        const int ch = pl.chain[j];
+        const int k = ch + Ctx::kLanes * (int)(per_chain[ch]++ % 2);  // a chain alternates between its two staging buffers
         const size_t ni = n[i];
         T* buf = reinterpret_cast<T*>(c->a_stage[k]);
         T* dd = reinterpret_cast<T*>(c->de2) + (size_t)2 * k * (c->max_n + 8);
@@ -739,24 +722,6 @@ int svdb200_create(svdb200_handle* out, int device, size_t max_n, size_t band, i
         SVDB_CREATE_CHECK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         SVDB_CREATE_CHECK(cudaStreamCreateWithPriority(&c->aux_stream, cudaStreamNonBlocking, hi));
         for (auto& e : c->lev) SVDB_CREATE_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        const char* la = getenv("SVDB200_LOOKAHEAD");
-        if (la && la[0] == '0') c->lookahead = 0;
-        const char* pr = getenv("SVDB200_PANEL_REG");
-        if (pr && pr[0] == '0') c->panel_reg = 0;
-        const char* ln = getenv("SVDB200_LANES");
-        if (ln && ln[0] >= '1' && ln[0] <= '4') c->lanes = ln[0] - '0';
-        const char* pl = getenv("SVDB200_PIPE_LIGHT");
-        if (pl && pl[0] == '1') c->pipe_light = 1;
-        const char* s2l = getenv("SVDB200_S2_LIGHT");
-        if (s2l && s2l[0] == '1') c->stage2_light = 1;
-        const char* s2c = getenv("SVDB200_S2_CONST");
-        if (s2c && s2c[0] == '0') c->stage2_const_band = 0;
-        const char* s2f = getenv("SVDB200_S2_FAST");
-        if (s2f && s2f[0] == '0') c->stage2_fast = 0;
-        const char* pb = getenv("SVDB200_PANEL_BLK");
-        if (pb && pb[0] == '0') c->panel_blk = 0;
-        const char* prm = getenv("SVDB200_PANEL_REG_MIN");
-        if (prm && prm[0]) c->panel_reg_min = atoi(prm);
     }
     SVDB_CREATE_CHECK(cudaMalloc(&c->w, es * nb * band));
     c->wpart_elems = 16 * nb * band;
@@ -770,16 +735,6 @@ int svdb200_create(svdb200_handle* out, int device, size_t max_n, size_t band, i
     SVDB_CREATE_CHECK(cudaMemset(c->red2, 0, 512 * 1024));
     SVDB_CREATE_CHECK(cudaMalloc(&c->chol_ws, 1 << 20));
     SVDB_CREATE_CHECK(cudaMemset(c->chol_ws, 0, 1 << 20));
-    {
-        const char* rs = getenv("SVDB200_RESERVE_SMS");
-        if (rs && rs[0]) c->lookahead_reserve = atoi(rs);
-        const char* pc = getenv("SVDB200_PANEL_CHOL");
-        if (pc && pc[0] == '0') c->panel_chol = 0;
-        const char* pp = getenv("SVDB200_PIPE_CHOL");
-        if (pp && pp[0]) c->pipe_chol = pp[0] != '0';
-        const char* pg = getenv("SVDB200_CHOL_GUARD");
-        if (pg && pg[0]) c->chol_guard = atof(pg);
-    }
     SVDB_CREATE_CHECK(cudaMalloc(&c->bar, 64));
     SVDB_CREATE_CHECK(cudaMemset(c->bar, 0, 64));
     SVDB_CREATE_CHECK(cudaMalloc(&c->prog, sizeof(int) * (max_n + 8)));
@@ -1085,7 +1040,8 @@ int svdb200_debug_stage2_fast_timing(long long* out16) { return out16 ? stage2_f
 int svdb200_debug_panel_timing(long long* out16) { return out16 ? panel_reg_debug_read(out16) : SVDB200_E_ARG; }
 int svdb200_debug_panel_blk_timing(long long* out16) { return out16 ? panel_blk_debug_read(out16) : SVDB200_E_ARG; }
 int svdb200_list_plan(int lanes, size_t count, const size_t* n, size_t* order_out, int* chain_out) {
-    if (lanes < 1 || lanes > Ctx::kLanes || (count > 0 && (!n || !order_out || !chain_out))) return SVDB200_E_ARG;
+    constexpr int kMaxPlanLanes = 4;                                  // plans for more chains than the pipeline runs (Ctx::kLanes)
+    if (lanes < 1 || lanes > kMaxPlanLanes || (count > 0 && (!n || !order_out || !chain_out))) return SVDB200_E_ARG;
     const ListPlan pl = plan_list(lanes, count, n);
     for (size_t j = 0; j < count; ++j) { order_out[j] = pl.order[j]; chain_out[j] = pl.chain[j]; }
     return 0;
@@ -1094,14 +1050,13 @@ int svdb200_debug_panel_chol_timing(long long* out16) { return out16 ? panel_cho
 int svdb200_set_panel_kernel(svdb200_handle h, int blocked) {
     if (!h || blocked < 0 || blocked > 2) return SVDB200_E_ARG;
     Ctx* c = reinterpret_cast<Ctx*>(h);
-    c->panel_blk = blocked >= 1;
-    c->panel_chol = blocked == 2;
-    for (auto* s : c->pool) if (s) { s->panel_blk = c->panel_blk; s->panel_chol = c->panel_chol; }
+    c->cfg.panel_blk = blocked >= 1;
+    c->cfg.panel_chol = blocked == 2;
     return 0;
 }
 int svdb200_set_chol_guard(svdb200_handle h, double guard) {
     if (!h || !(guard >= 0.0)) return SVDB200_E_ARG;
-    reinterpret_cast<Ctx*>(h)->chol_guard = guard;
+    reinterpret_cast<Ctx*>(h)->cfg.chol_guard = guard;
     return 0;
 }
 int svdb200_chol_fallback_count(svdb200_handle h, long long* count) {
@@ -1119,17 +1074,15 @@ int svdb200_chol_fallback_count(svdb200_handle h, long long* count) {
 int svdb200_set_stage2_schedule(svdb200_handle h, int mode) {
     if (!h || mode < 0 || mode > 1) return SVDB200_E_ARG;
     Ctx* c = reinterpret_cast<Ctx*>(h);
-    c->stage2_complete = mode;
-    for (auto* s : c->pool) if (s) s->stage2_complete = mode;
+    c->cfg.stage2_complete = mode;
     return 0;
 }
 
 int svdb200_set_qr_method(svdb200_handle h, int method, size_t auto_limit) {
     if (!h || method < 0 || method > 3) return SVDB200_E_ARG;
     Ctx* c = reinterpret_cast<Ctx*>(h);
-    c->qr_method = method;
-    if (auto_limit > 0) c->qr_auto_limit = auto_limit;
-    for (auto* s : c->pool) if (s) { s->qr_method = method; if (auto_limit > 0) s->qr_auto_limit = auto_limit; }
+    c->cfg.qr_method = method;
+    if (auto_limit > 0) c->cfg.qr_auto_limit = auto_limit;
     return 0;
 }
 
@@ -1143,9 +1096,8 @@ int svdb200_tc05_selftest(svdb200_handle h, int a_mn, int b_mn, const float* a, 
 int svdb200_set_tc05(svdb200_handle h, int mode, long long min_elems) {
     if (!h || mode < 0 || mode > 2) return SVDB200_E_ARG;
     Ctx* c = reinterpret_cast<Ctx*>(h);
-    c->use_tc05 = mode;
-    if (min_elems > 0) c->tc05_min_elems = min_elems;
-    for (auto* s : c->pool) if (s) { s->use_tc05 = mode; if (min_elems > 0) s->tc05_min_elems = min_elems; }
+    c->cfg.use_tc05 = mode;
+    if (min_elems > 0) c->cfg.tc05_min_elems = min_elems;
     return 0;
 }
 

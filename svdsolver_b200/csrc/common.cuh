@@ -13,6 +13,21 @@ namespace svdb200 {
 
 constexpr int kMaxBand = 128;          // stage-1 panel width / stage-2 band supported by the kernels
 constexpr int kMaxPanelCtas = 148;     // one CTA per SM in the cooperative panel kernel
+constexpr int kLookaheadReserve = 20;  // SMs the persistent tcgen05 rank update leaves free while a look-ahead panel runs beside it
+
+// Run-time choices set through the C ABI setters.  Sub-handles (batch pool, stage-1 chains of the list pipeline) copy
+// them from their parent before every use.
+struct Settings {
+    int stage2_complete = 0;                // 0: the reference's window schedule (parity), 1: complete chase
+    // singular values of the bidiagonal: 0 auto (zero-shift QR up to qr_auto_limit, bisection above), 1 QR, 2 bisection
+    int qr_method = 0;
+    size_t qr_auto_limit = 1024;
+    int use_tc05 = 1;                       // 0 off, 1 when the update is large enough, 2 always (tests)
+    long long tc05_min_elems = 8LL << 20;   // smallest M*N the tcgen05 kernels are used for in mode 1
+    int panel_blk = 1;                      // blocked panel kernel (one exchange per 8 columns, stage1_panel_blk.cu) where the shape allows
+    int panel_chol = 1;                     // Cholesky-QR panel with reconstructed Householder vectors (stage1_panel_chol.cu)
+    double chol_guard = 1e-3;               // smallest accepted pivot ratio R_jj^2 / G_jj; below, the exchange-based kernels redo the panel
+};
 
 struct Ctx {
     int device = 0;
@@ -27,9 +42,6 @@ struct Ctx {
     void* vb = nullptr; void* v2b = nullptr;   // second reflector pair (LQ panels) for the look-ahead
     cudaStream_t aux_stream = nullptr;         // high-priority stream the look-ahead panels run on
     cudaEvent_t lev[4] = {};
-    int lookahead = 1;
-    int panel_reg = 1;             // use the register-resident panel kernel when the shape allows
-    int panel_reg_min = 768;       // ... for panels taller than this (SVDB200_PANEL_REG_MIN); below, the shared-memory kernel
     void* w = nullptr;             // band * max_n  : W = V^T A  /  max_n * band : W = A U^T
     void* wpart = nullptr;         // split-K partials
     size_t wpart_elems = 0;
@@ -63,37 +75,22 @@ struct Ctx {
     // tcgen05 FP32 path (gemm_tc05.cu): hi/lo split scratch for the O(n b) operands, allocated on first use
     void* tcsplit = nullptr;
     size_t tcsplit_elems = 0;
-    int use_tc05 = 1;                       // 0 off, 1 when the update is large enough, 2 always (tests)
-    long long tc05_min_elems = 8LL << 20;   // smallest M*N the tcgen05 kernels are used for in mode 1
-    // singular values of the bidiagonal: 0 auto (zero-shift QR up to qr_auto_limit, bisection above), 1 QR, 2 bisection
+    Settings cfg;
     // pipelined multi-matrix driver (bidiagonalize_many): stage 2 of matrix i on s2_stream beside stage 1 of matrix i+1
-    int lanes = 2;                          // chains actually used (<= kLanes; SVDB200_LANES)
-    int pipe_light = 0;                     // pipelined driver: light stage-2 variant (SVDB200_PIPE_LIGHT)
-    static constexpr int kLanes = 4;        // chains in flight: each = one stage 1 (own sub-handle) and one stage-2 kernel (85-register
-                                            // variant, 3 CTAs per SM: four sweep pipelines of n <= 4096 fit the GPU beside the stage-1 kernels)
+    static constexpr int kLanes = 2;        // chains in flight: each = one stage 1 (own sub-handle) and one stage-2 kernel
+                                            // (more chains measured slower: they disturb each other's stage-2 sweep pipelines)
     cudaStream_t s2_stream[kLanes] = {};
     int* s2_prog[kLanes] = {};              // progress counters per lane
     cudaEvent_t s2ev[4 + kLanes] = {};
     int onestage = 0;                       // stage-1 driver in the one-stage Golub-Kahan order (band 1, no skipped row reflector)
     int s2_ready = 0;                       // the pipeline's streams / counters / sub-handles below exist (all or nothing)
-    int panel_blk = 1;                      // blocked panel kernel (one exchange per 8 columns, stage1_panel_blk.cu) where the shape allows
-    int panel_chol = 1;                     // Cholesky-QR panel with reconstructed Householder vectors (stage1_panel_chol.cu); env SVDB200_PANEL_CHOL=0: off
-    int pipe_chol = 0;                      // ... also for stage 1 beside resident stage-2 grids (list pipeline; SVDB200_PIPE_CHOL=1): measured slower there (its kernels disturb the latency-bound stage-2 chains: 2896 -> 2211-2551 GFLOP/s on the bench sweep)
-    void* chol_ws = nullptr;                // its workspace: status word, [M1 | M2], partial Gram matrices (1 MB)
-    double chol_guard = 1e-3;               // smallest accepted pivot ratio R_jj^2 / G_jj; below, the exchange-based kernels redo the panel
+    void* chol_ws = nullptr;                // Cholesky-QR panel workspace: status word, [M1 | M2], partial Gram matrices (1 MB)
     const int* panel_run_if = nullptr;      // set while a gated fallback panel launch is being enqueued
-    int lookahead_reserve = 20;             // SMs the persistent tcgen05 rank update leaves free while a look-ahead panel runs beside it (SVDB200_RESERVE_SMS)
     int reserve_now = 0;                    // set by the stage-1 drivers around the part of an update that overlaps a panel
     int overlap_safe = 0;                   // stage 1 may only use kernels without cross-cluster / grid-wide waits
     Ctx* s1ctx[kLanes] = {};                // sub-handles (own workspace + streams): stage 1 of two matrices at a time
     void* a_stage[2 * kLanes] = {};         // staging buffers + bidiagonal rows for the host-pointer variant
     void* de2 = nullptr;
-    int stage2_light = 0;                   // single matrix: use the 85-register stage-2 variant (3 CTAs per SM) -- pipelined driver
-    int stage2_complete = 0;                // 0: the reference's window schedule (parity), 1: complete chase
-    int stage2_fast = 1;                // band 32: helper-warp / split-product kernel (stage2_chase_fast.cu; env SVDB200_S2_FAST=0: off)
-    int stage2_const_band = 1;          // band-specialised stage-2 kernels for band 32 / 64 (env SVDB200_S2_CONST=0: generic)
-    int qr_method = 0;
-    size_t qr_auto_limit = 1024;
     void* bis_ws = nullptr;
     size_t bis_ws_elems = 0;
     std::vector<void*> band_capture;           // test hook of bidiagonalize_many_*: device buffers that receive matrix i's band

@@ -14,7 +14,7 @@
 //                  The panel's status word is read back by the host (after the concurrent part of the QR update has been
 //                  enqueued): a row panel below the pivot-ratio guard -- e.g. the first one of a matrix with a large
 //                  common mean -- is redone through the fallback, identically on every rank.
-//                  Fallback (also: band not 8/16/32/64, panels narrower than 2 b, SVDB200_PANEL_CHOL=0): ncclAllGather of
+//                  Fallback (also: band not 8/16/32/64, panels narrower than 2 b, svdb200_dist_configure_panels(h, 0)): ncclAllGather of
 //                  the local pieces, every rank factorises the SAME assembled panel redundantly.
 //                  W = A U^T is a sum over the column distribution: local partial product +
 //                  ncclAllReduce(sum) of m' x b, then the local rank-b update.
@@ -97,8 +97,7 @@ struct Dist {
     cudaEvent_t ev_status = nullptr, ev_qstatus = nullptr;
     void* qsend = nullptr;       // QR panel message: raw rows | [M1 | M2] | top blocks of V, V2 | status
     int qr_dist = 1;             // 1: QR panels travel as raw rows + band x band factors (second pass on every rank); 0: [V | V S^T]
-    int qr_early = 1;            // the raw rows are broadcast on a third stream while the owner factorises (SVDB200_DIST_EARLY_BCAST=0: off)
-    cudaStream_t bc_stream = nullptr;
+    cudaStream_t bc_stream = nullptr;  // the raw QR panel rows are broadcast on this third stream while the owner factorises
     cudaEvent_t ev_raw = nullptr, ev_rawdone = nullptr;
     long long qr_fallbacks = 0;
     long long lq_fallbacks = 0;  // row panels the Cholesky-QR path gave up on (redone through the gather path)
@@ -228,7 +227,7 @@ int dist_stage1(Dist* d, T* a, size_t n, size_t band) {
     T* sendbuf = reinterpret_cast<T*>(d->sendbuf);
     T* ut_loc = reinterpret_cast<T*>(d->ut_loc);
     T* u2_loc = reinterpret_cast<T*>(d->u2_loc);
-    const bool ahead = !c->profile && c->aux_stream != nullptr && c->lookahead;
+    const bool ahead = !c->profile && c->aux_stream != nullptr;
     cudaStream_t s0 = c->stream, s1 = ahead ? c->aux_stream : c->stream;
     cudaEvent_t evQ = c->lev[1], evR = c->lev[2], evL = c->lev[3], evP = c->lev[0];
     if (ahead) {   // the aux stream must see everything enqueued on the main stream so far
@@ -248,10 +247,10 @@ int dist_stage1(Dist* d, T* a, size_t n, size_t band) {
         const int owner = (int)(k % P);
         T* v2k = V + m * band;
         if (rk == owner) {
-            const int keep = c->panel_chol;
-            if (!allow_chol) c->panel_chol = 0;
+            const int keep = c->cfg.panel_chol;
+            if (!allow_chol) c->cfg.panel_chol = 0;
             const int st = launch_panel_public<T, false>(c, a + o * ldl + (k / P) * band, ldl, (int)m, b, V, v2k, s1);
-            c->panel_chol = keep;
+            c->cfg.panel_chol = keep;
             SVDB_TRY(st);
         }
         if (P > 1) SVDB_NCCL(d, nccl().Broadcast(V, V, 2 * m * band, nccl_type<T>(), owner, d->comm, s1));
@@ -263,7 +262,7 @@ int dist_stage1(Dist* d, T* a, size_t n, size_t band) {
         qr_pending = false;
         if (P > 1 && d->qr_dist && chol_dist_supported(c, b) && m >= 2 * band) {
             T* qs = reinterpret_cast<T*>(d->qsend);
-            if (ahead && d->qr_early && d->bc_stream) {
+            if (ahead && d->bc_stream) {
                 // the raw rows travel on a third stream while the owner runs pass 1 and the algebra on its copy; the small
                 // tail of the message ([M1 | M2], top blocks, status) follows on s1.  Every rank issues the two broadcasts
                 // in this order.
@@ -369,7 +368,7 @@ int dist_stage1(Dist* d, T* a, size_t n, size_t band) {
         }
         // s0: the rest of the QR update runs beside the LQ panel
         if (ncl > 0 && mr > 0) {
-            c->reserve_now = ahead ? c->lookahead_reserve : 0;               // the LQ panel runs beside this
+            c->reserve_now = ahead ? kLookaheadReserve : 0;                  // the LQ panel runs beside this
             const int st = rank_update<T>(c, A2 + band * ldl, ldl, mr, ncl, band, V2 + band * band, W, ncl);
             c->reserve_now = 0;
             SVDB_TRY(st);
@@ -400,7 +399,7 @@ int dist_stage1(Dist* d, T* a, size_t n, size_t band) {
             }
             SVDB_TRY(qr_panel_and_bcast(k + 1));                           // s1: panel k+1 + broadcast
             if (ahead && ncl > 0) {
-                c->reserve_now = c->lookahead_reserve;                       // QR panel k+1 (on its owner) runs beside this
+                c->reserve_now = kLookaheadReserve;                          // QR panel k+1 (on its owner) runs beside this
                 int st = 0;
                 if (own_next) { if (ncl > band) st = rank_update<T>(c, A3 + band, ldl, mr, ncl - band, band, W, u2_loc + band, ncl); }
                 else st = rank_update<T>(c, A3, ldl, mr, ncl, band, W, u2_loc, ncl);
@@ -532,8 +531,6 @@ int svdb200_dist_create(svdb200_dist_handle* out, int device, int rank, int nran
         int lo = 0, hi = 0;
         e = cudaDeviceGetStreamPriorityRange(&lo, &hi);
         if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&d->bc_stream, cudaStreamNonBlocking, hi);
-        const char* eb = getenv("SVDB200_DIST_EARLY_BCAST");
-        if (eb && eb[0] == '0') d->qr_early = 0;
     }
     if (e == cudaSuccess) e = cudaMalloc(&d->qsend, es * ((n + 256) * band + 4 * band * band + 64));
     if (e != cudaSuccess) { int s2 = cuda_status(d->ctx, e, "cudaMalloc(dist)"); svdb200_dist_destroy(reinterpret_cast<svdb200_dist_handle>(d)); return s2; }

@@ -711,10 +711,10 @@ static int launch_split(Ctx* c, const float* src, size_t ld_src, int rows, int c
 }
 
 static bool wanted(Ctx* c, int M, int N, int B) {
-    if (c->use_tc05 == 0) return false;
+    if (c->cfg.use_tc05 == 0) return false;
     if (B != 32 && B != 64) return false;
-    if (c->use_tc05 >= 2) return true;
-    return (long long)M * N >= (long long)c->tc05_min_elems;
+    if (c->cfg.use_tc05 >= 2) return true;
+    return (long long)M * N >= (long long)c->cfg.tc05_min_elems;
 }
 
 }  // namespace tc05

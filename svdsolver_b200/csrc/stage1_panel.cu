@@ -262,7 +262,7 @@ int launch_panel(Ctx* c, T* a, size_t lda, int m, int b, T* V = nullptr, T* V2 =
     if (!V) V = reinterpret_cast<T*>(c->v);
     if (!V2) V2 = reinterpret_cast<T*>(c->v2);
     c->panel_run_if = nullptr;
-    if (c->panel_chol) {
+    if (c->cfg.panel_chol) {
         const int st = launch_panel_chol<T, kTrans>(c, a, lda, m, b, V, V2, stream);
         if (st == 0) c->panel_run_if = chol_status(c);        // the exchange-based kernel below runs only if the guard tripped
         else if (st != 1) return st;
@@ -274,13 +274,14 @@ int launch_panel(Ctx* c, T* a, size_t lda, int m, int b, T* V = nullptr, T* V2 =
 
 template <typename T, bool kTrans>
 int launch_panel_exchange(Ctx* c, T* a, size_t lda, int m, int b, T* V, T* V2, cudaStream_t stream) {
-    if (c->panel_blk) {
+    if (c->cfg.panel_blk) {
         int st = launch_panel_blk<T, kTrans>(c, a, lda, m, b, V, V2, stream);
         if (st != 1) return st;
     }
     // register-resident kernel for tall panels (grid transport); cluster-sized panels are issue-bound
     // either way and stay on the shared-memory kernel below
-    if (c->panel_reg && m > c->panel_reg_min) {
+    constexpr int kPanelRegMinRows = 768;
+    if (m > kPanelRegMinRows) {
         int st = launch_panel_reg<T, kTrans>(c, a, lda, m, b, V, V2, stream, stream == c->stream);
         if (st != 1) return st;
     }
@@ -415,7 +416,7 @@ int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
     T* Vl = reinterpret_cast<T*>(c->vb);
     T* V2l = reinterpret_cast<T*>(c->v2b);
     T* W = reinterpret_cast<T*>(c->w);
-    const bool ahead = !c->profile && c->aux_stream != nullptr && c->lookahead;
+    const bool ahead = !c->profile && c->aux_stream != nullptr;
     cudaStream_t s0 = c->stream, s1 = ahead ? c->aux_stream : c->stream;
     if (ahead) {   // the aux stream must see everything enqueued on the main stream so far
         SVDB_CHECK(c, cudaEventRecord(c->lev[0], s0));
@@ -443,7 +444,7 @@ int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
                 SVDB_TRY((launch_panel<T, true>(c, A2, n, (int)nc, b, Vl, V2l, s1)));    // LQ panel (look-ahead)
                 if (ahead) SVDB_CHECK(c, cudaEventRecord(c->lev[3], s1));
                 if (m > band) {
-                    c->reserve_now = ahead ? c->lookahead_reserve : 0;       // the LQ panel runs beside this
+                    c->reserve_now = ahead ? kLookaheadReserve : 0;          // the LQ panel runs beside this
                     const int st = rank_update<T>(c, A2 + band * n, n, m - band, nc, band, V2q + band * band, W, nc);
                     c->reserve_now = 0;
                     SVDB_TRY(st);
@@ -466,7 +467,7 @@ int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
                 SVDB_TRY((launch_panel<T, false>(c, A3, n, (int)mr, b, Vq, V2q, s1)));   // QR panel k+1 (look-ahead)
                 if (ahead) SVDB_CHECK(c, cudaEventRecord(c->lev[1], s1));
                 if (nc > band) {
-                    c->reserve_now = ahead ? c->lookahead_reserve : 0;       // QR panel k+1 runs beside this
+                    c->reserve_now = ahead ? kLookaheadReserve : 0;          // QR panel k+1 runs beside this
                     const int st = rank_update<T>(c, A3 + band, n, mr, nc - band, band, W, V2l + band, nc);
                     c->reserve_now = 0;
                     SVDB_TRY(st);

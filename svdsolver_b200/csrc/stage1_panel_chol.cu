@@ -653,19 +653,9 @@ inline cudaError_t smem_attr_once(Ctx* c, K kern, size_t smem, bool (&done)[16])
 }
 
 struct GramShape { int rows, ng, cs, np; };
-// small: beside resident stage-2 grids (list pipeline) -- at most 32 CTAs and no cluster, so that the launch needs no group of
-// free SMs in one GPC
-inline GramShape gram_shape(int mrows, int num_sms, bool small = false) {
+inline GramShape gram_shape(int mrows, int num_sms) {
     GramShape g;
     if (mrows <= 0) { g.rows = 8; g.ng = 0; g.cs = 1; g.np = 0; return g; }
-    if (small) {
-        const int target = std::max(1, std::min(18, (mrows + 127) / 128));
-        g.rows = ((mrows + target - 1) / target + 7) / 8 * 8;
-        g.ng = (mrows + g.rows - 1) / g.rows;
-        g.cs = 1;
-        g.np = g.ng;
-        return g;
-    }
     const int target = std::max(1, std::min(num_sms / kGramCluster * kGramCluster, (mrows + 63) / 64));
     g.rows = ((mrows + target - 1) / target + 7) / 8 * 8;
     g.ng = (mrows + g.rows - 1) / g.rows;
@@ -704,14 +694,14 @@ int launch_chol(Ctx* c, T* a, size_t lda, int m, T* V, T* V2, cudaStream_t strea
     int* status = reinterpret_cast<int*>(ws);
     T* mcat = reinterpret_cast<T*>(ws + 256);
     double* part = reinterpret_cast<double*>(ws + 256 + 64 * 128 * 8);
-    const GramShape g = gram_shape(m, c->num_sms, c->overlap_safe != 0);     // pass 1 over ALL rows: the partials sum to G itself
+    const GramShape g = gram_shape(m, c->num_sms);     // pass 1 over ALL rows: the partials sum to G itself
     SVDB_TRY((gram_launch<T, kTrans, B>(c, a, lda, 0, m, part, g, stream)));
     {
         auto kern = chol_algebra_kernel<T, kTrans, B>;
         const size_t smem = chol_algebra_smem(B);
         { static bool attr_done[16] = {}; SVDB_CHECK(c, smem_attr_once(c, kern, smem, attr_done)); }
         const size_t ldv2r = kTrans ? 1 : (size_t)B, ldv2c = kTrans ? (size_t)m : 1;
-        kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, V, V2, ldv2r, ldv2c, mcat, status, c->chol_guard, 0);
+        kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, V, V2, ldv2r, ldv2c, mcat, status, c->cfg.chol_guard, 0);
         c->launches++;
     }
     {
@@ -732,8 +722,9 @@ int launch_chol(Ctx* c, T* a, size_t lda, int m, T* V, T* V2, cudaStream_t strea
 // 0: launched (the caller must enqueue a fallback panel kernel gated on chol_status()); 1: shape not covered
 template <typename T, bool kTrans>
 int launch_panel_chol(Ctx* c, T* a, size_t lda, int m, int b, T* V, T* V2, cudaStream_t stream) {
-    if (!c->chol_ws || m < 2 * b) return 1;
-    if (c->overlap_safe && !c->pipe_chol) return 1;
+    // not beside resident stage-2 grids (overlap_safe): measured slower there, its kernels disturb the latency-bound stage-2
+    // chains of the list pipeline (2896 -> 2211-2551 GFLOP/s on the bench sweep)
+    if (!c->chol_ws || m < 2 * b || c->overlap_safe) return 1;
     switch (b) {
         case 8: return launch_chol<T, kTrans, 8>(c, a, lda, m, V, V2, stream);
         case 16: return launch_chol<T, kTrans, 16>(c, a, lda, m, V, V2, stream);
@@ -802,10 +793,10 @@ int dist_lq_finish(Ctx* c, T* a2, size_t ldl, int row0, int ncl, bool own_top, c
         const size_t smem = chol_algebra_smem(B);
         { static bool attr_done[16] = {}; SVDB_CHECK(c, smem_attr_once(c, kern, smem, attr_done)); }
         if (own_top)
-            kern<<<1, kAlgThreads, smem, stream>>>(a2, ldl, buf + NE, buf, 1, ut_loc, u2_loc, (size_t)1, (size_t)ncl, mcat, status, c->chol_guard, 0);
+            kern<<<1, kAlgThreads, smem, stream>>>(a2, ldl, buf + NE, buf, 1, ut_loc, u2_loc, (size_t)1, (size_t)ncl, mcat, status, c->cfg.chol_guard, 0);
         else
             kern<<<1, kAlgThreads, smem, stream>>>(scratch, (size_t)B, buf + NE, buf, 1, scratch + B * B, scratch + 2 * B * B, (size_t)1, (size_t)B,
-                                                   mcat, status, c->chol_guard, 0);
+                                                   mcat, status, c->cfg.chol_guard, 0);
         c->launches++;
     }
     if (ncl > row0) {
@@ -822,7 +813,7 @@ int dist_lq_finish(Ctx* c, T* a2, size_t ldl, int row0, int ncl, bool own_top, c
 }  // namespace
 
 size_t chol_dist_buf_elems(int b) { const int nb8 = b / 8; return (size_t)nb8 * (nb8 + 1) / 2 * 64 + (size_t)b * b; }
-bool chol_dist_supported(const Ctx* c, int b) { return c->chol_ws && c->panel_chol && (b == 8 || b == 16 || b == 32 || b == 64); }
+bool chol_dist_supported(const Ctx* c, int b) { return c->chol_ws && c->cfg.panel_chol && (b == 8 || b == 16 || b == 32 || b == 64); }
 
 template <typename T>
 int chol_dist_lq_gram(Ctx* c, const T* a2, size_t ldl, int b, int row0, int ncl, bool own_top, double* buf, cudaStream_t stream) {
@@ -913,7 +904,7 @@ int dist_qr_owner(Ctx* c, T* a, size_t lda, int m, T* qsend, cudaStream_t stream
     auto kern = chol_algebra_kernel<T, false, B>;
     const size_t smem = chol_algebra_smem(B);
     { static bool attr_done[16] = {}; SVDB_CHECK(c, smem_attr_once(c, kern, smem, attr_done)); }
-    kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, vtop, v2top, (size_t)B, (size_t)1, mcat, status, c->chol_guard, 1);
+    kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, vtop, v2top, (size_t)B, (size_t)1, mcat, status, c->cfg.chol_guard, 1);
     c->launches++;
     const size_t tot = (size_t)(m - B) * B;
     int blocks = (int)std::min<size_t>((tot + 1023) / 1024, (size_t)4 * c->num_sms);
@@ -947,7 +938,7 @@ int dist_qr_owner_early(Ctx* c, T* a, size_t lda, int m, T* qsend, int phase, cu
     auto kern = chol_algebra_kernel<T, false, B>;
     const size_t smem = chol_algebra_smem(B);
     { static bool attr_done[16] = {}; SVDB_CHECK(c, smem_attr_once(c, kern, smem, attr_done)); }
-    kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, vtop, v2top, (size_t)B, (size_t)1, mcat, status, c->chol_guard, 1);
+    kern<<<1, kAlgThreads, smem, stream>>>(a, lda, (const double*)nullptr, part, g.np, vtop, v2top, (size_t)B, (size_t)1, mcat, status, c->cfg.chol_guard, 1);
     c->launches++;
     qr_zero_kernel<T><<<blocks, 256, 0, stream>>>(a, lda, m, B, flag, status);
     c->launches++;

@@ -206,13 +206,11 @@ int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int co
     if (smem > 227 * 1024) return SVDB200_E_CAPACITY;
     // small bands run with <= 256 threads: instantiate that case without the 64-register cap; a batch wants
     // several CTAs per SM instead (the window product is FP64-issue bound for ~40 % of an op, the rest is latency)
-    const bool light = count > 1 || c->stage2_light;
+    const bool light = count > 1;
     auto kern = nt <= 256 ? (light ? stage2_chase_kernel<T, 256, 3, 0> : stage2_chase_kernel<T, 256, 1, 0>)
                           : stage2_chase_kernel<T, 1024, 1, 0>;
-    if (c->stage2_const_band) {                                      // band-specialised instances (same arithmetic)
-        if (cb == 32) kern = light ? stage2_chase_kernel<T, 256, 3, 32> : stage2_chase_kernel<T, 256, 1, 32>;
-        else if (cb == 64) kern = stage2_chase_kernel<T, 1024, 1, 64>;
-    }
+    if (cb == 32) kern = light ? stage2_chase_kernel<T, 256, 3, 32> : stage2_chase_kernel<T, 256, 1, 32>;   // band-specialised
+    else if (cb == 64) kern = stage2_chase_kernel<T, 1024, 1, 64>;                                           // (same arithmetic)
     SVDB_CHECK(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     SVDB_CHECK(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nt, smem));
@@ -238,9 +236,9 @@ int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int co
         prog = c->batch_prog;
     }
     SVDB_CHECK(c, cudaMemsetAsync(prog, 0, sizeof(int) * n * (size_t)count, c->stream));
-    int ni = (int)n, bi = cb, cnt = count, gi = (int)G, complete = c->stage2_complete;
+    int ni = (int)n, bi = cb, cnt = count, gi = (int)G, complete = c->cfg.stage2_complete;
     int fast = 1;                                                      // 0 = the latency-optimised band-32 kernel ran
-    if (count == 1 && c->stage2_fast && !light) {
+    if (count == 1) {
         fast = stage2_chase_fast<T>(c, a, n, band, prog);
         if (fast != 0 && fast != 1) return fast;
     }

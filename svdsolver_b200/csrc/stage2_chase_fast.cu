@@ -319,7 +319,7 @@ int stage2_chase_fast(Ctx* c, T* a, size_t n, size_t band, int* prog) {
     long long inflight = (long long)(n / band) / 2 + 2;
     long long G = std::min(inflight, std::min((long long)per_sm * c->num_sms, (long long)n - 1));
     if (G < 1) G = 1;
-    int ni = (int)n, complete = c->stage2_complete;
+    int ni = (int)n, complete = c->cfg.stage2_complete;
     void* args[] = {&a, &ni, &prog, &complete};
     SVDB_CHECK(c, cudaLaunchCooperativeKernel((void*)kern, dim3((unsigned)G), dim3(kFastThreads), args, smem, c->stream));
     c->launches++;
