@@ -210,8 +210,8 @@ int svdb200_debug_panel_chol_timing(long long* out16);
 int svdb200_debug_panel_timing(long long* out16);
 /* same for the stage-2 kernel (-DSVDB_S2_TIMING=1): RIGHT ops of CTA 1 */
 int svdb200_debug_stage2_timing(long long* out16);
-/* same for the band-32 latency-optimised kernel (interior RIGHT ops of CTA 1; slots documented in tools/stage2_only.py) */
-int svdb200_debug_stage2_fast_timing(long long* out16);
+/* 24 cycle counters of the band-32 latency-optimised kernel (CTA 1; slots documented in tools/stage2_only.py) */
+int svdb200_debug_stage2_fast_timing(long long* out24);
 /* Singular values of the bidiagonal (svdb200_bidiag_qr_*, svdb200_svdvals_*): method 0 = automatic (the
  * reference's zero-shift QR sweeps, serial::qrd svd_serial.h:368, for n <= auto_limit, bisection on the
  * Golub-Kahan form above: zero-shift QR needs ~n log(1/tol) sweeps), 1 = always zero-shift QR, 2 = always

@@ -1036,7 +1036,7 @@ int svdb200_probe_peak(svdb200_handle h, int kind, double* tflops) {
 }
 
 int svdb200_debug_stage2_timing(long long* out16) { return out16 ? stage2_debug_read(out16) : SVDB200_E_ARG; }
-int svdb200_debug_stage2_fast_timing(long long* out16) { return out16 ? stage2_fast_debug_read(out16) : SVDB200_E_ARG; }
+int svdb200_debug_stage2_fast_timing(long long* out24) { return out24 ? stage2_fast_debug_read(out24) : SVDB200_E_ARG; }
 int svdb200_debug_panel_timing(long long* out16) { return out16 ? panel_reg_debug_read(out16) : SVDB200_E_ARG; }
 int svdb200_debug_panel_blk_timing(long long* out16) { return out16 ? panel_blk_debug_read(out16) : SVDB200_E_ARG; }
 int svdb200_list_plan(int lanes, size_t count, const size_t* n, size_t* order_out, int* chain_out) {

@@ -231,7 +231,7 @@ int panel_reg_debug_read(long long* out16);
 int panel_blk_debug_read(long long* out16);
 int panel_chol_debug_read(long long* out16);
 int stage2_debug_read(long long* out16);
-int stage2_fast_debug_read(long long* out16);
+int stage2_fast_debug_read(long long* out24);
 int tc05_selftest(Ctx* c, int a_mn, int b_mn, const float* a, const float* b, float* out, float* dump);
 
 }  // namespace svdb200

@@ -11,8 +11,18 @@
 //   * the window product is split by operand: warps 0-3 multiply the block that is already in shared memory (forwarded
 //     by the previous op) while warps 4-7 fetch the new block from L2, store it and multiply it -- the L2 latency of the
 //     fetch hides behind the first half instead of behind the scalars.
-// Only interior windows (full c x c blocks) take this path; the top pair of a sweep and the clamped windows at the matrix
-// edge run the generic code of the original kernel (inside this kernel, on the same shared-memory layout).
+//   * the head of a sweep runs on the same split: RIGHT(0)'s Householder vector is row i, cols [i+1, i+1+c), which sweep
+//     i-1 writes for the last time in its op 2 (RIGHT(1); sweeps further back in earlier ops, tests/test_stage2_head.py).
+//     So the helper warp loads that row and prepares H as soon as the predecessor has finished 3 ops, while thread 0
+//     still waits for the 4 that guard the window.  RIGHT(0)'s window is then row i (to global: F warps) over the c x c
+//     block forwarded to LEFT(0) (N warps), and the helper prepares LEFT(0)'s reflector from that block as in any
+//     interior RIGHT.  Per sweep this takes the one-thread scalars, build_h and the generic product off ops 0 and 1,
+//     which are the ops that gate when the successor sweep may start;
+//   * progress is released when the op's global accesses are done, not when the op is: the N warps arrive on bar 2 once
+//     the new block sits in shared memory, the F warps sync on it after storing the finished block, and an F thread
+//     releases.  The N product and the helper's reflector only touch shared memory and finish behind the release.
+// Clamped windows at the matrix edge run the generic code of the original kernel (inside this kernel, on the same
+// shared-memory layout), which releases after its closing barrier.
 #include <algorithm>
 #include <climits>
 #include "common.cuh"
@@ -26,8 +36,9 @@ using namespace s2;
 #ifndef SVDB_S2_TIMING
 #define SVDB_S2_TIMING 0
 #endif
-// per-phase cycle counters of interior RIGHT ops of CTA 1 (debug builds: -DSVDB_S2_TIMING=1); every slot has one writer
-__device__ long long g_s2f_dbg[16];
+// cycle counters of CTA 1 (debug builds: -DSVDB_S2_TIMING=1; slots named in tools/stage2_only.py); every slot has one writer
+constexpr int kDbgSlots = 24;
+__device__ long long g_s2f_dbg[kDbgSlots];
 #define S2F_T() (SVDB_S2_TIMING ? clock64() : 0ll)
 #define S2F_ADD(k, v)                                                   \
     do {                                                                \
@@ -39,6 +50,10 @@ constexpr int kMain = 256;             // main threads: warps 0-3 = F half, warp
 constexpr int kFastThreads = kMain + 32;
 
 __device__ __forceinline__ void bar_n_helper() { asm volatile("bar.sync 1, 160;" ::: "memory"); }   // N warps + helper warp
+// F + N warps: the N warps arrive once their fetched block is in shared memory, the F warps sync after their global stores,
+// so an F thread may then release progress: every global load and store of the op is done
+__device__ __forceinline__ void bar_fn_arrive() { asm volatile("bar.arrive 2, 256;" ::: "memory"); }
+__device__ __forceinline__ void bar_fn_sync() { asm volatile("bar.sync 2, 256;" ::: "memory"); }
 
 // Helper warp: reflector of the next op from its Householder vector xv (lane l holds x_l), exactly as
 // reflector_scalars + build_h do it (sequential unfused sum of squares in index order; scalars in double; H = I - tau w w^T
@@ -109,7 +124,23 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
         const int top_j2 = min(i + 2 * w - 1, n);
         const int npairs = complete ? (n - i - 1 + c - 1) / c : 1 + (n - top_j2) / c + 1;
         int fr = 0;
-        bool hready = false;                    // Hc already holds the H of the op about to run (written by the helper)
+        // Hc already holds the H of the op about to run (written by the helper).  The head window is full exactly when
+        // LEFT(0) can be interior, so every split op starts with its H ready.
+        bool hready = i + 1 + c <= n;
+        if (SVDB_S2_TIMING && tid == 0) { S2F_ADD(14, 1); if (hready) S2F_ADD(22, 1); }
+        if (hready && is_helper) {              // RIGHT(0)'s H from row i, as soon as sweep i-1 has written it (op 2)
+            const int lane = tid & 31;
+            const long long t_h0 = S2F_T();
+            if (i > 0) {
+                if (lane == 0) wait_progress(&prog[i - 1], 3, 0);
+                __syncwarp();
+            }
+            const long long t_h1 = S2F_T();
+            const T xv = ld_cg(&A[(size_t)i * N + (i + 1 + lane)]);
+            WR[lane] = xv;
+            helper_reflector<T>(xv, xst, Hc, ldh, complete != 0);
+            if (tid == kMain) { S2F_ADD(20, t_h1 - t_h0); S2F_ADD(21, S2F_T() - t_h1); }
+        }
         for (int p = 0; p < npairs; ++p) {
             const int r0 = (p == 0) ? i : min(i + 1 + (p - 1) * c, n);
             const int r1 = min(i + 1 + p * c, n), r2 = min(i + 1 + (p + 1) * c, n), c3 = min(i + 1 + (p + 2) * c, n);
@@ -122,59 +153,60 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                 const long long t_polled = S2F_T();
                 __syncthreads();
                 const long long t_start = S2F_T();
-                const int nc = r2 - r1, nr = r2 - r0, have = fr;
-                const bool interior = (have == c) && (nr == 2 * c) && (nc == c);
-                if (interior) {
-                    if (tid == 0) { S2F_ADD(0, t_polled - t_op0); S2F_ADD(9, t_start - t_polled); S2F_ADD(7, 1); if (!hready) S2F_ADD(10, 1); }
+                if (tid == 0 && q == 0) S2F_ADD(15, t_polled - t_op0);
+                const int nc = r2 - r1, nr = r2 - r0, have = fr, keep = r1 - r0;
+                // split: F = the rows finished here (c of them; row i only at the head), N = the c x c block forwarded to LEFT(p)
+                const bool split = (nc == c) && (p == 0 || (have == c && nr == 2 * c));
+                if (split) {
+                    const bool tm = p > 0 && tid == 0;        // the per-phase counters cover interior ops only
+                    if (tm) { S2F_ADD(0, t_polled - t_op0); S2F_ADD(9, t_start - t_polled); S2F_ADD(7, 1); }
                     T nv[8];
-                    if (n_warp) {                 // new block: rows [c,2c) of the window, 8 elements per thread
+                    if (n_warp) {                 // new block: rows [keep, keep+c) of the window, 8 elements per thread
 #pragma unroll
                         for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[(size_t)(r1 + (ht >> 5) + 4 * u) * N + (r1 + (ht & 31))]);
                     }
-                    if (!hready) {                // first interior op of a sweep: H the classic way
-                        if (tid == 0) reflector_scalars<T>(WR, 1, c, sc, complete != 0);
-                        __syncthreads();
-                        if (is_main) build_h<T>(WR, 1, c, sc, Hc, ldh, tx, ty, tys);
-                        __syncthreads();
-                    }
-                    const long long t_h = S2F_T();
                     long long t_done = 0;
                     if (f_warp) {                 // F half: finished rows [r0,r1) -> global
-                        window_product<T, kC>(WR, ldr, Hc, ldh, c, c, c, 16, 8,
+                        window_product<T, kC>(WR, ldr, Hc, ldh, keep, c, c, 16, 8,
                                               [&](int r, int cc, T v) { st_cg(&A[(size_t)(r0 + r) * N + (r1 + cc)], v); }, tid);
                         t_done = S2F_T();
-                        if (tid == 0) { S2F_ADD(11, t_h - t_start); S2F_ADD(1, t_done - t_h); }
+                        bar_fn_sync();
+                        const long long t_rel = S2F_T();
+                        if (tid == rel_tid) st_release(&prog[i], q + 1);
+                        if (tm) { S2F_ADD(1, t_done - t_start); S2F_ADD(10, t_rel - t_done); }
+                        if (p > 0 && tid == rel_tid) S2F_ADD(11, t_rel - t_start);
                     } else if (n_warp) {
 #pragma unroll
-                        for (int u = 0; u < 8; ++u) WR[(c + (ht >> 5) + 4 * u) * ldr + (ht & 31)] = nv[u];
+                        for (int u = 0; u < 8; ++u) WR[(keep + (ht >> 5) + 4 * u) * ldr + (ht & 31)] = nv[u];
                         const long long t_ld = S2F_T();
+                        bar_fn_arrive();
                         bar_n_helper();
                         const long long t_b = S2F_T();
-                        window_product<T, kC>(WR + c * ldr, ldr, Hc, ldh, c, c, c, 16, 8,
+                        window_product<T, kC>(WR + keep * ldr, ldr, Hc, ldh, c, c, c, 16, 8,
                                               [&](int r, int cc, T v) { WL[r * ldl + cc] = v; }, ht);
                         t_done = S2F_T();
-                        if (tid == kMain / 2) { S2F_ADD(3, t_ld - t_start); S2F_ADD(12, t_b - t_ld); S2F_ADD(4, t_done - t_b); }
+                        if (p > 0 && tid == kMain / 2) { S2F_ADD(3, t_ld - t_start); S2F_ADD(12, t_b - t_ld); S2F_ADD(4, t_done - t_b); }
                     } else {                      // helper: x' = column 0 of N * H  (LEFT(p)'s Householder vector)
                         bar_n_helper();
                         const long long t_b = S2F_T();
                         const int lane = tid & 31;
                         T xo[kC], yo[kC];
 #pragma unroll
-                        for (int k = 0; k < c; ++k) { xo[k] = WR[(c + lane) * ldr + k]; yo[k] = Hc[k * ldh]; }
+                        for (int k = 0; k < c; ++k) { xo[k] = WR[(keep + lane) * ldr + k]; yo[k] = Hc[k * ldh]; }
                         T acc = (T)0;
 #pragma unroll
                         for (int k = 0; k < c; ++k) acc = RN<T>::add(acc, RN<T>::mul(xo[k], yo[k]));
                         const long long t_x = S2F_T();
                         helper_reflector<T>(acc, xst, Hn, ldh, complete != 0);
                         t_done = S2F_T();
-                        if (tid == kMain) { S2F_ADD(6, t_b - t_start); S2F_ADD(13, t_x - t_b); S2F_ADD(5, t_done - t_x); }
+                        if (p > 0 && tid == kMain) { S2F_ADD(6, t_b - t_start); S2F_ADD(13, t_x - t_b); S2F_ADD(5, t_done - t_x); }
                     }
                     __syncthreads();
-                    if (tid == 0) { S2F_ADD(2, S2F_T() - t_done); S2F_ADD(8, S2F_T() - t_op0); }
+                    if (tm) { S2F_ADD(2, S2F_T() - t_done); S2F_ADD(8, S2F_T() - t_op0); }
                     { T* t = Hc; Hc = Hn; Hn = t; }
                     hready = true;
                 } else {
-                    // -------- generic path (top pair, clamped windows): the original kernel's code on the main threads
+                    // -------- generic path (clamped windows): the original kernel's code on the main threads
                     T nv[kNewPerThread];
                     const int newcnt = (nr - have) * nc;
                     if (have == 0) {
@@ -202,7 +234,6 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                         }
                     }
                     __syncthreads();
-                    const int keep = r1 - r0;
                     if (is_main)
                         window_product<T, kC>(WR, ldr, Hc, ldh, nr, nc, nc, (c + 1) / 2, (c + 1) / 2,
                                               [&](int r, int cc, T v) {
@@ -211,8 +242,9 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                                               }, tid);
                     __syncthreads();
                     hready = false;
+                    if (tid == rel_tid) st_release(&prog[i], q + 1);
                 }
-                if (tid == rel_tid) st_release(&prog[i], q + 1);
+                if (SVDB_S2_TIMING && tid == 0 && q < 4) S2F_ADD(16 + q, S2F_T() - t_start);
             }
             // ================= LEFT(p): rows [r1,r2) x cols [r1,c3), window = [F | N] ====================
             const int nn = c3 - r2;
@@ -221,6 +253,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                 const int q = 2 * p + 1;
                 if (i > 0 && tid == 0) seen = wait_progress(&prog[i - 1], q + 4, seen);
                 __syncthreads();
+                const long long t_start = S2F_T();
                 const int nr = r2 - r1, fc = r2 - r1, nc = fc + nn;
                 const bool interior = (nr == c) && (nn == c) && fwd;
                 if (interior) {
@@ -229,18 +262,15 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
 #pragma unroll
                         for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[(size_t)(r1 + (ht >> 5) + 4 * u) * N + (r2 + (ht & 31))]);
                     }
-                    if (!hready) {
-                        if (tid == 0) reflector_scalars<T>(WL, ldl, c, sc, complete != 0);
-                        __syncthreads();
-                        if (is_main) build_h<T>(WL, ldl, c, sc, Hc, ldh, tx, ty, tys);
-                        __syncthreads();
-                    }
                     if (f_warp) {                 // F half: finished cols [r1,r2) -> global
                         window_product<T, kC>(Hc, ldh, WL, ldl, c, c, c, 16, 8,
                                               [&](int r, int cc, T v) { st_cg(&A[(size_t)(r1 + r) * N + (r1 + cc)], v); }, tid);
+                        bar_fn_sync();
+                        if (tid == rel_tid) st_release(&prog[i], q + 1);
                     } else if (n_warp) {
 #pragma unroll
                         for (int u = 0; u < 8; ++u) WL[((ht >> 5) + 4 * u) * ldl + c + (ht & 31)] = nv[u];
+                        bar_fn_arrive();
                         bar_n_helper();
                         window_product<T, kC>(Hc, ldh, WL + c, ldl, c, c, c, 16, 8,
                                               [&](int r, int cc, T v) { WR[r * ldr + cc] = v; }, ht);
@@ -288,8 +318,9 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     fr = fwd ? nr : 0;
                     __syncthreads();
                     hready = false;
+                    if (tid == rel_tid && fwd) st_release(&prog[i], q + 1);
                 }
-                if (tid == rel_tid && fwd) st_release(&prog[i], q + 1);
+                if (SVDB_S2_TIMING && tid == 0 && q < 4) S2F_ADD(16 + q, S2F_T() - t_start);
             }
             if (!fwd) break;
         }
@@ -299,9 +330,9 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
 
 }  // namespace
 
-int stage2_fast_debug_read(long long* out16) {
-    long long z[16] = {};
-    if (cudaMemcpyFromSymbol(out16, g_s2f_dbg, sizeof(z)) != cudaSuccess) return 1;
+int stage2_fast_debug_read(long long* out24) {
+    long long z[kDbgSlots] = {};
+    if (cudaMemcpyFromSymbol(out24, g_s2f_dbg, sizeof(z)) != cudaSuccess) return 1;
     cudaMemcpyToSymbol(g_s2f_dbg, z, sizeof(z));
     return 0;
 }

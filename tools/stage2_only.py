@@ -41,14 +41,22 @@ if any(out):
     for i, nme in enumerate(names):
         print(f"  phase {i} {nme:44s} {out[i]:12d} cycles {100.0*out[i]/tot:5.1f}%")
 
-out = (ctypes.c_longlong * 16)()
+out = (ctypes.c_longlong * 24)()
 capi.lib().svdb200_debug_stage2_fast_timing(out)
 if any(out):
     cnt = max(out[7], 1)
-    names = {0: "thread 0: poll predecessor", 9: "barrier after poll", 11: "inline scalars + H (first interior op only)", 1: "F warps: product of the forwarded block",
+    names = {0: "thread 0: poll predecessor", 9: "barrier after poll", 1: "F warps: product of the forwarded block",
+             10: "F warps: wait for the N fetch at bar 2", 11: "release thread: op start .. release issued",
              2: "thread 0: wait at the closing barrier", 8: "whole op (thread 0)", 3: "N warps: fetch new block (issue .. stored)",
              12: "N warps: wait for helper at bar 1", 4: "N warps: product of the new block", 6: "helper: op start .. bar 1",
              13: "helper: 32 dot products (next Householder vector)", 5: "helper: sum of squares + scalars + H"}
-    print(f"  fast kernel, interior RIGHT ops of CTA 1: {cnt} ops ({out[10]} without a prepared H)")
+    print(f"  fast kernel, interior RIGHT ops (p > 0) of CTA 1: {cnt} ops")
     for k, nme in names.items():
         print(f"    {nme:52s} {out[k] / cnt:9.0f} cycles per op")
+    sw, heads = max(out[14], 1), max(out[22], 1)
+    print(f"  fast kernel, sweep heads of CTA 1: {out[14]} sweeps ({out[22]} with the head reflector prepared early)")
+    print(f"    {'thread 0: op-0 wait (predecessor >= 4 ops)':52s} {out[15] / sw:9.0f} cycles per sweep")
+    for q in range(4):
+        print(f"    {f'op {q} (after its wait .. closing barrier)':52s} {out[16 + q] / sw:9.0f} cycles per sweep")
+    print(f"    {'helper: head wait (predecessor >= 3 ops)':52s} {out[20] / heads:9.0f} cycles per prepared head")
+    print(f"    {'helper: head row load + scalars + H':52s} {out[21] / heads:9.0f} cycles per prepared head")
