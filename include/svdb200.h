@@ -84,6 +84,27 @@ int svdb200_band_to_bidiag_f64(svdb200_handle h, double* a, size_t m, size_t n, 
 int svdb200_band_to_bidiag_dev_f32(svdb200_handle h, float* a_dev, size_t m, size_t n, size_t band, float* d_dev, float* e_dev);
 int svdb200_band_to_bidiag_dev_f64(svdb200_handle h, double* a_dev, size_t m, size_t n, size_t band, double* d_dev, double* e_dev);
 
+/* Stage 2 and singular values of a band matrix in band storage: O(n band) device memory instead of n^2.
+ * ab is LAPACK's upper band storage (dgbbrd / dsbtrd AB(ku+1+i-j, j); scipy's `ab` form, transposed), column by column:
+ * ab[j*(band+1) + t] = A[j-band+t][j], t = 0..band, entries above the matrix ignored -- n x (band+1) elements, the layout
+ * svdb200_dist_gather_band_dev_* returns.  A LOWER band matrix is passed as its transpose (same singular values).  ab is
+ * const and not modified: it is copied into the handle's working buffer (max_n x 3 band elements, allocated on the first
+ * call, freed by svdb200_destroy), which holds the 3 band diagonals every window of the chase lies in.  The windows, the
+ * arithmetic and therefore d (n), e (n-1) are byte-identical to svdb200_band_to_bidiag_dev_* on the dense embedding of
+ * the band.  n >= 2 (else SVDB200_E_SHAPE), 1 <= band <= the handle's band and n <= max_n (else SVDB200_E_CAPACITY); band
+ * need not divide n.  The calls follow the handle's stage-2 schedule and singular-value method like svdb200_svdvals_*:
+ * for the singular values of a generic band matrix set svdb200_set_stage2_schedule(h, 1) first -- under the default
+ * (reference) schedule the un-chased last bulges leave sigma off by 1e-2 ... 1e-1 sigma_1.  Host-pointer variants copy ab
+ * in and d / e / sigma out inside the call and fill svdb200_last_timings (h2d, stage 2, qr, d2h). */
+int svdb200_band_to_bidiag_packed_f32(svdb200_handle h, const float* ab, size_t n, size_t band, float* d, float* e);
+int svdb200_band_to_bidiag_packed_f64(svdb200_handle h, const double* ab, size_t n, size_t band, double* d, double* e);
+int svdb200_band_to_bidiag_packed_dev_f32(svdb200_handle h, const float* ab_dev, size_t n, size_t band, float* d_dev, float* e_dev);
+int svdb200_band_to_bidiag_packed_dev_f64(svdb200_handle h, const double* ab_dev, size_t n, size_t band, double* d_dev, double* e_dev);
+int svdb200_band_svdvals_packed_f32(svdb200_handle h, const float* ab, size_t n, size_t band, float* sigma);
+int svdb200_band_svdvals_packed_f64(svdb200_handle h, const double* ab, size_t n, size_t band, double* sigma);
+int svdb200_band_svdvals_packed_dev_f32(svdb200_handle h, const float* ab_dev, size_t n, size_t band, float* sigma_dev);
+int svdb200_band_svdvals_packed_dev_f64(svdb200_handle h, const double* ab_dev, size_t n, size_t band, double* sigma_dev);
+
 /* ---- QR diagonalisation of the bidiagonal ----------------------------------------------------
  * Replaces csc586::serial::qrd<T> (svd_serial.h:368-422): Demmel-Kahan implicit zero-shift QR
  * sweeps (314-333) with the reference's convergence criteria (138-166), |sigma| sorted

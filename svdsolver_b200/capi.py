@@ -60,6 +60,20 @@ def _p(a):
 Z = ctypes.c_size_t
 
 
+def pack_upper_band(a, band):
+    """LAPACK upper band storage of the diagonals 0..band of a square matrix, column by column: ab[j, t] = a[j - band + t, j]
+    (zero above the matrix).  n x (band+1), the input of Handle.band_to_bidiag_packed / band_svdvals_packed; scipy's upper
+    `ab` (ab[band + i - j, j] = a[i, j]) transposed."""
+    a = np.asarray(a)
+    n = a.shape[0]
+    ab = np.zeros((n, band + 1), a.dtype)
+    for t in range(band + 1):
+        k = band - t                      # super-diagonal
+        if k < n:
+            ab[k:, t] = np.diagonal(a, k)
+    return ab
+
+
 class Handle:
     """svdb200_handle: workspace for matrices up to max_n x max_n with band `band`."""
 
@@ -117,6 +131,29 @@ class Handle:
         e = np.zeros(max(n - 1, 0), self.dtype)
         self._check(self._fn("band_to_bidiag")(self.h, _p(a), Z(a.shape[0]), Z(n), Z(band), _p(d), _p(e)))
         return a, d, e
+
+    def _band(self, ab, band):
+        ab = np.ascontiguousarray(ab, dtype=self.dtype)
+        if ab.ndim != 2 or ab.shape[1] != band + 1:
+            raise ValueError("band storage n x (band+1) expected")
+        return ab
+
+    def band_to_bidiag_packed(self, ab, band):
+        """stage 2 of the band matrix in upper band storage `ab` (pack_upper_band): returns (d, e); ab is not modified"""
+        ab = self._band(ab, band)
+        n = ab.shape[0]
+        d = np.zeros(n, self.dtype)
+        e = np.zeros(max(n - 1, 0), self.dtype)
+        self._check(self._fn("band_to_bidiag_packed")(self.h, _p(ab), Z(n), Z(band), _p(d), _p(e)))
+        return d, e
+
+    def band_svdvals_packed(self, ab, band):
+        """singular values (descending) of the band matrix in upper band storage `ab`; use set_stage2_schedule(1) for a
+        generic band matrix"""
+        ab = self._band(ab, band)
+        sigma = np.zeros(ab.shape[0], self.dtype)
+        self._check(self._fn("band_svdvals_packed")(self.h, _p(ab), Z(ab.shape[0]), Z(band), _p(sigma)))
+        return sigma
 
     def bidiag_qr(self, d, e):
         d = np.ascontiguousarray(d, dtype=self.dtype)
@@ -213,6 +250,12 @@ class Handle:
 
     def band_to_bidiag_dev(self, a_ptr, n, band, d_ptr, e_ptr):
         self._check(self._fn("band_to_bidiag_dev")(self.h, _p(a_ptr), Z(n), Z(n), Z(band), _p(d_ptr), _p(e_ptr)))
+
+    def band_to_bidiag_packed_dev(self, ab_ptr, n, band, d_ptr, e_ptr):
+        self._check(self._fn("band_to_bidiag_packed_dev")(self.h, _p(ab_ptr), Z(n), Z(band), _p(d_ptr), _p(e_ptr)))
+
+    def band_svdvals_packed_dev(self, ab_ptr, n, band, sigma_ptr):
+        self._check(self._fn("band_svdvals_packed_dev")(self.h, _p(ab_ptr), Z(n), Z(band), _p(sigma_ptr)))
 
     def bidiag_qr_dev(self, d_ptr, e_ptr, n, sigma_ptr):
         self._check(self._fn("bidiag_qr_dev")(self.h, _p(d_ptr), _p(e_ptr), Z(n), _p(sigma_ptr)))

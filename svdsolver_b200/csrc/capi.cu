@@ -654,6 +654,55 @@ int host_chain(Ctx* c, T* a, size_t n, size_t band, int order, int what, T* d, T
 
 size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Shape rules of stage 2 from band storage: those of svdb200_band_to_bidiag_dev_* (no m, band need not divide n)
+int check_packed(Ctx* c, size_t n, size_t band) {
+    if (n < 2) return SVDB200_E_SHAPE;
+    if (band == 0 || band > c->band || n > c->max_n) return SVDB200_E_CAPACITY;
+    return 0;
+}
+
+// Host-pointer stage 2 (sigma == nullptr: d / e out) or stage 2 + singular values from band storage, with the per-stage
+// timing of host_chain.  The n x (band+1) input is staged in a buffer of its own for the call.
+template <typename T>
+int packed_host(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e, T* sigma) {
+    T* abd = nullptr;
+    SVDB_CHECK(c, cudaMalloc(&abd, sizeof(T) * n * (band + 1)));
+    T* dd = reinterpret_cast<T*>(c->d);
+    T* ed = reinterpret_cast<T*>(c->e);
+    cudaStream_t s = c->stream;
+    long long info[3] = {0, 0, 0};
+    auto run = [&]() -> int {
+        SVDB_CHECK(c, cudaEventRecord(c->ev[0], s));
+        SVDB_CHECK(c, cudaMemcpyAsync(abd, ab, sizeof(T) * n * (band + 1), cudaMemcpyHostToDevice, s));
+        SVDB_CHECK(c, cudaEventRecord(c->ev[1], s));
+        SVDB_TRY(stage2_chase_packed<T>(c, abd, n, band, dd, ed));
+        SVDB_CHECK(c, cudaEventRecord(c->ev[2], s));
+        if (sigma) SVDB_TRY(bidiag_qr<T>(c, dd, ed, n, reinterpret_cast<T*>(c->sigma)));
+        SVDB_CHECK(c, cudaEventRecord(c->ev[3], s));
+        if (sigma) {
+            SVDB_CHECK(c, cudaMemcpyAsync(sigma, c->sigma, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
+            SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
+        } else {
+            if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, dd, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
+            if (e) SVDB_CHECK(c, cudaMemcpyAsync(e, ed, sizeof(T) * (n - 1), cudaMemcpyDeviceToHost, s));
+        }
+        SVDB_CHECK(c, cudaEventRecord(c->ev[4], s));
+        return 0;
+    };
+    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
+    const int st = run();
+    const cudaError_t se = cudaStreamSynchronize(s);
+    cudaFree(abd);
+    if (st != 0) return st;
+    if (se != cudaSuccess) return cuda_status(c, se, "cudaStreamSynchronize");
+    c->ms_h2d = elapsed(c->ev[0], c->ev[1]);
+    c->ms_stage2 = elapsed(c->ev[1], c->ev[2]);
+    c->ms_qr = elapsed(c->ev[2], c->ev[3]);
+    c->ms_d2h = elapsed(c->ev[3], c->ev[4]);
+    if (sigma && info[1] != 0) return SVDB200_E_NOCONV;
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -758,7 +807,8 @@ int svdb200_destroy(svdb200_handle h) {
     for (auto& ph : c->pool) if (ph) svdb200_destroy(reinterpret_cast<svdb200_handle>(ph));
     c->pool.clear();
     void* ptrs[] = {c->a_dev, c->v, c->v2, c->vb, c->v2b, c->w, c->wpart, c->s, c->tau, c->red, c->red2, c->chol_ws, c->bar, c->prog,
-                    c->d, c->e, c->sigma, c->qr_info, c->tileq, c->tilestate, c->tcsplit, c->bis_ws, c->batch_prog, c->batch_ws, c->de2};
+                    c->d, c->e, c->sigma, c->qr_info, c->tileq, c->tilestate, c->tcsplit, c->bis_ws, c->batch_prog, c->batch_ws, c->de2,
+                    c->band_ws};
     for (int k = 1; k < 2 * Ctx::kLanes; ++k) if (c->a_stage[k]) cudaFree(c->a_stage[k]);
     for (int l = 0; l < Ctx::kLanes; ++l) if (c->s1ctx[l]) svdb200_destroy(reinterpret_cast<svdb200_handle>(c->s1ctx[l]));
     for (int l = 1; l < Ctx::kLanes; ++l) if (c->s2_prog[l]) cudaFree(c->s2_prog[l]);
@@ -820,6 +870,33 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
         if (band == 0 || band > c->band) return SVDB200_E_CAPACITY;                                                      \
         return stage2_chase<T>(c, a, n, band, d, e);                                                                     \
+    }                                                                                                                    \
+    int svdb200_band_to_bidiag_packed_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* d, T* e) {            \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!ab) return SVDB200_E_ARG;                                                                                   \
+        SVDB_TRY(check_packed(c, n, band));                                                                              \
+        return packed_host<T>(c, ab, n, band, d, e, nullptr);                                                            \
+    }                                                                                                                    \
+    int svdb200_band_to_bidiag_packed_dev_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* d, T* e) {        \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!ab) return SVDB200_E_ARG;                                                                                   \
+        SVDB_TRY(check_packed(c, n, band));                                                                              \
+        return stage2_chase_packed<T>(c, ab, n, band, d, e);                                                             \
+    }                                                                                                                    \
+    int svdb200_band_svdvals_packed_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* sigma) {                \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!ab || !sigma) return SVDB200_E_ARG;                                                                         \
+        SVDB_TRY(check_packed(c, n, band));                                                                              \
+        return packed_host<T>(c, ab, n, band, nullptr, nullptr, sigma);                                                  \
+    }                                                                                                                    \
+    int svdb200_band_svdvals_packed_dev_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* sigma) {            \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!ab || !sigma) return SVDB200_E_ARG;                                                                         \
+        SVDB_TRY(check_packed(c, n, band));                                                                              \
+        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
+        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
+        SVDB_TRY(stage2_chase_packed<T>(c, ab, n, band, dd, ed));                                                        \
+        return bidiag_qr<T>(c, dd, ed, n, sigma);                                                                        \
     }                                                                                                                    \
     int svdb200_bidiag_qr_##S(svdb200_handle h, const T* d, const T* e, size_t n, T* sigma, long long* sweeps) {         \
         SVDB_ENTER(T)                                                                                                    \

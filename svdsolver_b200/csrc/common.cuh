@@ -52,6 +52,7 @@ struct Ctx {
     void* red2 = nullptr;          // blocked panel kernel: flag-stamped words exchanged between clusters through L2 (512 KB)
     unsigned int* bar = nullptr;   // software grid barrier state (2 words) + misc counters
     int* prog = nullptr;           // stage-2 per-sweep progress counters (max_n)
+    void* band_ws = nullptr;       // max_n * 3 band: stage 2 from band storage, packed 3-band-diagonal layout (first use)
     void* d = nullptr; void* e = nullptr; void* sigma = nullptr;   // max_n each
     long long* qr_info = nullptr;  // [0] sweeps, [1] status
     void* tileq = nullptr;         // tile order: per-chain-step Q matrices, (max_n/band) * 4*band*band
@@ -205,7 +206,8 @@ __device__ __forceinline__ void grid_barrier(unsigned* bar, unsigned nctas, unsi
 // ---- internal entry points (one per .cu) ----------------------------------------------------------
 template <typename T> int stage2_chase(Ctx* c, T* a, size_t n, size_t band, T* d, T* e);
 template <typename T> int extract_bidiagonal(Ctx* c, const T* a, size_t n, T* d, T* e);
-template <typename T> int stage2_chase_fast(Ctx* c, T* a, size_t n, size_t band, int* prog);   // 0 ran, 1 shape not covered
+template <typename T> int stage2_chase_packed(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e);   // ab: LAPACK upper band storage
+template <typename T, bool kPacked> int stage2_chase_fast(Ctx* c, T* a, size_t n, size_t band, int* prog);   // 0 ran, 1 shape not covered
 template <typename T> int bidiag_qr(Ctx* c, T* d, T* e, size_t n, T* sigma);
 template <typename T> int bidiag_bisect(Ctx* c, const T* d, const T* e, size_t n, T* sigma);
 template <typename T> int bidiag_sqr(Ctx* c, T* d, T* e, size_t n, T* sigma);

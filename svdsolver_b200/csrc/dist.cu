@@ -90,7 +90,6 @@ struct Dist {
     void* vv = nullptr;          // [V | V S^T] of a QR panel, contiguous (2 x n x band): ONE broadcast per panel
     void* bandsend = nullptr;    // ncl_max x (band+1) : this rank's band columns, packed
     void* bandall = nullptr;     // nranks x ncl_max x (band+1) : all-gather landing zone
-    void* dense = nullptr;       // rank 0, svdvals only: n x n staging for stage 2 (allocated on first use)
     double* lqbuf = nullptr;     // distributed LQ panel: [tile-packed Gram matrix | top block], all-reduced in double
     int lq_dist = 1;             // 1: LQ panels by local Gram matrix + all-reduce (no gather of the row panel); 0: gather + redundant panel
     int* h_status = nullptr;     // pinned: [0..3] status words of the last distributed LQ panel, [8..11] of the last QR panel
@@ -190,16 +189,6 @@ __global__ void unpack_band_global_kernel(const T* __restrict__ gathered, size_t
     const int r = (int)(gb % P);
     const size_t lc = (gb / P) * b + gc % b;
     packed[e] = gathered[((size_t)r * ncl_max + lc) * (b + 1) + t];
-}
-// packed band -> dense n x n (zero elsewhere)
-template <typename T>
-__global__ void band_to_dense_kernel(const T* __restrict__ packed, size_t n, int b, T* __restrict__ dense) {
-    const size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n * (size_t)(b + 1)) return;
-    const size_t gc = e / (b + 1);
-    const int t = (int)(e - gc * (b + 1));
-    const long long row = (long long)gc - b + t;
-    if (row >= 0) dense[(size_t)row * n + gc] = packed[e];
 }
 
 // Look-ahead (same scheme as the single-GPU driver, stage1_panel.cu): the part of an update that the NEXT panel lives in
@@ -445,28 +434,19 @@ int dist_gather_band(Dist* d, const T* a, T* packed) {
     return 0;
 }
 
-// stage 1 distributed, then the band goes to rank 0, which runs stage 2 and the singular values (replicas only there:
-// one sequential wavefront over an O(n b) band, SURVEY 8e)
+// stage 1 distributed, then the band goes to rank 0, which runs stage 2 on the packed band and the singular values
+// (replicas only there: one sequential wavefront over an O(n b) band, SURVEY 8e)
 template <typename T>
 int dist_svdvals(Dist* d, T* a, T* sigma) {
     Ctx* c = d->ctx;
     const size_t n = d->n, band = d->band;
     SVDB_TRY(dist_stage1<T>(d, a, n, band));
-    if (!d->dense && d->rank == 0) SVDB_CHECK(c, cudaMalloc(&d->dense, sizeof(T) * n * n));
     void* pk = nullptr;
     SVDB_CHECK(c, cudaMalloc(&pk, sizeof(T) * n * (band + 1)));
     T* packed = reinterpret_cast<T*>(pk);
     int st = dist_gather_band<T>(d, a, packed);
     if (st == 0 && d->rank == 0) {
-        T* dense = reinterpret_cast<T*>(d->dense);
-        cudaError_t e = cudaMemsetAsync(dense, 0, sizeof(T) * n * n, c->stream);
-        if (e != cudaSuccess) st = cuda_status(c, e, "cudaMemsetAsync(dense)");
-        if (st == 0) {
-            const size_t tot = n * (band + 1);
-            band_to_dense_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, c->stream>>>(packed, n, (int)band, dense);
-            c->launches++;
-            st = stage2_chase<T>(c, dense, n, band, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e));
-        }
+        st = stage2_chase_packed<T>(c, packed, n, band, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e));
         if (st == 0) st = bidiag_qr<T>(c, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), n, sigma);
     }
     cudaStreamSynchronize(c->stream);
@@ -549,7 +529,7 @@ int svdb200_dist_destroy(svdb200_dist_handle h) {
     Dist* d = reinterpret_cast<Dist*>(h);
     if (d->ctx) { cudaSetDevice(d->ctx->device); cudaStreamSynchronize(d->ctx->stream); }
     if (d->comm) nccl().CommDestroy(d->comm);
-    void* ptrs[] = {d->rowpanel, d->gather, d->sendbuf, d->ut_loc, d->u2_loc, d->vv, d->bandsend, d->bandall, d->dense, d->lqbuf, d->qsend};
+    void* ptrs[] = {d->rowpanel, d->gather, d->sendbuf, d->ut_loc, d->u2_loc, d->vv, d->bandsend, d->bandall, d->lqbuf, d->qsend};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (d->h_status) cudaFreeHost(d->h_status);
     if (d->ev_status) cudaEventDestroy(d->ev_status);

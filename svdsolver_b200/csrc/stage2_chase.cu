@@ -41,7 +41,8 @@ __device__ long long g_s2_dbg[16];
 using namespace s2;
 
 // kC: the band as a compile-time constant (32 / 64: the sizes the configs use), 0 = any band at run time
-template <typename T, int kMaxThreads, int kMinBlocks, int kC>
+// kPacked: the matrix is held in the packed 3c-diagonal layout (Layout, stage2_common.cuh); single matrix only
+template <typename T, int kMaxThreads, int kMinBlocks, int kC, bool kPacked>
 __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T* __restrict__ A0, int n, int band, int* __restrict__ prog0,
                                                                       int count, int G, int complete) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -53,6 +54,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
     T* sc = H + c * ldh;                        // alpha, tau
     const int tid = threadIdx.x, nt = blockDim.x;
     const size_t N = (size_t)n;
+    const Layout<kPacked, kC> at = make_layout<kPacked, kC>(n, c);
     const int tx = tid % c, ty = tid / c, tys = nt / c;   // 2-D view of the CTA: c columns x tys rows (nt >= c)
 
     // Batched use: the grid is split into groups of G CTAs; a group pipelines the sweeps of one matrix at a time
@@ -93,13 +95,13 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
                 const int newcnt = (nr - have) * nc;
                 if (have == 0) {                  // top pair: the whole window (x included) comes from L2
                     for (int e = tid; e < newcnt; e += nt)
-                        WR[(e / nc) * ldr + e % nc] = ld_cg(&A[(size_t)(r0 + e / nc) * N + (r1 + e % nc)]);
+                        WR[(e / nc) * ldr + e % nc] = ld_cg(&A[at(r0 + e / nc, r1 + e % nc)]);
                     __syncthreads();
                 } else {                          // issue the fetch of N, consume it after H is built
 #pragma unroll
                     for (int u = 0; u < kNewPerThread; ++u) {
                         int r = ty + u * tys;
-                        if (r < nr - have && tx < nc) nv[u] = ld_cg(&A[(size_t)(r0 + have + r) * N + (r1 + tx)]);
+                        if (r < nr - have && tx < nc) nv[u] = ld_cg(&A[at(r0 + have + r, r1 + tx)]);
                     }
                 }
                 S2_TICK(3);
@@ -120,7 +122,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
                 const int keep = r1 - r0;
                 window_product<T, kC>(WR, ldr, H, ldh, nr, nc, nc, (c + 1) / 2, (c + 1) / 2,
                                   [&](int r, int cc, T v) {
-                                      if (r < keep) st_cg(&A[(size_t)(r0 + r) * N + (r1 + cc)], v);
+                                      if (r < keep) st_cg(&A[at(r0 + r, r1 + cc)], v);
                                       else WL[(r - keep) * ldl + cc] = v;
                                   }, tid);
                 S2_TICK(6);
@@ -142,7 +144,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
 #pragma unroll
                 for (int u = 0; u < kNewPerThread; ++u) {
                     int r = ty + u * tys;
-                    if (r < nr && tx < nn) nv[u] = ld_cg(&A[(size_t)(r1 + r) * N + (r2 + tx)]);
+                    if (r < nr && tx < nn) nv[u] = ld_cg(&A[at(r1 + r, r2 + tx)]);
                 }
                 if (tid == 0) reflector_scalars<T>(WL, ldl, nr, sc, complete != 0);
                 __syncthreads();
@@ -156,7 +158,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
                 // cols [r1,r2) are finished; cols [r2,c3) become the top block of RIGHT(p+1)
                 window_product<T, kC>(H, ldh, WL, ldl, nr, nc, nr, c, (c + 3) / 4,
                                   [&](int r, int cc, T v) {
-                                      if (cc < fc || !fwd) st_cg(&A[(size_t)(r1 + r) * N + (r1 + cc)], v);
+                                      if (cc < fc || !fwd) st_cg(&A[at(r1 + r, r1 + cc)], v);
                                       else WR[r * ldr + (cc - fc)] = v;
                                   }, tid);
                 fr = fwd ? nr : 0;
@@ -179,22 +181,34 @@ int stage2_debug_read(long long* out16) {
 }
 namespace {
 
-template <typename T>
-__global__ void extract_bidiagonal_kernel(const T* __restrict__ A, int n, T* __restrict__ d, T* __restrict__ e) {
+template <typename T, bool kPacked>
+__global__ void extract_bidiagonal_kernel(const T* __restrict__ A, int n, int band, T* __restrict__ d, T* __restrict__ e) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    A += (size_t)blockIdx.y * n * n;                 // batched: one matrix per blockIdx.y, d/e rows of length n
+    const Layout<kPacked> at = make_layout<kPacked>(n, band);
+    A += (size_t)blockIdx.y * n * n;                 // batched (dense only): one matrix per blockIdx.y, d/e rows of length n
     if (d) d += (size_t)blockIdx.y * n;
     if (e) e += (size_t)blockIdx.y * n;
     if (i < n) {
-        if (d) d[i] = A[(size_t)i * n + i];
-        if (e && i + 1 < n) e[i] = A[(size_t)i * n + i + 1];
+        if (d) d[i] = A[at(i, i)];
+        if (e && i + 1 < n) e[i] = A[at(i, i + 1)];
     }
 }
 
-}  // namespace
-
+// LAPACK upper band storage (n x (b+1), ab[j*(b+1) + t] = A[j-b+t][j]) -> the packed working layout of the chase (row r
+// holds columns r-b+1 .. r+2b); every entry outside the input's b+1 diagonals starts as zero, as in the dense array
 template <typename T>
-int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
+__global__ void pack_band_kernel(const T* __restrict__ ab, int n, int b, T* __restrict__ w) {
+    const size_t ld = (size_t)3 * b, total = (size_t)n * ld;
+    for (size_t x = (size_t)blockIdx.x * blockDim.x + threadIdx.x; x < total; x += (size_t)gridDim.x * blockDim.x) {
+        const int r = (int)(x / ld), k = (int)(x - (size_t)r * ld);
+        const int off = k - (b - 1), col = r + off;  // off = col - r, the super-diagonal
+        w[x] = (off >= 0 && off <= b && col < n) ? ab[(size_t)col * (b + 1) + (b - off)] : (T)0;
+    }
+}
+
+// Stage 2 of `count` dense matrices (count > 1: back to back, n x n each), or of ONE matrix in the packed layout
+template <typename T, bool kPacked>
+int stage2_run(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
     if (n < 2 || band < 1 || count < 1) return SVDB200_E_SHAPE;
     if (n > (size_t)INT_MAX / 4) return SVDB200_E_CAPACITY;
     const int cb = (int)band;
@@ -206,11 +220,12 @@ int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int co
     if (smem > 227 * 1024) return SVDB200_E_CAPACITY;
     // small bands run with <= 256 threads: instantiate that case without the 64-register cap; a batch wants
     // several CTAs per SM instead (the window product is FP64-issue bound for ~40 % of an op, the rest is latency)
-    const bool light = count > 1;
-    auto kern = nt <= 256 ? (light ? stage2_chase_kernel<T, 256, 3, 0> : stage2_chase_kernel<T, 256, 1, 0>)
-                          : stage2_chase_kernel<T, 1024, 1, 0>;
-    if (cb == 32) kern = light ? stage2_chase_kernel<T, 256, 3, 32> : stage2_chase_kernel<T, 256, 1, 32>;   // band-specialised
-    else if (cb == 64) kern = stage2_chase_kernel<T, 1024, 1, 64>;                                           // (same arithmetic)
+    auto kern = nt <= 256 ? stage2_chase_kernel<T, 256, 1, 0, kPacked> : stage2_chase_kernel<T, 1024, 1, 0, kPacked>;
+    if (cb == 32) kern = stage2_chase_kernel<T, 256, 1, 32, kPacked>;          // band-specialised
+    else if (cb == 64) kern = stage2_chase_kernel<T, 1024, 1, 64, kPacked>;    // (same arithmetic)
+    if constexpr (!kPacked) {
+        if (count > 1 && nt <= 256) kern = cb == 32 ? stage2_chase_kernel<T, 256, 3, 32, false> : stage2_chase_kernel<T, 256, 3, 0, false>;
+    }
     SVDB_CHECK(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     SVDB_CHECK(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nt, smem));
@@ -239,7 +254,7 @@ int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int co
     int ni = (int)n, bi = cb, cnt = count, gi = (int)G, complete = c->cfg.stage2_complete;
     int fast = 1;                                                      // 0 = the latency-optimised band-32 kernel ran
     if (count == 1) {
-        fast = stage2_chase_fast<T>(c, a, n, band, prog);
+        fast = stage2_chase_fast<T, kPacked>(c, a, n, band, prog);
         if (fast != 0 && fast != 1) return fast;
     }
     if (fast != 0) {
@@ -248,11 +263,32 @@ int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int co
         c->launches++;
     }
     if (d || e) {
-        extract_bidiagonal_kernel<T><<<dim3((unsigned)((n + 255) / 256), (unsigned)count), 256, 0, c->stream>>>(a, ni, d, e);
+        extract_bidiagonal_kernel<T, kPacked><<<dim3((unsigned)((n + 255) / 256), (unsigned)count), 256, 0, c->stream>>>(a, ni, cb, d, e);
         SVDB_CHECK(c, cudaGetLastError());
         c->launches++;
     }
     return 0;
+}
+
+}  // namespace
+
+template <typename T>
+int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) { return stage2_run<T, false>(c, a, n, band, d, e, count); }
+
+// Stage 2 of a band matrix given in LAPACK upper band storage: packed into the handle's working buffer (max_n x 3 band,
+// allocated on first use) and chased there; `ab` is not modified.
+template <typename T>
+int stage2_chase_packed(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e) {
+    if (n < 2 || band < 1) return SVDB200_E_SHAPE;
+    if (n > c->max_n || band > c->band) return SVDB200_E_CAPACITY;
+    if (!c->band_ws) SVDB_CHECK(c, cudaMalloc(&c->band_ws, c->esz * c->max_n * 3 * c->band));
+    T* w = reinterpret_cast<T*>(c->band_ws);
+    const size_t total = n * 3 * band;
+    const unsigned blocks = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)c->num_sms * 16);
+    pack_band_kernel<T><<<blocks, 256, 0, c->stream>>>(ab, (int)n, (int)band, w);
+    SVDB_CHECK(c, cudaGetLastError());
+    c->launches++;
+    return stage2_run<T, true>(c, w, n, band, d, e, 1);
 }
 
 template <typename T>
@@ -262,7 +298,7 @@ int stage2_chase(Ctx* c, T* a, size_t n, size_t band, T* d, T* e) { return stage
 template <typename T>
 int extract_bidiagonal(Ctx* c, const T* a, size_t n, T* d, T* e) {
     if (!d && !e) return 0;
-    extract_bidiagonal_kernel<T><<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(a, (int)n, d, e);
+    extract_bidiagonal_kernel<T, false><<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(a, (int)n, 1, d, e);
     SVDB_CHECK(c, cudaGetLastError());
     c->launches++;
     return 0;
@@ -274,5 +310,7 @@ template int stage2_chase_batched<float>(Ctx*, float*, size_t, size_t, float*, f
 template int stage2_chase_batched<double>(Ctx*, double*, size_t, size_t, double*, double*, int);
 template int stage2_chase<float>(Ctx*, float*, size_t, size_t, float*, float*);
 template int stage2_chase<double>(Ctx*, double*, size_t, size_t, double*, double*);
+template int stage2_chase_packed<float>(Ctx*, const float*, size_t, size_t, float*, float*);
+template int stage2_chase_packed<double>(Ctx*, const double*, size_t, size_t, double*, double*);
 
 }  // namespace svdb200

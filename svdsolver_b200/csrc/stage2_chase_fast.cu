@@ -97,7 +97,8 @@ __device__ __forceinline__ void helper_reflector(T xv, T* __restrict__ xst, T* _
     __syncwarp();
 }
 
-template <typename T>
+// kPacked: the matrix is held in the packed 3c-diagonal layout (Layout, stage2_common.cuh)
+template <typename T, bool kPacked>
 __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restrict__ A, int n, int* __restrict__ prog, int complete) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int c = kC, w = c + 1;
@@ -111,7 +112,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
     const int tid = threadIdx.x;
     const bool is_main = tid < kMain, is_helper = !is_main;
     const bool f_warp = tid < kMain / 2, n_warp = is_main && !f_warp;
-    const size_t N = (size_t)n;
+    const Layout<kPacked, kC> at = make_layout<kPacked, kC>(n, kC);
     const int tx = tid % c, ty = tid / c;       // generic path: c columns x tys rows of main threads
     constexpr int tys = kMain / c;
     const int ht = tid - kMain / 2;             // N warps: 0..127
@@ -136,7 +137,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                 __syncwarp();
             }
             const long long t_h1 = S2F_T();
-            const T xv = ld_cg(&A[(size_t)i * N + (i + 1 + lane)]);
+            const T xv = ld_cg(&A[at(i, i + 1 + lane)]);
             WR[lane] = xv;
             helper_reflector<T>(xv, xst, Hc, ldh, complete != 0);
             if (tid == kMain) { S2F_ADD(20, t_h1 - t_h0); S2F_ADD(21, S2F_T() - t_h1); }
@@ -163,12 +164,12 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     T nv[8];
                     if (n_warp) {                 // new block: rows [keep, keep+c) of the window, 8 elements per thread
 #pragma unroll
-                        for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[(size_t)(r1 + (ht >> 5) + 4 * u) * N + (r1 + (ht & 31))]);
+                        for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[at(r1 + (ht >> 5) + 4 * u, r1 + (ht & 31))]);
                     }
                     long long t_done = 0;
                     if (f_warp) {                 // F half: finished rows [r0,r1) -> global
                         window_product<T, kC>(WR, ldr, Hc, ldh, keep, c, c, 16, 8,
-                                              [&](int r, int cc, T v) { st_cg(&A[(size_t)(r0 + r) * N + (r1 + cc)], v); }, tid);
+                                              [&](int r, int cc, T v) { st_cg(&A[at(r0 + r, r1 + cc)], v); }, tid);
                         t_done = S2F_T();
                         bar_fn_sync();
                         const long long t_rel = S2F_T();
@@ -212,13 +213,13 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     if (have == 0) {
                         if (is_main)
                             for (int e = tid; e < newcnt; e += kMain)
-                                WR[(e / nc) * ldr + e % nc] = ld_cg(&A[(size_t)(r0 + e / nc) * N + (r1 + e % nc)]);
+                                WR[(e / nc) * ldr + e % nc] = ld_cg(&A[at(r0 + e / nc, r1 + e % nc)]);
                         __syncthreads();
                     } else if (is_main) {
 #pragma unroll
                         for (int u = 0; u < kNewPerThread; ++u) {
                             int r = ty + u * tys;
-                            if (r < nr - have && tx < nc) nv[u] = ld_cg(&A[(size_t)(r0 + have + r) * N + (r1 + tx)]);
+                            if (r < nr - have && tx < nc) nv[u] = ld_cg(&A[at(r0 + have + r, r1 + tx)]);
                         }
                     }
                     if (!hready && tid == 0) reflector_scalars<T>(WR, 1, nc, sc, complete != 0);
@@ -237,7 +238,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     if (is_main)
                         window_product<T, kC>(WR, ldr, Hc, ldh, nr, nc, nc, (c + 1) / 2, (c + 1) / 2,
                                               [&](int r, int cc, T v) {
-                                                  if (r < keep) st_cg(&A[(size_t)(r0 + r) * N + (r1 + cc)], v);
+                                                  if (r < keep) st_cg(&A[at(r0 + r, r1 + cc)], v);
                                                   else WL[(r - keep) * ldl + cc] = v;
                                               }, tid);
                     __syncthreads();
@@ -260,11 +261,11 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     T nv[8];
                     if (n_warp) {                 // new block: cols [c,2c) of the window
 #pragma unroll
-                        for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[(size_t)(r1 + (ht >> 5) + 4 * u) * N + (r2 + (ht & 31))]);
+                        for (int u = 0; u < 8; ++u) nv[u] = ld_cg(&A[at(r1 + (ht >> 5) + 4 * u, r2 + (ht & 31))]);
                     }
                     if (f_warp) {                 // F half: finished cols [r1,r2) -> global
                         window_product<T, kC>(Hc, ldh, WL, ldl, c, c, c, 16, 8,
-                                              [&](int r, int cc, T v) { st_cg(&A[(size_t)(r1 + r) * N + (r1 + cc)], v); }, tid);
+                                              [&](int r, int cc, T v) { st_cg(&A[at(r1 + r, r1 + cc)], v); }, tid);
                         bar_fn_sync();
                         if (tid == rel_tid) st_release(&prog[i], q + 1);
                     } else if (n_warp) {
@@ -295,7 +296,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
 #pragma unroll
                         for (int u = 0; u < kNewPerThread; ++u) {
                             int r = ty + u * tys;
-                            if (r < nr && tx < nn) nv[u] = ld_cg(&A[(size_t)(r1 + r) * N + (r2 + tx)]);
+                            if (r < nr && tx < nn) nv[u] = ld_cg(&A[at(r1 + r, r2 + tx)]);
                         }
                     }
                     if (!hready && tid == 0) reflector_scalars<T>(WL, ldl, nr, sc, complete != 0);
@@ -312,7 +313,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) stage2_fast_kernel(T* __restr
                     if (is_main)
                         window_product<T, kC>(Hc, ldh, WL, ldl, nr, nc, nr, c, (c + 3) / 4,
                                               [&](int r, int cc, T v) {
-                                                  if (cc < fc || !fwd) st_cg(&A[(size_t)(r1 + r) * N + (r1 + cc)], v);
+                                                  if (cc < fc || !fwd) st_cg(&A[at(r1 + r, r1 + cc)], v);
                                                   else WR[r * ldr + (cc - fc)] = v;
                                               }, tid);
                     fr = fwd ? nr : 0;
@@ -338,11 +339,11 @@ int stage2_fast_debug_read(long long* out24) {
 }
 
 // returns 0 when it ran, 1 when the shape is outside this kernel's range (the caller runs stage2_chase_kernel)
-template <typename T>
+template <typename T, bool kPacked>
 int stage2_chase_fast(Ctx* c, T* a, size_t n, size_t band, int* prog) {
     if (band != (size_t)kC || n < 2 * band + 2) return 1;
     const size_t smem = (size_t)(2 * kC * (kC + 1) + kC * (2 * kC + 1) + 2 * kC * (kC + 1) + 8 + kC + 8) * sizeof(T);
-    auto kern = stage2_fast_kernel<T>;
+    auto kern = stage2_fast_kernel<T, kPacked>;
     SVDB_CHECK(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     SVDB_CHECK(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kFastThreads, smem));
@@ -356,7 +357,9 @@ int stage2_chase_fast(Ctx* c, T* a, size_t n, size_t band, int* prog) {
     c->launches++;
     return 0;
 }
-template int stage2_chase_fast<float>(Ctx*, float*, size_t, size_t, int*);
-template int stage2_chase_fast<double>(Ctx*, double*, size_t, size_t, int*);
+template int stage2_chase_fast<float, false>(Ctx*, float*, size_t, size_t, int*);
+template int stage2_chase_fast<double, false>(Ctx*, double*, size_t, size_t, int*);
+template int stage2_chase_fast<float, true>(Ctx*, float*, size_t, size_t, int*);
+template int stage2_chase_fast<double, true>(Ctx*, double*, size_t, size_t, int*);
 
 }  // namespace svdb200

@@ -13,6 +13,27 @@ namespace s2 {
 // most two) distinct X rows of a warp in different banks.
 constexpr int kTileR = 4, kTileC = 2, kNewPerThread = 4;
 
+// Where element (r, col) of the matrix being chased lives (DESIGN §3.4c).  Dense: row-major n x n, r*n + col.  Packed:
+// the 3c diagonals -(c-1) .. 2c-1 that every window of either schedule lies in, row-major with 3c entries per row,
+// r*3c + col - r + c - 1.  A window row segment is contiguous in both.  kC > 0: the band as a compile-time constant.
+template <bool kPacked, int kC = 0>
+struct Layout {
+    size_t ld;      // elements per row: n (dense) or 3c (packed)
+    int c;
+    __device__ __forceinline__ size_t operator()(int r, int col) const {
+        if constexpr (kPacked) {
+            const int cc = kC > 0 ? kC : c;
+            return (size_t)r * (size_t)(3 * cc - 1) + (size_t)(col + cc - 1);      // = r*3c + (col - r + c - 1)
+        } else {
+            return (size_t)r * ld + col;
+        }
+    }
+};
+template <bool kPacked, int kC = 0>
+__host__ __device__ __forceinline__ Layout<kPacked, kC> make_layout(int n, int c) {
+    return Layout<kPacked, kC>{kPacked ? (size_t)3 * c : (size_t)n, c};
+}
+
 __host__ __device__ inline int stage2_threads(int c) {
     int ct = (c + 1) / 2;
     int need = ct * ct;                         // RIGHT: CT = RT = ceil(c/2); LEFT: CT = c, RT = ceil(c/4)
