@@ -8,7 +8,8 @@
  *
  * Conventions
  *   - matrices are square n x n, dense ROW-MAJOR (what Matrix::flatten() yields, matrix.h:258,
- *     svd_cuda_2.cu:549), band | n, updated in place unless stated;
+ *     svd_cuda_2.cu:549), band | n, updated in place unless stated; the *_mn calls take
+ *     rectangular m x n matrices (band | min(m, n));
  *   - every function returns an int status: 0 ok, <0 argument/shape error (SVDB200_E_*),
  *     >0 a CUDA / NCCL error code offset by SVDB200_CUDA_ERR / SVDB200_NCCL_ERR;
  *     no exceptions cross this boundary (the reference assert()s and ignores CUDA errors);
@@ -42,7 +43,8 @@ enum { SVDB200_ORDER_PANEL = 0, SVDB200_ORDER_TILE = 1 };
 enum {
     SVDB200_OK = 0,
     SVDB200_E_ARG = -1,        /* null pointer / bad enum */
-    SVDB200_E_SHAPE = -2,      /* m != n, band == 0, n % band != 0 (matrix.h:407 needs t | n) */
+    SVDB200_E_SHAPE = -2,      /* square calls: m != n, band == 0, n % band != 0 (matrix.h:407 needs t | n);
+                                  m x n calls (*_mn): min(m, n) < 2, band == 0, min(m, n) % band != 0 */
     SVDB200_E_CAPACITY = -3,   /* exceeds what the handle was created for / what the kernel supports */
     SVDB200_E_NODEVICE = -4,   /* no usable CUDA device: there is no CPU fallback */
     SVDB200_E_NOCONV = -5,     /* QR diagonalisation hit max_iter (svd_serial.h:419) */
@@ -157,6 +159,34 @@ int svdb200_svdvals_f32(svdb200_handle h, float* a, size_t m, size_t n, size_t b
 int svdb200_svdvals_f64(svdb200_handle h, double* a, size_t m, size_t n, size_t band, int order, double* sigma);
 int svdb200_svdvals_dev_f32(svdb200_handle h, float* a_dev, size_t m, size_t n, size_t band, int order, float* sigma_dev);
 int svdb200_svdvals_dev_f64(svdb200_handle h, double* a_dev, size_t m, size_t n, size_t band, int order, double* sigma_dev);
+
+/* ---- Rectangular m x n matrices (tall m > n and wide m < n; m == n allowed) -------------------------------------------
+ * The panel order on A (m >= n) or on A^T (m < n): sigma(A) = sigma(A^T).  LAPACK gebrd's convention: `a` (m x n,
+ * row-major) is overwritten by the reduced matrix in A's own shape -- for m >= n an upper band (dense_to_band_mn) or upper
+ * bidiagonal matrix in the top n x n block with the rows below it zero; for m < n a LOWER band / bidiagonal matrix in the
+ * left m x m block with the columns right of it zero.  d has min(m, n) entries, e min(m, n) - 1: the super-diagonal for
+ * m >= n, the sub-diagonal for m < n.  sigma (min(m, n)) is descending.  With m == n each call returns byte for byte what
+ * svdb200_dense_to_band_* / svdb200_bidiagonalize_* / svdb200_svdvals_* return with SVDB200_ORDER_PANEL.
+ * Statuses: SVDB200_E_ARG for a null pointer or a dtype mismatch; SVDB200_E_SHAPE when min(m, n) < 2, band == 0 or band
+ * does not divide min(m, n) (the longer side is arbitrary); SVDB200_E_CAPACITY when max(m, n) > max_n or band > the
+ * handle's band.  Stage 2 and the singular values follow the handle's stage-2 schedule and singular-value method like
+ * svdb200_svdvals_*: for the singular values of a generic matrix set svdb200_set_stage2_schedule(h, 1) first.
+ * A wide matrix is transposed into a scratch buffer of the handle (m * n elements, allocated on the first wide call,
+ * grown when a larger wide matrix arrives, freed by svdb200_destroy), reduced there and transposed back.  Host-pointer
+ * variants stage through the handle's max_n^2 buffer and fill svdb200_last_timings, with both transposes counted in
+ * stage 1. */
+int svdb200_dense_to_band_mn_f32(svdb200_handle h, float* a, size_t m, size_t n, size_t band);
+int svdb200_dense_to_band_mn_f64(svdb200_handle h, double* a, size_t m, size_t n, size_t band);
+int svdb200_dense_to_band_mn_dev_f32(svdb200_handle h, float* a_dev, size_t m, size_t n, size_t band);
+int svdb200_dense_to_band_mn_dev_f64(svdb200_handle h, double* a_dev, size_t m, size_t n, size_t band);
+int svdb200_bidiagonalize_mn_f32(svdb200_handle h, float* a, size_t m, size_t n, size_t band, float* d, float* e);
+int svdb200_bidiagonalize_mn_f64(svdb200_handle h, double* a, size_t m, size_t n, size_t band, double* d, double* e);
+int svdb200_bidiagonalize_mn_dev_f32(svdb200_handle h, float* a_dev, size_t m, size_t n, size_t band, float* d_dev, float* e_dev);
+int svdb200_bidiagonalize_mn_dev_f64(svdb200_handle h, double* a_dev, size_t m, size_t n, size_t band, double* d_dev, double* e_dev);
+int svdb200_svdvals_mn_f32(svdb200_handle h, float* a, size_t m, size_t n, size_t band, float* sigma);
+int svdb200_svdvals_mn_f64(svdb200_handle h, double* a, size_t m, size_t n, size_t band, double* sigma);
+int svdb200_svdvals_mn_dev_f32(svdb200_handle h, float* a_dev, size_t m, size_t n, size_t band, float* sigma_dev);
+int svdb200_svdvals_mn_dev_f64(svdb200_handle h, double* a_dev, size_t m, size_t n, size_t band, double* sigma_dev);
 
 /* ---- Batched small matrices (BASELINE config 5) ------------------------------------------------
  * `count` independent n x n matrices stored back to back; sigma is count x n.  One matrix per

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsvdb200.so")
-SOURCES = ["capi.cu", "stage1_panel.cu", "stage1_panel_reg.cu", "stage1_panel_blk.cu", "stage1_panel_chol.cu", "stage1_tile.cu", "gemm.cu", "gemm_fast.cu", "gemm_tc05.cu", "stage2_chase.cu", "stage2_chase_fast.cu", "bidiag_qr.cu", "bidiag_bisect.cu", "bidiag_sqr.cu", "dist.cu"]
+SOURCES = ["capi.cu", "stage1_panel.cu", "stage1_panel_reg.cu", "stage1_panel_blk.cu", "stage1_panel_chol.cu", "stage1_tile.cu", "gemm.cu", "gemm_fast.cu", "gemm_tc05.cu", "stage2_chase.cu", "stage2_chase_fast.cu", "bidiag_qr.cu", "bidiag_bisect.cu", "bidiag_sqr.cu", "dist.cu", "rect.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--expt-relaxed-constexpr",

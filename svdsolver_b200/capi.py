@@ -224,6 +224,30 @@ class Handle:
         self._check(self._fn("svdvals")(self.h, _p(a), Z(a.shape[0]), Z(a.shape[1]), Z(band), ctypes.c_int(order), _p(sigma)))
         return sigma, a
 
+    # ---- rectangular m x n (tall or wide); for m < n the result is lower band / bidiagonal, e the sub-diagonal ----
+    def dense_to_band_mn(self, a, band):
+        """stage 1 of an m x n matrix: returns the reduced matrix (upper band in the top n x n block for m >= n, lower band
+        in the left m x m block for m < n, zeros elsewhere)"""
+        a = self._mat(a)
+        self._check(self._fn("dense_to_band_mn")(self.h, _p(a), Z(a.shape[0]), Z(a.shape[1]), Z(band)))
+        return a
+
+    def bidiagonalize_mn(self, a, band):
+        """stages 1 and 2 of an m x n matrix: returns (A_out, d, e) with min(m, n) and min(m, n) - 1 entries"""
+        a = self._mat(a)
+        k = min(a.shape)
+        d = np.zeros(k, self.dtype)
+        e = np.zeros(max(k - 1, 0), self.dtype)
+        self._check(self._fn("bidiagonalize_mn")(self.h, _p(a), Z(a.shape[0]), Z(a.shape[1]), Z(band), _p(d), _p(e)))
+        return a, d, e
+
+    def svdvals_mn(self, a, band):
+        """singular values (descending, min(m, n)) of an m x n matrix: returns (sigma, A_out)"""
+        a = self._mat(a)
+        sigma = np.zeros(min(a.shape), self.dtype)
+        self._check(self._fn("svdvals_mn")(self.h, _p(a), Z(a.shape[0]), Z(a.shape[1]), Z(band), _p(sigma)))
+        return sigma, a
+
     def svdvals_batched(self, a, band):
         a = np.ascontiguousarray(a, dtype=self.dtype).copy()
         count, n, _ = a.shape
@@ -262,6 +286,15 @@ class Handle:
 
     def svdvals_dev(self, a_ptr, n, band, sigma_ptr, order=ORDER_PANEL):
         self._check(self._fn("svdvals_dev")(self.h, _p(a_ptr), Z(n), Z(n), Z(band), ctypes.c_int(order), _p(sigma_ptr)))
+
+    def dense_to_band_mn_dev(self, a_ptr, m, n, band):
+        self._check(self._fn("dense_to_band_mn_dev")(self.h, _p(a_ptr), Z(m), Z(n), Z(band)))
+
+    def bidiagonalize_mn_dev(self, a_ptr, m, n, band, d_ptr, e_ptr):
+        self._check(self._fn("bidiagonalize_mn_dev")(self.h, _p(a_ptr), Z(m), Z(n), Z(band), _p(d_ptr), _p(e_ptr)))
+
+    def svdvals_mn_dev(self, a_ptr, m, n, band, sigma_ptr):
+        self._check(self._fn("svdvals_mn_dev")(self.h, _p(a_ptr), Z(m), Z(n), Z(band), _p(sigma_ptr)))
 
     def svdvals_batched_dev(self, a_ptr, count, n, band, sigma_ptr):
         self._check(self._fn("svdvals_batched_dev")(self.h, _p(a_ptr), Z(count), Z(n), Z(band), _p(sigma_ptr)))

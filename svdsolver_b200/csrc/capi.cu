@@ -288,7 +288,7 @@ int batched_svdvals(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma)
         T* e = reinterpret_cast<T*>(s->e);
         const long long before = s->launches;
         s->overlap_safe = (concurrent && K > 1) ? 1 : 0;
-        const int st1 = stage1_panel_order<T>(s, ai, n, band);
+        const int st1 = stage1_panel_order<T>(s, ai, n, n, band);
         s->overlap_safe = 0;
         if (st1 != 0) { c->last_error = s->last_error; return st1; }
         SVDB_TRY(stage2_chase<T>(s, ai, n, band, d, e));
@@ -399,7 +399,7 @@ static int pipeline_one(Ctx* c, size_t i, T* a_dev, const T* a_host, size_t n, s
         // no overlap: wait for everything, run on the parent handle, and hold the pipeline back until it is done
         SVDB_TRY(drain_into(c, c->stream));
         if (a_host) SVDB_CHECK(c, cudaMemcpyAsync(a_dev, a_host, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream));
-        SVDB_TRY(order == SVDB200_ORDER_PANEL ? stage1_panel_order<T>(c, a_dev, n, band) : stage1_tile_order<T>(c, a_dev, n, band));
+        SVDB_TRY(order == SVDB200_ORDER_PANEL ? stage1_panel_order<T>(c, a_dev, n, n, band) : stage1_tile_order<T>(c, a_dev, n, band));
         if (i < c->band_capture.size() && c->band_capture[i])
             SVDB_CHECK(c, cudaMemcpyAsync(c->band_capture[i], a_dev, sizeof(T) * n * n, cudaMemcpyDeviceToDevice, c->stream));
         SVDB_TRY(stage2_chase<T>(c, a_dev, n, band, d, e));
@@ -415,7 +415,7 @@ static int pipeline_one(Ctx* c, size_t i, T* a_dev, const T* a_host, size_t n, s
     inherit_settings(c, s);
     if (a_host) SVDB_CHECK(c, cudaMemcpyAsync(a_dev, a_host, sizeof(T) * n * n, cudaMemcpyHostToDevice, s->stream));
     s->overlap_safe = 1;
-    int st = stage1_panel_order<T>(s, a_dev, n, band);
+    int st = stage1_panel_order<T>(s, a_dev, n, n, band);
     s->overlap_safe = 0;
     c->launches += s->launches; s->launches = 0;
     if (st != 0) { c->last_error = s->last_error; return st; }
@@ -589,7 +589,7 @@ int check_square(Ctx* c, size_t m, size_t n, size_t band, int dtype) {
 
 template <typename T>
 int stage1_dispatch(Ctx* c, T* a_dev, size_t n, size_t band, int order) {
-    if (order == SVDB200_ORDER_PANEL) return stage1_panel_order<T>(c, a_dev, n, band);
+    if (order == SVDB200_ORDER_PANEL) return stage1_panel_order<T>(c, a_dev, n, n, band);
     if (order == SVDB200_ORDER_TILE) return stage1_tile_order<T>(c, a_dev, n, band);
     return SVDB200_E_ARG;
 }
@@ -649,6 +649,51 @@ int host_chain(Ctx* c, T* a, size_t n, size_t band, int order, int what, T* d, T
         if (sweeps) *sweeps = info[0];
         if (info[1] != 0) return SVDB200_E_NOCONV;
     }
+    return 0;
+}
+
+// Shape rules of the m x n calls: any orientation, band | min(m, n) (the panel order needs whole panels along the
+// shorter side; the longer side is arbitrary)
+int check_mn(Ctx* c, size_t m, size_t n, size_t band) {
+    const size_t k = std::min(m, n);
+    if (k < 2 || band == 0 || k % band != 0) return SVDB200_E_SHAPE;
+    if (std::max(m, n) > c->max_n || band > c->band) return SVDB200_E_CAPACITY;
+    return 0;
+}
+
+// Host-pointer m x n chain (what as rect_chain): staged through a_dev (m n <= max_n^2 elements), per-stage timing as
+// host_chain with both transposes of a wide matrix counted in stage 1.
+template <typename T>
+int host_chain_mn(Ctx* c, T* a, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma) {
+    SVDB_TRY(ensure_staging(c));
+    T* ad = reinterpret_cast<T*>(c->a_dev);
+    T* dd = reinterpret_cast<T*>(c->d);
+    T* ed = reinterpret_cast<T*>(c->e);
+    T* sd = reinterpret_cast<T*>(c->sigma);
+    const size_t k = std::min(m, n);
+    cudaStream_t s = c->stream;
+    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
+    SVDB_CHECK(c, cudaEventRecord(c->ev[0], s));
+    SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * m * n, cudaMemcpyHostToDevice, s));
+    SVDB_CHECK(c, cudaEventRecord(c->ev[1], s));
+    SVDB_TRY(rect_chain<T>(c, ad, m, n, band, what, dd, ed, sd, c->ev + 2));   // ev[2..5]
+    SVDB_CHECK(c, cudaMemcpyAsync(a, ad, sizeof(T) * m * n, cudaMemcpyDeviceToHost, s));
+    long long info[3] = {0, 0, 0};
+    if (what & 4) {
+        SVDB_CHECK(c, cudaMemcpyAsync(sigma, sd, sizeof(T) * k, cudaMemcpyDeviceToHost, s));
+        SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
+    } else if (what & 2) {
+        if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, dd, sizeof(T) * k, cudaMemcpyDeviceToHost, s));
+        if (e) SVDB_CHECK(c, cudaMemcpyAsync(e, ed, sizeof(T) * (k - 1), cudaMemcpyDeviceToHost, s));
+    }
+    SVDB_CHECK(c, cudaEventRecord(c->ev[6], s));
+    SVDB_CHECK(c, cudaStreamSynchronize(s));
+    c->ms_h2d = elapsed(c->ev[0], c->ev[1]);
+    c->ms_stage1 = elapsed(c->ev[1], c->ev[2]) + elapsed(c->ev[4], c->ev[5]);
+    c->ms_stage2 = elapsed(c->ev[2], c->ev[3]);
+    c->ms_qr = elapsed(c->ev[3], c->ev[4]);
+    c->ms_d2h = elapsed(c->ev[5], c->ev[6]);
+    if ((what & 4) && info[1] != 0) return SVDB200_E_NOCONV;
     return 0;
 }
 
@@ -713,7 +758,7 @@ const char* svdb200_strerror(int s) {
     switch (s) {
         case SVDB200_OK: return "ok";
         case SVDB200_E_ARG: return "invalid argument";
-        case SVDB200_E_SHAPE: return "shape error: need square n x n with band | n";
+        case SVDB200_E_SHAPE: return "shape error: need square n x n with band | n (m x n calls: band | min(m, n) >= 2)";
         case SVDB200_E_CAPACITY: return "exceeds handle capacity or kernel limits";
         case SVDB200_E_NODEVICE: return "no usable CUDA device (there is no CPU fallback)";
         case SVDB200_E_NOCONV: return "QR diagonalisation reached max_iter";
@@ -808,7 +853,7 @@ int svdb200_destroy(svdb200_handle h) {
     c->pool.clear();
     void* ptrs[] = {c->a_dev, c->v, c->v2, c->vb, c->v2b, c->w, c->wpart, c->s, c->tau, c->red, c->red2, c->chol_ws, c->bar, c->prog,
                     c->d, c->e, c->sigma, c->qr_info, c->tileq, c->tilestate, c->tcsplit, c->bis_ws, c->batch_prog, c->batch_ws, c->de2,
-                    c->band_ws};
+                    c->band_ws, c->rect_ws};
     for (int k = 1; k < 2 * Ctx::kLanes; ++k) if (c->a_stage[k]) cudaFree(c->a_stage[k]);
     for (int l = 0; l < Ctx::kLanes; ++l) if (c->s1ctx[l]) svdb200_destroy(reinterpret_cast<svdb200_handle>(c->s1ctx[l]));
     for (int l = 1; l < Ctx::kLanes; ++l) if (c->s2_prog[l]) cudaFree(c->s2_prog[l]);
@@ -929,7 +974,7 @@ int svdb200_synchronize(svdb200_handle h) {
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
         c->onestage = 1;                                                                                                 \
-        const int st = stage1_panel_order<T>(c, a, n, 1);                                                                \
+        const int st = stage1_panel_order<T>(c, a, n, n, 1);                                                              \
         c->onestage = 0;                                                                                                 \
         if (st != 0) return st;                                                                                          \
         return extract_bidiagonal<T>(c, a, n, d, e);                                                                     \
@@ -942,7 +987,7 @@ int svdb200_synchronize(svdb200_handle h) {
         T* ad = reinterpret_cast<T*>(c->a_dev);                                                                          \
         SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream));                     \
         c->onestage = 1;                                                                                                 \
-        int st = stage1_panel_order<T>(c, ad, n, 1);                                                                     \
+        int st = stage1_panel_order<T>(c, ad, n, n, 1);                                                                   \
         c->onestage = 0;                                                                                                 \
         if (st == 0) st = extract_bidiagonal<T>(c, ad, n, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e));       \
         if (st != 0) return st;                                                                                          \
@@ -985,6 +1030,42 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_TRY(stage1_dispatch<T>(c, a, n, band, order));                                                              \
         SVDB_TRY(stage2_chase<T>(c, a, n, band, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e)));                \
         return bidiag_qr<T>(c, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), n, sigma);                        \
+    }                                                                                                                    \
+    int svdb200_dense_to_band_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band) {                          \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a) return SVDB200_E_ARG;                                                                                    \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return host_chain_mn<T>(c, a, m, n, band, 1, nullptr, nullptr, nullptr);                                         \
+    }                                                                                                                    \
+    int svdb200_dense_to_band_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band) {                      \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a) return SVDB200_E_ARG;                                                                                    \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return rect_chain<T>(c, a, m, n, band, 1, nullptr, nullptr, nullptr, nullptr);                                   \
+    }                                                                                                                    \
+    int svdb200_bidiagonalize_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {              \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !d || !e) return SVDB200_E_ARG;                                                                        \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return host_chain_mn<T>(c, a, m, n, band, 3, d, e, nullptr);                                                     \
+    }                                                                                                                    \
+    int svdb200_bidiagonalize_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {          \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !d || !e) return SVDB200_E_ARG;                                                                        \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return rect_chain<T>(c, a, m, n, band, 3, d, e, nullptr, nullptr);                                               \
+    }                                                                                                                    \
+    int svdb200_svdvals_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* sigma) {                      \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return host_chain_mn<T>(c, a, m, n, band, 7, nullptr, nullptr, sigma);                                           \
+    }                                                                                                                    \
+    int svdb200_svdvals_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* sigma) {                  \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return rect_chain<T>(c, a, m, n, band, 7, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), sigma, nullptr); \
     }                                                                                                                    \
     int svdb200_svdvals_batched_dev_##S(svdb200_handle h, T* a, size_t count, size_t n, size_t band, T* sigma) {         \
         SVDB_ENTER(T)                                                                                                    \

@@ -53,6 +53,8 @@ struct Ctx {
     unsigned int* bar = nullptr;   // software grid barrier state (2 words) + misc counters
     int* prog = nullptr;           // stage-2 per-sweep progress counters (max_n)
     void* band_ws = nullptr;       // max_n * 3 band: stage 2 from band storage, packed 3-band-diagonal layout (first use)
+    void* rect_ws = nullptr;       // m * n: A^T of a wide m x n matrix (m < n), reduced there; grown on demand
+    size_t rect_ws_elems = 0;
     void* d = nullptr; void* e = nullptr; void* sigma = nullptr;   // max_n each
     long long* qr_info = nullptr;  // [0] sweeps, [1] status
     void* tileq = nullptr;         // tile order: per-chain-step Q matrices, (max_n/band) * 4*band*band
@@ -211,7 +213,9 @@ template <typename T, bool kPacked> int stage2_chase_fast(Ctx* c, T* a, size_t n
 template <typename T> int bidiag_qr(Ctx* c, T* d, T* e, size_t n, T* sigma);
 template <typename T> int bidiag_bisect(Ctx* c, const T* d, const T* e, size_t n, T* sigma);
 template <typename T> int bidiag_sqr(Ctx* c, T* d, T* e, size_t n, T* sigma);
-template <typename T> int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band);
+template <typename T> int stage1_panel_order(Ctx* c, T* a, size_t rows, size_t n, size_t band);   // a: rows x n, rows >= n
+// m x n (either orientation) through stage 1 / stage 2 / singular values; rect.cu
+template <typename T> int rect_chain(Ctx* c, T* a, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma, cudaEvent_t* marks);
 template <typename T> int stage1_tile_order(Ctx* c, T* a, size_t n, size_t band);
 template <typename T> int gemm_tn(Ctx* c, const T* v, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, T* w);
 template <typename T> int gemm_nn(Ctx* c, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, const T* ut, T* w);

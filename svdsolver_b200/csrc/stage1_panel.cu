@@ -406,10 +406,15 @@ template int panel_batched<double, true>(Ctx*, double*, size_t, size_t, int, int
 // QR reflectors use (v, v2), LQ reflectors (vb, v2b), so a panel in flight never overwrites
 // reflectors that the concurrent update still reads.  In profiling mode the steps are serialised
 // so that per-kernel-class times stay meaningful.
+//
+// `a` is rows x n (rows >= n), row-major with ld = n.  The QR panel of step k spans rows k .. rows-1;
+// everything else depends on the height only through it.  The top n x n block ends up upper band
+// (b+1 diagonals) and rows n .. rows-1 exact zeros: each QR panel writes R with zeros below it, and
+// later updates only touch columns to its right.  rows == n is the square reduction.
 template <typename T>
-int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
-    if (band == 0 || n == 0 || n % band != 0) return SVDB200_E_SHAPE;
-    if (band > (size_t)kMaxBand || n > c->max_n || band > c->band) return SVDB200_E_CAPACITY;
+int stage1_panel_order(Ctx* c, T* a, size_t rows, size_t n, size_t band) {
+    if (band == 0 || n == 0 || n % band != 0 || rows < n) return SVDB200_E_SHAPE;
+    if (band > (size_t)kMaxBand || rows > c->max_n || band > c->band) return SVDB200_E_CAPACITY;
     const int b = (int)band;
     T* Vq = reinterpret_cast<T*>(c->v);
     T* V2q = reinterpret_cast<T*>(c->v2);
@@ -423,10 +428,10 @@ int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
         SVDB_CHECK(c, cudaStreamWaitEvent(s1, c->lev[0], 0));
     }
     // first QR panel
-    SVDB_TRY((launch_panel<T, false>(c, a, n, (int)n, b, Vq, V2q, s1)));
+    SVDB_TRY((launch_panel<T, false>(c, a, n, (int)rows, b, Vq, V2q, s1)));
     if (ahead) SVDB_CHECK(c, cudaEventRecord(c->lev[1], s1));
     for (size_t k = 0; k < n; k += band) {
-        const size_t m = n - k;                 // panel height
+        const size_t m = rows - k;              // panel height
         const size_t nc = n - k - band;         // columns right of the QR panel
         // svd_cpu.h:396 skips the LQ half-step when only one column is left; the one-stage Golub-Kahan order
         // (serial::brd, svd_serial.h:248) still applies that length-1 reflector (a sign flip): c->onestage
@@ -488,7 +493,7 @@ int stage1_panel_order(Ctx* c, T* a, size_t n, size_t band) {
     return 0;
 }
 
-template int stage1_panel_order<float>(Ctx*, float*, size_t, size_t);
-template int stage1_panel_order<double>(Ctx*, double*, size_t, size_t);
+template int stage1_panel_order<float>(Ctx*, float*, size_t, size_t, size_t);
+template int stage1_panel_order<double>(Ctx*, double*, size_t, size_t, size_t);
 
 }  // namespace svdb200
