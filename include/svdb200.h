@@ -207,7 +207,10 @@ int svdb200_chain_batched_dev_f64(svdb200_handle h, double* a_dev, size_t count,
 int svdb200_set_band_capture(svdb200_handle h, void* const* dev_bufs, size_t count);
 
 /* ---- Measurement helpers ------------------------------------------------------------------------
- * Device time (CUDA events on the handle's stream) of the stages of the LAST host-pointer call, ms.
+ * Device time (CUDA events on the handle's stream) of the stages of the LAST host-pointer compute call
+ * (not the list calls), ms: h2d, d2h and every stage the call ran (stage 1 includes the transposes of a
+ * wide matrix and the one-stage reduction); a stage the call did not run reports exactly 0.
+ * svdvals_batched interleaves the stages of its matrices and reports only h2d and d2h.
  * stage-1 sub-times: panel factorisations vs trailing updates are reported by svdb200_stage1_profile. */
 int svdb200_last_timings(svdb200_handle h, double* ms_stage1, double* ms_stage2, double* ms_qr, double* ms_h2d, double* ms_d2h);
 /* Per-kernel-class profiling.  When on, every launch of the hot-path kernels is bracketed by CUDA

@@ -76,14 +76,8 @@ template <typename T>
 int bidiag_bisect_batched(Ctx* c, const T* d, const T* e, size_t n, T* sigma, int count) {
     if (n < 1 || count < 1 || count > 65535) return SVDB200_E_SHAPE;
     const size_t need = (size_t)count * (2 * n + 8) + 16;
-    if (c->bis_ws_elems < need) {
-        if (c->bis_ws) cudaFree(c->bis_ws);
-        c->bis_ws = nullptr; c->bis_ws_elems = 0;
-        const size_t want = std::max(need, (size_t)(2 * c->max_n + 24));
-        SVDB_CHECK(c, cudaMalloc(&c->bis_ws, sizeof(double) * want));
-        c->bis_ws_elems = want;
-    }
-    double* params = reinterpret_cast<double*>(c->bis_ws);
+    SVDB_TRY(reserve(c, c->bis_ws, sizeof(double) * std::max(need, (size_t)(2 * c->max_n + 24))));
+    double* params = reinterpret_cast<double*>(c->bis_ws.p);
     double* z2 = params + 8 * (size_t)count;
     const int ni = (int)n;
     bisect_prep_kernel<T><<<count, 1024, 0, c->stream>>>(d, e, ni, z2, params, c->qr_info);

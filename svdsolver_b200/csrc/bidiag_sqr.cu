@@ -175,15 +175,9 @@ int bidiag_sqr(Ctx* c, T* d, T* e, size_t n, T* sigma) {
         SVDB_CHECK(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<1, 32, smem, c->stream>>>(d, e, ni, sigma, sortbuf, npad, c->qr_info, (double*)nullptr);
     } else {
-        if (c->bis_ws_elems < 2 * n + 24) {                      // double workspace shared with the bisection solver
-            if (c->bis_ws) cudaFree(c->bis_ws);
-            c->bis_ws = nullptr; c->bis_ws_elems = 0;
-            const size_t want = 2 * c->max_n + 24;
-            SVDB_CHECK(c, cudaMalloc(&c->bis_ws, sizeof(double) * want));
-            c->bis_ws_elems = want;
-        }
+        SVDB_TRY(reserve(c, c->bis_ws, sizeof(double) * (2 * c->max_n + 24)));   // double workspace shared with the bisection solver
         auto kern = bidiag_sqr_kernel<T, false>;
-        kern<<<1, 32, 0, c->stream>>>(d, e, ni, sigma, sortbuf, npad, c->qr_info, reinterpret_cast<double*>(c->bis_ws));
+        kern<<<1, 32, 0, c->stream>>>(d, e, ni, sigma, sortbuf, npad, c->qr_info, reinterpret_cast<double*>(c->bis_ws.p));
     }
     SVDB_CHECK(c, cudaGetLastError());
     c->launches++;

@@ -1,6 +1,9 @@
 // C ABI of libsvdb200.so (declared in include/svdb200.h).  Thin: argument checks, workspace
 // ownership, host<->device staging and CUDA-event timing; all arithmetic lives in the kernels.
+// Every dense single-matrix call runs run_chain on the device; every single-matrix host-pointer
+// call is one host_call (copies in, device work, copies out, one synchronise, stage timings).
 #include <algorithm>
+#include <initializer_list>
 #include <new>
 #include "common.cuh"
 
@@ -198,15 +201,9 @@ int batched_small(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma, i
     const size_t per_mat = 5 * n * band + 2 * n;
     size_t chunk = std::min<size_t>(count, 8192);
     while (chunk > 1 && chunk * per_mat * sizeof(T) > ((size_t)2 << 30)) chunk = (chunk + 1) / 2;
-    const size_t need = chunk * per_mat * sizeof(T);
-    if (c->batch_ws_bytes < need) {
-        if (c->batch_ws) cudaFree(c->batch_ws);
-        c->batch_ws = nullptr; c->batch_ws_bytes = 0;
-        SVDB_CHECK(c, cudaMalloc(&c->batch_ws, need));
-        c->batch_ws_bytes = need;
-    }
+    SVDB_TRY(reserve(c, c->batch_ws, chunk * per_mat * sizeof(T)));
     const size_t sV = n * band, sA = n * n;
-    T* Vq = reinterpret_cast<T*>(c->batch_ws);
+    T* Vq = reinterpret_cast<T*>(c->batch_ws.p);
     T* V2q = Vq + chunk * sV;
     T* Vl = V2q + chunk * sV;
     T* V2l = Vl + chunk * sV;
@@ -502,8 +499,8 @@ int bidiagonalize_many_host(Ctx* c, size_t count, T* const* a, const size_t* n, 
     if (count == 0) return 0;
     SVDB_TRY(ensure_s2(c));
     constexpr int NB = 2 * Ctx::kLanes;
-    if (!c->a_dev) SVDB_CHECK(c, cudaMalloc(&c->a_dev, c->esz * c->max_n * c->max_n));
-    c->a_stage[0] = c->a_dev;
+    SVDB_TRY(reserve(c, c->a_dev, c->esz * c->max_n * c->max_n));
+    c->a_stage[0] = c->a_dev.p;
     for (int k = 1; k < NB; ++k)
         if (!c->a_stage[k]) SVDB_CHECK(c, cudaMalloc(&c->a_stage[k], c->esz * c->max_n * c->max_n));
     if (!c->de2) SVDB_CHECK(c, cudaMalloc(&c->de2, c->esz * 2 * NB * (c->max_n + 8)));
@@ -587,69 +584,133 @@ int check_square(Ctx* c, size_t m, size_t n, size_t band, int dtype) {
     return 0;
 }
 
-template <typename T>
-int stage1_dispatch(Ctx* c, T* a_dev, size_t n, size_t band, int order) {
-    if (order == SVDB200_ORDER_PANEL) return stage1_panel_order<T>(c, a_dev, n, n, band);
-    if (order == SVDB200_ORDER_TILE) return stage1_tile_order<T>(c, a_dev, n, band);
-    return SVDB200_E_ARG;
-}
-
 float elapsed(cudaEvent_t a, cudaEvent_t b) {
     float ms = 0;
     cudaEventElapsedTime(&ms, a, b);
     return ms;
 }
 
-// Host-pointer chain with per-stage CUDA-event timing.  what: bit0 stage1, bit1 stage2, bit2 qr.
-int ensure_staging(Ctx* c) {
-    if (!c->a_dev) SVDB_CHECK(c, cudaMalloc(&c->a_dev, c->esz * c->max_n * c->max_n));
+// marks[k] recorded on the handle's stream (marks == nullptr: nothing recorded)
+int mark(Ctx* c, cudaEvent_t* marks, int k) {
+    if (marks) SVDB_CHECK(c, cudaEventRecord(marks[k], c->stream));
     return 0;
 }
 
+// The device chain of the dense single-matrix calls, square and m x n.  what: 1 = stage 1 (a -> band), 2 = stage 2 (band ->
+// d, e: min(m, n) and min(m, n) - 1 entries), 4 = singular values of d, e into sigma; each bit runs its own stage only.
+// Tall (m >= n): stage 1 runs in place on the m x n array; the top n x n block is then upper band, the rows below it zero,
+// and stage 2 / the singular values run on that block (contiguous, ld = n) exactly as for a square matrix.  Wide (m < n):
+// sigma(A) = sigma(A^T), so A is transposed into the handle's scratch, reduced there as tall and transposed back; `a` then
+// holds a LOWER band / bidiagonal matrix in its left m x m block (LAPACK gebrd's convention) and e is the sub-diagonal.
+// The tile order takes square matrices only.  marks (4 events, optional) are recorded after stage 1 (forward transpose
+// included), after stage 2, after the singular values and after the transpose back.  Shapes are checked by the caller.
 template <typename T>
-int host_chain(Ctx* c, T* a, size_t n, size_t band, int order, int what, T* d, T* e, T* sigma, long long* sweeps) {
-    if (what & 3) SVDB_TRY(ensure_staging(c));
-    T* ad = reinterpret_cast<T*>(c->a_dev);
-    T* dd = reinterpret_cast<T*>(c->d);
-    T* ed = reinterpret_cast<T*>(c->e);
-    T* sd = reinterpret_cast<T*>(c->sigma);
+int run_chain(Ctx* c, T* a, size_t m, size_t n, size_t band, int order, int what, T* d, T* e, T* sigma, cudaEvent_t* marks) {
+    const bool wide = m < n;
+    const size_t k = std::min(m, n);
+    T* x = a;
+    if (wide) {
+        SVDB_TRY(reserve(c, c->rect_ws, sizeof(T) * m * n));   // grown (never shrunk) when a larger wide matrix arrives
+        x = reinterpret_cast<T*>(c->rect_ws.p);
+        SVDB_TRY(transpose<T>(c, a, m, n, x));                 // x = A^T: n x m, tall
+    }
+    if (what & 1) {
+        if (order == SVDB200_ORDER_PANEL) SVDB_TRY(stage1_panel_order<T>(c, x, std::max(m, n), k, band));
+        else if (order == SVDB200_ORDER_TILE && m == n) SVDB_TRY(stage1_tile_order<T>(c, x, n, band));
+        else return SVDB200_E_ARG;
+    }
+    SVDB_TRY(mark(c, marks, 0));
+    if (what & 2) SVDB_TRY(stage2_chase<T>(c, x, k, band, d, e));
+    SVDB_TRY(mark(c, marks, 1));
+    if (what & 4) SVDB_TRY(bidiag_qr<T>(c, d, e, k, sigma));
+    SVDB_TRY(mark(c, marks, 2));
+    if (wide) SVDB_TRY(transpose<T>(c, x, n, m, a));
+    return mark(c, marks, 3);
+}
+
+// One-stage Golub-Kahan bidiagonalisation: the stage-1 panel driver with band 1 in the one-stage order, then d, e (optional)
+// read off the result.  All four marks (as run_chain's) follow the reduction: it is all stage 1.
+template <typename T>
+int onestage_chain(Ctx* c, T* a, size_t n, T* d, T* e, cudaEvent_t* marks) {
+    c->onestage = 1;
+    const int st = stage1_panel_order<T>(c, a, n, n, 1);
+    c->onestage = 0;
+    if (st != 0) return st;
+    SVDB_TRY(extract_bidiagonal<T>(c, a, n, d, e));
+    for (int k = 0; k < 4; ++k) SVDB_TRY(mark(c, marks, k));
+    return 0;
+}
+
+// Stage 2 from LAPACK upper band storage and, when sigma is given, the singular values of d, e; marks as run_chain's
+// (there is no stage 1)
+template <typename T>
+int packed_chain(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e, T* sigma, cudaEvent_t* marks) {
+    SVDB_TRY(mark(c, marks, 0));
+    SVDB_TRY(stage2_chase_packed<T>(c, ab, n, band, d, e));
+    SVDB_TRY(mark(c, marks, 1));
+    if (sigma) SVDB_TRY(bidiag_qr<T>(c, d, e, n, sigma));
+    SVDB_TRY(mark(c, marks, 2));
+    return mark(c, marks, 3);
+}
+
+// One copy of a host-pointer call; skipped when dst is null (an optional output) or bytes is 0
+struct Copy { void* dst; const void* src; size_t bytes; };
+
+// Every single-matrix host-pointer call: the input copies (host -> device), run(marks), which enqueues the device work and
+// records the four marks of run_chain, and the output copies (device -> host).  The stream is synchronised once before
+// returning, on success and on error, so that no copy from or to the caller's buffers is in flight after the call; a
+// failed stage's status wins over a later CUDA error.  The device buffers are the caller's.  svdb200_last_timings gets
+// h2d, d2h and the time of every stage whose `what` bit is set (1 stage 1 with the transpose back of a wide matrix,
+// 2 stage 2, 4 singular values); a stage whose bit is clear reports 0.  With bit 4 the status of the singular values is
+// read back: non-convergence returns SVDB200_E_NOCONV, and the sweep count goes to *sweeps.
+template <typename Run>
+int host_call(Ctx* c, std::initializer_list<Copy> in, Run&& run, std::initializer_list<Copy> out, int what,
+              long long* sweeps = nullptr) {
     cudaStream_t s = c->stream;
-    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
-    SVDB_CHECK(c, cudaEventRecord(c->ev[0], s));
-    if (what & 3) SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * n * n, cudaMemcpyHostToDevice, s));
-    if (!(what & 3) && (what & 4)) {
-        SVDB_CHECK(c, cudaMemcpyAsync(dd, d, sizeof(T) * n, cudaMemcpyHostToDevice, s));
-        SVDB_CHECK(c, cudaMemcpyAsync(ed, e, sizeof(T) * (n - 1), cudaMemcpyHostToDevice, s));
-    }
-    SVDB_CHECK(c, cudaEventRecord(c->ev[1], s));
-    if (what & 1) SVDB_TRY(stage1_dispatch<T>(c, ad, n, band, order));
-    SVDB_CHECK(c, cudaEventRecord(c->ev[2], s));
-    if (what & 2) SVDB_TRY(stage2_chase<T>(c, ad, n, band, dd, ed));
-    SVDB_CHECK(c, cudaEventRecord(c->ev[3], s));
-    if (what & 4) SVDB_TRY(bidiag_qr<T>(c, dd, ed, n, sd));
-    SVDB_CHECK(c, cudaEventRecord(c->ev[4], s));
-    if ((what & 3) && a) SVDB_CHECK(c, cudaMemcpyAsync(a, ad, sizeof(T) * n * n, cudaMemcpyDeviceToHost, s));
-    if ((what & 2) && !(what & 4)) {
-        if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, dd, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
-        if (e) SVDB_CHECK(c, cudaMemcpyAsync(e, ed, sizeof(T) * (n - 1), cudaMemcpyDeviceToHost, s));
-    }
+    cudaEvent_t* ev = c->ev;
     long long info[3] = {0, 0, 0};
-    if (what & 4) {
-        SVDB_CHECK(c, cudaMemcpyAsync(sigma, sd, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
-        SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
-    }
-    SVDB_CHECK(c, cudaEventRecord(c->ev[5], s));
-    SVDB_CHECK(c, cudaStreamSynchronize(s));
-    c->ms_h2d = elapsed(c->ev[0], c->ev[1]);
-    c->ms_stage1 = elapsed(c->ev[1], c->ev[2]);
-    c->ms_stage2 = elapsed(c->ev[2], c->ev[3]);
-    c->ms_qr = elapsed(c->ev[3], c->ev[4]);
-    c->ms_d2h = elapsed(c->ev[4], c->ev[5]);
+    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
+    auto enqueue = [&]() -> int {
+        SVDB_CHECK(c, cudaEventRecord(ev[0], s));
+        for (const Copy& x : in)
+            if (x.dst && x.bytes) SVDB_CHECK(c, cudaMemcpyAsync(x.dst, x.src, x.bytes, cudaMemcpyHostToDevice, s));
+        SVDB_CHECK(c, cudaEventRecord(ev[1], s));
+        SVDB_TRY(run(ev + 2));                                    // ev[2..5]
+        for (const Copy& x : out)
+            if (x.dst && x.bytes) SVDB_CHECK(c, cudaMemcpyAsync(x.dst, x.src, x.bytes, cudaMemcpyDeviceToHost, s));
+        if (what & 4) SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
+        SVDB_CHECK(c, cudaEventRecord(ev[6], s));
+        return 0;
+    };
+    const int st = enqueue();
+    const cudaError_t se = cudaStreamSynchronize(s);
+    if (st != 0) return st;
+    if (se != cudaSuccess) return cuda_status(c, se, "cudaStreamSynchronize");
+    c->ms_h2d = elapsed(ev[0], ev[1]);
+    if (what & 1) c->ms_stage1 = elapsed(ev[1], ev[2]) + elapsed(ev[4], ev[5]);
+    if (what & 2) c->ms_stage2 = elapsed(ev[2], ev[3]);
+    if (what & 4) c->ms_qr = elapsed(ev[3], ev[4]);
+    c->ms_d2h = elapsed(ev[5], ev[6]);
     if (what & 4) {
         if (sweeps) *sweeps = info[0];
         if (info[1] != 0) return SVDB200_E_NOCONV;
     }
     return 0;
+}
+
+// Host-pointer dense call (square or m x n) through run_chain, staged through the handle's max_n^2 buffer; d, e, sigma
+// (host, each optional) receive min(m, n), min(m, n) - 1 and min(m, n) entries
+template <typename T>
+int dense_host(Ctx* c, T* a, size_t m, size_t n, size_t band, int order, int what, T* d, T* e, T* sigma) {
+    SVDB_TRY(reserve(c, c->a_dev, c->esz * c->max_n * c->max_n));
+    T* ad = reinterpret_cast<T*>(c->a_dev.p);
+    T* dd = reinterpret_cast<T*>(c->d);
+    T* ed = reinterpret_cast<T*>(c->e);
+    T* sd = reinterpret_cast<T*>(c->sigma);
+    const size_t k = std::min(m, n), bytes = sizeof(T) * m * n;
+    return host_call(
+        c, {{ad, a, bytes}}, [&](cudaEvent_t* marks) { return run_chain<T>(c, ad, m, n, band, order, what, dd, ed, sd, marks); },
+        {{a, ad, bytes}, {d, dd, sizeof(T) * k}, {e, ed, sizeof(T) * (k - 1)}, {sigma, sd, sizeof(T) * k}}, what);
 }
 
 // Shape rules of the m x n calls: any orientation, band | min(m, n) (the panel order needs whole panels along the
@@ -661,90 +722,12 @@ int check_mn(Ctx* c, size_t m, size_t n, size_t band) {
     return 0;
 }
 
-// Host-pointer m x n chain (what as rect_chain): staged through a_dev (m n <= max_n^2 elements), per-stage timing as
-// host_chain with both transposes of a wide matrix counted in stage 1.
-template <typename T>
-int host_chain_mn(Ctx* c, T* a, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma) {
-    SVDB_TRY(ensure_staging(c));
-    T* ad = reinterpret_cast<T*>(c->a_dev);
-    T* dd = reinterpret_cast<T*>(c->d);
-    T* ed = reinterpret_cast<T*>(c->e);
-    T* sd = reinterpret_cast<T*>(c->sigma);
-    const size_t k = std::min(m, n);
-    cudaStream_t s = c->stream;
-    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
-    SVDB_CHECK(c, cudaEventRecord(c->ev[0], s));
-    SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * m * n, cudaMemcpyHostToDevice, s));
-    SVDB_CHECK(c, cudaEventRecord(c->ev[1], s));
-    SVDB_TRY(rect_chain<T>(c, ad, m, n, band, what, dd, ed, sd, c->ev + 2));   // ev[2..5]
-    SVDB_CHECK(c, cudaMemcpyAsync(a, ad, sizeof(T) * m * n, cudaMemcpyDeviceToHost, s));
-    long long info[3] = {0, 0, 0};
-    if (what & 4) {
-        SVDB_CHECK(c, cudaMemcpyAsync(sigma, sd, sizeof(T) * k, cudaMemcpyDeviceToHost, s));
-        SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
-    } else if (what & 2) {
-        if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, dd, sizeof(T) * k, cudaMemcpyDeviceToHost, s));
-        if (e) SVDB_CHECK(c, cudaMemcpyAsync(e, ed, sizeof(T) * (k - 1), cudaMemcpyDeviceToHost, s));
-    }
-    SVDB_CHECK(c, cudaEventRecord(c->ev[6], s));
-    SVDB_CHECK(c, cudaStreamSynchronize(s));
-    c->ms_h2d = elapsed(c->ev[0], c->ev[1]);
-    c->ms_stage1 = elapsed(c->ev[1], c->ev[2]) + elapsed(c->ev[4], c->ev[5]);
-    c->ms_stage2 = elapsed(c->ev[2], c->ev[3]);
-    c->ms_qr = elapsed(c->ev[3], c->ev[4]);
-    c->ms_d2h = elapsed(c->ev[5], c->ev[6]);
-    if ((what & 4) && info[1] != 0) return SVDB200_E_NOCONV;
-    return 0;
-}
-
 size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // Shape rules of stage 2 from band storage: those of svdb200_band_to_bidiag_dev_* (no m, band need not divide n)
 int check_packed(Ctx* c, size_t n, size_t band) {
     if (n < 2) return SVDB200_E_SHAPE;
     if (band == 0 || band > c->band || n > c->max_n) return SVDB200_E_CAPACITY;
-    return 0;
-}
-
-// Host-pointer stage 2 (sigma == nullptr: d / e out) or stage 2 + singular values from band storage, with the per-stage
-// timing of host_chain.  The n x (band+1) input is staged in a buffer of its own for the call.
-template <typename T>
-int packed_host(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e, T* sigma) {
-    T* abd = nullptr;
-    SVDB_CHECK(c, cudaMalloc(&abd, sizeof(T) * n * (band + 1)));
-    T* dd = reinterpret_cast<T*>(c->d);
-    T* ed = reinterpret_cast<T*>(c->e);
-    cudaStream_t s = c->stream;
-    long long info[3] = {0, 0, 0};
-    auto run = [&]() -> int {
-        SVDB_CHECK(c, cudaEventRecord(c->ev[0], s));
-        SVDB_CHECK(c, cudaMemcpyAsync(abd, ab, sizeof(T) * n * (band + 1), cudaMemcpyHostToDevice, s));
-        SVDB_CHECK(c, cudaEventRecord(c->ev[1], s));
-        SVDB_TRY(stage2_chase_packed<T>(c, abd, n, band, dd, ed));
-        SVDB_CHECK(c, cudaEventRecord(c->ev[2], s));
-        if (sigma) SVDB_TRY(bidiag_qr<T>(c, dd, ed, n, reinterpret_cast<T*>(c->sigma)));
-        SVDB_CHECK(c, cudaEventRecord(c->ev[3], s));
-        if (sigma) {
-            SVDB_CHECK(c, cudaMemcpyAsync(sigma, c->sigma, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
-            SVDB_CHECK(c, cudaMemcpyAsync(info, c->qr_info, sizeof(info), cudaMemcpyDeviceToHost, s));
-        } else {
-            if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, dd, sizeof(T) * n, cudaMemcpyDeviceToHost, s));
-            if (e) SVDB_CHECK(c, cudaMemcpyAsync(e, ed, sizeof(T) * (n - 1), cudaMemcpyDeviceToHost, s));
-        }
-        SVDB_CHECK(c, cudaEventRecord(c->ev[4], s));
-        return 0;
-    };
-    c->ms_stage1 = c->ms_stage2 = c->ms_qr = c->ms_h2d = c->ms_d2h = 0;
-    const int st = run();
-    const cudaError_t se = cudaStreamSynchronize(s);
-    cudaFree(abd);
-    if (st != 0) return st;
-    if (se != cudaSuccess) return cuda_status(c, se, "cudaStreamSynchronize");
-    c->ms_h2d = elapsed(c->ev[0], c->ev[1]);
-    c->ms_stage2 = elapsed(c->ev[1], c->ev[2]);
-    c->ms_qr = elapsed(c->ev[2], c->ev[3]);
-    c->ms_d2h = elapsed(c->ev[3], c->ev[4]);
-    if (sigma && info[1] != 0) return SVDB200_E_NOCONV;
     return 0;
 }
 
@@ -851,9 +834,8 @@ int svdb200_destroy(svdb200_handle h) {
     if (c->own_stream) cudaStreamSynchronize(c->own_stream);
     for (auto& ph : c->pool) if (ph) svdb200_destroy(reinterpret_cast<svdb200_handle>(ph));
     c->pool.clear();
-    void* ptrs[] = {c->a_dev, c->v, c->v2, c->vb, c->v2b, c->w, c->wpart, c->s, c->tau, c->red, c->red2, c->chol_ws, c->bar, c->prog,
-                    c->d, c->e, c->sigma, c->qr_info, c->tileq, c->tilestate, c->tcsplit, c->bis_ws, c->batch_prog, c->batch_ws, c->de2,
-                    c->band_ws, c->rect_ws};
+    void* ptrs[] = {c->v, c->v2, c->vb, c->v2b, c->w, c->wpart, c->s, c->tau, c->red, c->red2, c->chol_ws, c->bar, c->prog,
+                    c->d, c->e, c->sigma, c->qr_info, c->tileq, c->tilestate, c->de2};   // the DevBuf members free themselves with c
     for (int k = 1; k < 2 * Ctx::kLanes; ++k) if (c->a_stage[k]) cudaFree(c->a_stage[k]);
     for (int l = 0; l < Ctx::kLanes; ++l) if (c->s1ctx[l]) svdb200_destroy(reinterpret_cast<svdb200_handle>(c->s1ctx[l]));
     for (int l = 1; l < Ctx::kLanes; ++l) if (c->s2_prog[l]) cudaFree(c->s2_prog[l]);
@@ -894,33 +876,39 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        return host_chain<T>(c, a, n, band, order, 1, nullptr, nullptr, nullptr, nullptr);                               \
+        return dense_host<T>(c, a, n, n, band, order, 1, nullptr, nullptr, nullptr);                                     \
     }                                                                                                                    \
     int svdb200_dense_to_band_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, int order) {              \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        return stage1_dispatch<T>(c, a, n, band, order);                                                                 \
+        return run_chain<T>(c, a, n, n, band, order, 1, nullptr, nullptr, nullptr, nullptr);                             \
     }                                                                                                                    \
     int svdb200_band_to_bidiag_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {                \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
         if (band == 0 || band > c->band) return SVDB200_E_CAPACITY;                                                      \
-        return host_chain<T>(c, a, n, band, 0, 2, d, e, nullptr, nullptr);                                               \
+        return dense_host<T>(c, a, n, n, band, SVDB200_ORDER_PANEL, 2, d, e, nullptr);                                   \
     }                                                                                                                    \
     int svdb200_band_to_bidiag_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {            \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
         if (band == 0 || band > c->band) return SVDB200_E_CAPACITY;                                                      \
-        return stage2_chase<T>(c, a, n, band, d, e);                                                                     \
+        return run_chain<T>(c, a, n, n, band, SVDB200_ORDER_PANEL, 2, d, e, nullptr, nullptr);                           \
     }                                                                                                                    \
     int svdb200_band_to_bidiag_packed_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* d, T* e) {            \
         SVDB_ENTER(T)                                                                                                    \
         if (!ab) return SVDB200_E_ARG;                                                                                   \
         SVDB_TRY(check_packed(c, n, band));                                                                              \
-        return packed_host<T>(c, ab, n, band, d, e, nullptr);                                                            \
+        DevBuf abd;                                        /* per call: the handle does not keep n (band + 1) elements */ \
+        SVDB_TRY(reserve(c, abd, sizeof(T) * n * (band + 1)));                                                           \
+        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
+        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
+        return host_call(c, {{abd.p, ab, abd.bytes}},                                                                    \
+                         [&](cudaEvent_t* mk) { return packed_chain<T>(c, (const T*)abd.p, n, band, dd, ed, nullptr, mk); }, \
+                         {{d, dd, sizeof(T) * n}, {e, ed, sizeof(T) * (n - 1)}}, 2);                                     \
     }                                                                                                                    \
     int svdb200_band_to_bidiag_packed_dev_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* d, T* e) {        \
         SVDB_ENTER(T)                                                                                                    \
@@ -932,23 +920,32 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!ab || !sigma) return SVDB200_E_ARG;                                                                         \
         SVDB_TRY(check_packed(c, n, band));                                                                              \
-        return packed_host<T>(c, ab, n, band, nullptr, nullptr, sigma);                                                  \
+        DevBuf abd;                                                                                                      \
+        SVDB_TRY(reserve(c, abd, sizeof(T) * n * (band + 1)));                                                           \
+        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
+        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
+        T* sd = reinterpret_cast<T*>(c->sigma);                                                                          \
+        return host_call(c, {{abd.p, ab, abd.bytes}},                                                                    \
+                         [&](cudaEvent_t* mk) { return packed_chain<T>(c, (const T*)abd.p, n, band, dd, ed, sd, mk); },  \
+                         {{sigma, sd, sizeof(T) * n}}, 6);                                                               \
     }                                                                                                                    \
     int svdb200_band_svdvals_packed_dev_##S(svdb200_handle h, const T* ab, size_t n, size_t band, T* sigma) {            \
         SVDB_ENTER(T)                                                                                                    \
         if (!ab || !sigma) return SVDB200_E_ARG;                                                                         \
         SVDB_TRY(check_packed(c, n, band));                                                                              \
-        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
-        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
-        SVDB_TRY(stage2_chase_packed<T>(c, ab, n, band, dd, ed));                                                        \
-        return bidiag_qr<T>(c, dd, ed, n, sigma);                                                                        \
+        return packed_chain<T>(c, ab, n, band, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), sigma, nullptr);  \
     }                                                                                                                    \
     int svdb200_bidiag_qr_##S(svdb200_handle h, const T* d, const T* e, size_t n, T* sigma, long long* sweeps) {         \
         SVDB_ENTER(T)                                                                                                    \
         if (!d || !e || !sigma) return SVDB200_E_ARG;                                                                    \
         if (n < 2) return SVDB200_E_SHAPE;                                                                               \
         if (n > c->max_n) return SVDB200_E_CAPACITY;                                                                     \
-        return host_chain<T>(c, nullptr, n, 1, 0, 4, const_cast<T*>(d), const_cast<T*>(e), sigma, sweeps);               \
+        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
+        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
+        T* sd = reinterpret_cast<T*>(c->sigma);                                                                          \
+        return host_call(c, {{dd, d, sizeof(T) * n}, {ed, e, sizeof(T) * (n - 1)}},                                      \
+                         [&](cudaEvent_t* mk) { return run_chain<T>(c, (T*)nullptr, n, n, 1, SVDB200_ORDER_PANEL, 4, dd, ed, sd, mk); }, \
+                         {{sigma, sd, sizeof(T) * n}}, 4, sweeps);                                                       \
     }                                                                                                                    \
     int svdb200_bidiag_qr_dev_##S(svdb200_handle h, T* d, T* e, size_t n, T* sigma) {                                    \
         SVDB_ENTER(T)                                                                                                    \
@@ -960,42 +957,30 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        return host_chain<T>(c, a, n, band, order, 3, d, e, nullptr, nullptr);                                           \
+        return dense_host<T>(c, a, n, n, band, order, 3, d, e, nullptr);                                                 \
     }                                                                                                                    \
     int svdb200_bidiagonalize_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, int order, T* d, T* e) {  \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        SVDB_TRY(stage1_dispatch<T>(c, a, n, band, order));                                                              \
-        return stage2_chase<T>(c, a, n, band, d, e);                                                                     \
+        return run_chain<T>(c, a, n, n, band, order, 3, d, e, nullptr, nullptr);                                         \
     }                                                                                                                    \
     int svdb200_bidiagonalize_onestage_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, T* d, T* e) {                 \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
-        c->onestage = 1;                                                                                                 \
-        const int st = stage1_panel_order<T>(c, a, n, n, 1);                                                              \
-        c->onestage = 0;                                                                                                 \
-        if (st != 0) return st;                                                                                          \
-        return extract_bidiagonal<T>(c, a, n, d, e);                                                                     \
+        return onestage_chain<T>(c, a, n, d, e, nullptr);                                                                \
     }                                                                                                                    \
     int svdb200_bidiagonalize_onestage_##S(svdb200_handle h, T* a, size_t m, size_t n, T* d, T* e) {                     \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_square(c, m, n, 1, dtype_of<T>()));                                                               \
-        SVDB_TRY(ensure_staging(c));                                                                                     \
-        T* ad = reinterpret_cast<T*>(c->a_dev);                                                                          \
-        SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream));                     \
-        c->onestage = 1;                                                                                                 \
-        int st = stage1_panel_order<T>(c, ad, n, n, 1);                                                                   \
-        c->onestage = 0;                                                                                                 \
-        if (st == 0) st = extract_bidiagonal<T>(c, ad, n, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e));       \
-        if (st != 0) return st;                                                                                          \
-        SVDB_CHECK(c, cudaMemcpyAsync(a, ad, sizeof(T) * n * n, cudaMemcpyDeviceToHost, c->stream));                     \
-        if (d) SVDB_CHECK(c, cudaMemcpyAsync(d, c->d, sizeof(T) * n, cudaMemcpyDeviceToHost, c->stream));                \
-        if (e && n > 1) SVDB_CHECK(c, cudaMemcpyAsync(e, c->e, sizeof(T) * (n - 1), cudaMemcpyDeviceToHost, c->stream)); \
-        SVDB_CHECK(c, cudaStreamSynchronize(c->stream));                                                                 \
-        return 0;                                                                                                        \
+        SVDB_TRY(reserve(c, c->a_dev, c->esz * c->max_n * c->max_n));                                                    \
+        T* ad = reinterpret_cast<T*>(c->a_dev.p);                                                                        \
+        T* dd = reinterpret_cast<T*>(c->d);                                                                              \
+        T* ed = reinterpret_cast<T*>(c->e);                                                                              \
+        return host_call(c, {{ad, a, sizeof(T) * n * n}}, [&](cudaEvent_t* mk) { return onestage_chain<T>(c, ad, n, dd, ed, mk); }, \
+                         {{a, ad, sizeof(T) * n * n}, {d, dd, sizeof(T) * n}, {e, ed, sizeof(T) * (n - 1)}}, 1);         \
     }                                                                                                                    \
     int svdb200_bidiagonalize_many_dev_##S(svdb200_handle h, size_t count, T* const* a, const size_t* n, size_t band,    \
                                            int order, T* const* d, T* const* e) {                                        \
@@ -1021,51 +1006,49 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        return host_chain<T>(c, a, n, band, order, 7, nullptr, nullptr, sigma, nullptr);                                 \
+        return dense_host<T>(c, a, n, n, band, order, 7, nullptr, nullptr, sigma);                                       \
     }                                                                                                                    \
     int svdb200_svdvals_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, int order, T* sigma) {          \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
         SVDB_TRY(check_square(c, m, n, band, dtype_of<T>()));                                                            \
-        SVDB_TRY(stage1_dispatch<T>(c, a, n, band, order));                                                              \
-        SVDB_TRY(stage2_chase<T>(c, a, n, band, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e)));                \
-        return bidiag_qr<T>(c, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), n, sigma);                        \
+        return run_chain<T>(c, a, n, n, band, order, 7, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), sigma, nullptr); \
     }                                                                                                                    \
     int svdb200_dense_to_band_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band) {                          \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return host_chain_mn<T>(c, a, m, n, band, 1, nullptr, nullptr, nullptr);                                         \
+        return dense_host<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 1, nullptr, nullptr, nullptr);                       \
     }                                                                                                                    \
     int svdb200_dense_to_band_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band) {                      \
         SVDB_ENTER(T)                                                                                                    \
         if (!a) return SVDB200_E_ARG;                                                                                    \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return rect_chain<T>(c, a, m, n, band, 1, nullptr, nullptr, nullptr, nullptr);                                   \
+        return run_chain<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 1, nullptr, nullptr, nullptr, nullptr);               \
     }                                                                                                                    \
     int svdb200_bidiagonalize_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {              \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !d || !e) return SVDB200_E_ARG;                                                                        \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return host_chain_mn<T>(c, a, m, n, band, 3, d, e, nullptr);                                                     \
+        return dense_host<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 3, d, e, nullptr);                                   \
     }                                                                                                                    \
     int svdb200_bidiagonalize_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* d, T* e) {          \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !d || !e) return SVDB200_E_ARG;                                                                        \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return rect_chain<T>(c, a, m, n, band, 3, d, e, nullptr, nullptr);                                               \
+        return run_chain<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 3, d, e, nullptr, nullptr);                           \
     }                                                                                                                    \
     int svdb200_svdvals_mn_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* sigma) {                      \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return host_chain_mn<T>(c, a, m, n, band, 7, nullptr, nullptr, sigma);                                           \
+        return dense_host<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 7, nullptr, nullptr, sigma);                         \
     }                                                                                                                    \
     int svdb200_svdvals_mn_dev_##S(svdb200_handle h, T* a, size_t m, size_t n, size_t band, T* sigma) {                  \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
         SVDB_TRY(check_mn(c, m, n, band));                                                                               \
-        return rect_chain<T>(c, a, m, n, band, 7, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), sigma, nullptr); \
+        return run_chain<T>(c, a, m, n, band, SVDB200_ORDER_PANEL, 7, reinterpret_cast<T*>(c->d), reinterpret_cast<T*>(c->e), sigma, nullptr); \
     }                                                                                                                    \
     int svdb200_svdvals_batched_dev_##S(svdb200_handle h, T* a, size_t count, size_t n, size_t band, T* sigma) {         \
         SVDB_ENTER(T)                                                                                                    \
@@ -1077,21 +1060,17 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
         SVDB_TRY(check_square(c, n, n, band, dtype_of<T>()));                                                            \
-        T *ad = nullptr, *sd = nullptr;                                                                                  \
-        SVDB_CHECK(c, cudaMalloc(&ad, sizeof(T) * count * n * n));                                                       \
-        cudaError_t e2 = cudaMalloc(&sd, sizeof(T) * count * n);                                                         \
-        if (e2 != cudaSuccess) { cudaFree(ad); return cuda_status(c, e2, "cudaMalloc"); }                                \
-        int st = 0;                                                                                                      \
-        cudaError_t ce = cudaMemcpyAsync(ad, a, sizeof(T) * count * n * n, cudaMemcpyHostToDevice, c->stream);           \
-        if (ce == cudaSuccess) st = batched_svdvals<T>(c, ad, count, n, band, sd);                                       \
-        if (ce == cudaSuccess && st == 0) ce = cudaMemcpyAsync(sigma, sd, sizeof(T) * count * n, cudaMemcpyDeviceToHost, c->stream); \
-        if (ce == cudaSuccess && st == 0) ce = cudaMemcpyAsync(a, ad, sizeof(T) * count * n * n, cudaMemcpyDeviceToHost, c->stream); \
-        cudaError_t se = cudaStreamSynchronize(c->stream);                                                               \
-        cudaFree(ad); cudaFree(sd);                                                                                      \
-        if (st) return st;                                                                                               \
-        if (ce != cudaSuccess) return cuda_status(c, ce, "batched copy");                                                \
-        if (se != cudaSuccess) return cuda_status(c, se, "batched sync");                                                \
-        return 0;                                                                                                        \
+        DevBuf ad, sd;                                     /* per call: the handle does not keep count n^2 elements */   \
+        SVDB_TRY(reserve(c, ad, sizeof(T) * count * n * n));                                                             \
+        SVDB_TRY(reserve(c, sd, sizeof(T) * count * n));                                                                 \
+        /* the driver interleaves the stages of different matrices: what = 0, only the copies are timed */               \
+        return host_call(c, {{ad.p, a, ad.bytes}},                                                                       \
+                         [&](cudaEvent_t* mk) {                                                                          \
+                             SVDB_TRY(batched_svdvals<T>(c, (T*)ad.p, count, n, band, (T*)sd.p));                        \
+                             for (int k = 0; k < 4; ++k) SVDB_TRY(mark(c, mk, k));                                       \
+                             return 0;                                                                                   \
+                         },                                                                                              \
+                         {{sigma, sd.p, sd.bytes}, {a, ad.p, ad.bytes}}, 0);                                             \
     }                                                                                                                    \
     int svdb200_chain_batched_dev_##S(svdb200_handle h, T* a, size_t count, size_t n, size_t band, int what, T* d, T* e, T* sigma) { \
         SVDB_ENTER(T)                                                                                                    \
@@ -1102,22 +1081,20 @@ int svdb200_synchronize(svdb200_handle h) {
     int svdb200_panel_factor_dev_##S(svdb200_handle h, T* a, size_t lda, size_t m, size_t b, int trans, T* v, T* v2) {   \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !v || !v2 || m == 0 || b == 0 || b > c->band || m > c->max_n) return SVDB200_E_ARG;                    \
-        return trans ? launch_panel_public<T, true>(c, a, lda, (int)m, (int)b, v, v2, c->stream)                        \
+        return trans ? launch_panel_public<T, true>(c, a, lda, (int)m, (int)b, v, v2, c->stream)                         \
                      : launch_panel_public<T, false>(c, a, lda, (int)m, (int)b, v, v2, c->stream);                       \
     }                                                                                                                    \
     int svdb200_mse_##S(svdb200_handle h, const T* a, const T* b, size_t n, size_t band, T* out) {                       \
         SVDB_ENTER(T)                                                                                                    \
         if (!a || !b || !out || n == 0 || band == 0) return SVDB200_E_ARG;                                               \
         if (n > c->max_n) return SVDB200_E_CAPACITY;                                                                     \
-        SVDB_TRY(ensure_staging(c));                                                                                     \
-        T* ad = reinterpret_cast<T*>(c->a_dev);                                                                          \
-        T* bd = nullptr;                                                                                                 \
-        SVDB_CHECK(c, cudaMalloc(&bd, sizeof(T) * n * n));                                                               \
-        cudaMemcpyAsync(ad, a, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream);                                    \
-        cudaMemcpyAsync(bd, b, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream);                                    \
-        int st = mse_metric<T>(c, ad, bd, n, band, out);                                                                 \
-        cudaFree(bd);                                                                                                    \
-        return st;                                                                                                       \
+        SVDB_TRY(reserve(c, c->a_dev, c->esz * c->max_n * c->max_n));                                                    \
+        T* ad = reinterpret_cast<T*>(c->a_dev.p);                                                                        \
+        DevBuf bd;                                                                                                       \
+        SVDB_TRY(reserve(c, bd, sizeof(T) * n * n));                                                                     \
+        SVDB_CHECK(c, cudaMemcpyAsync(ad, a, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream));                     \
+        SVDB_CHECK(c, cudaMemcpyAsync(bd.p, b, sizeof(T) * n * n, cudaMemcpyHostToDevice, c->stream));                   \
+        return mse_metric<T>(c, ad, (const T*)bd.p, n, band, out);                                                       \
     }                                                                                                                    \
     int svdb200_fill_uniform_dev_##S(svdb200_handle h, T* a, size_t count, unsigned long long seed, double lo, double hi) { \
         SVDB_ENTER(T)                                                                                                    \

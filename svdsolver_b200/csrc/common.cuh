@@ -29,6 +29,16 @@ struct Settings {
     double chol_guard = 1e-3;               // smallest accepted pivot ratio R_jj^2 / G_jj; below, the exchange-based kernels redo the panel
 };
 
+// Device buffer allocated after svdb200_create, on first use or grown by reserve(); freed with its owner.
+struct DevBuf {
+    void* p = nullptr;
+    size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
+};
+
 struct Ctx {
     int device = 0;
     int dtype = SVDB200_F64;
@@ -36,7 +46,7 @@ struct Ctx {
     int num_sms = 148;
     cudaStream_t own_stream = nullptr, stream = nullptr;
     // device workspace (element type = dtype)
-    void* a_dev = nullptr;         // max_n * max_n : staging for host-pointer calls
+    DevBuf a_dev;                  // max_n * max_n : staging for host-pointer calls (first use)
     void* v = nullptr;             // max_n * band  : V (QR) / U^T (LQ), row-major, unit diagonal explicit
     void* v2 = nullptr;            // max_n * band  : V S^T (QR) ; band * max_n : S U (LQ)
     void* vb = nullptr; void* v2b = nullptr;   // second reflector pair (LQ panels) for the look-ahead
@@ -52,9 +62,8 @@ struct Ctx {
     void* red2 = nullptr;          // blocked panel kernel: flag-stamped words exchanged between clusters through L2 (512 KB)
     unsigned int* bar = nullptr;   // software grid barrier state (2 words) + misc counters
     int* prog = nullptr;           // stage-2 per-sweep progress counters (max_n)
-    void* band_ws = nullptr;       // max_n * 3 band: stage 2 from band storage, packed 3-band-diagonal layout (first use)
-    void* rect_ws = nullptr;       // m * n: A^T of a wide m x n matrix (m < n), reduced there; grown on demand
-    size_t rect_ws_elems = 0;
+    DevBuf band_ws;                // max_n * 3 band: stage 2 from band storage, packed 3-band-diagonal layout (first use)
+    DevBuf rect_ws;                // m * n: A^T of a wide m x n matrix (m < n), reduced there; grown on demand
     void* d = nullptr; void* e = nullptr; void* sigma = nullptr;   // max_n each
     long long* qr_info = nullptr;  // [0] sweeps, [1] status
     void* tileq = nullptr;         // tile order: per-chain-step Q matrices, (max_n/band) * 4*band*band
@@ -76,8 +85,7 @@ struct Ctx {
     std::vector<Ctx*> pool;
     size_t pool_n = 0, pool_band = 0;
     // tcgen05 FP32 path (gemm_tc05.cu): hi/lo split scratch for the O(n b) operands, allocated on first use
-    void* tcsplit = nullptr;
-    size_t tcsplit_elems = 0;
+    DevBuf tcsplit;
     Settings cfg;
     // pipelined multi-matrix driver (bidiagonalize_many): stage 2 of matrix i on s2_stream beside stage 1 of matrix i+1
     static constexpr int kLanes = 2;        // chains in flight: each = one stage 1 (own sub-handle) and one stage-2 kernel
@@ -94,14 +102,11 @@ struct Ctx {
     Ctx* s1ctx[kLanes] = {};                // sub-handles (own workspace + streams): stage 1 of two matrices at a time
     void* a_stage[2 * kLanes] = {};         // staging buffers + bidiagonal rows for the host-pointer variant
     void* de2 = nullptr;
-    void* bis_ws = nullptr;
-    size_t bis_ws_elems = 0;
+    DevBuf bis_ws;                             // bisection workspace: params + 2 * max_n squared off-diagonals (double)
     std::vector<void*> band_capture;           // test hook of bidiagonalize_many_*: device buffers that receive matrix i's band
     // batched small-matrix driver: per-matrix progress counters, reflector / W workspaces, d / e rows
-    int* batch_prog = nullptr;
-    size_t batch_prog_elems = 0;
-    void* batch_ws = nullptr;
-    size_t batch_ws_bytes = 0;                 // bisection workspace: params + 2 * max_n squared off-diagonals (double)
+    DevBuf batch_prog;
+    DevBuf batch_ws;
 };
 
 // Brackets one kernel launch with events when profiling is on (serialises host and device; the
@@ -139,6 +144,21 @@ inline int cuda_status(Ctx* c, cudaError_t e, const char* what) {
         int _s = (expr);               \
         if (_s != 0) return _s;        \
     } while (0)
+
+// At least `bytes` in b: returns at once when b is big enough; otherwise b is replaced by an allocation of exactly `bytes`
+// (after the handle's stream has finished, since work enqueued earlier may still use the old buffer).
+inline int reserve(Ctx* c, DevBuf& b, size_t bytes) {
+    if (b.bytes >= bytes) return 0;
+    if (b.p) {
+        SVDB_CHECK(c, cudaStreamSynchronize(c->stream));
+        SVDB_CHECK(c, cudaFree(b.p));
+        b.p = nullptr;
+        b.bytes = 0;
+    }
+    SVDB_CHECK(c, cudaMalloc(&b.p, bytes));
+    b.bytes = bytes;
+    return 0;
+}
 
 // ---- exactly-rounded, never-contracted arithmetic for the bit-faithful kernels -------------------
 // (the reference is compiled without FMA contraction: ISO C++ mode => -ffp-contract=off; SURVEY 0.7)
@@ -214,8 +234,7 @@ template <typename T> int bidiag_qr(Ctx* c, T* d, T* e, size_t n, T* sigma);
 template <typename T> int bidiag_bisect(Ctx* c, const T* d, const T* e, size_t n, T* sigma);
 template <typename T> int bidiag_sqr(Ctx* c, T* d, T* e, size_t n, T* sigma);
 template <typename T> int stage1_panel_order(Ctx* c, T* a, size_t rows, size_t n, size_t band);   // a: rows x n, rows >= n
-// m x n (either orientation) through stage 1 / stage 2 / singular values; rect.cu
-template <typename T> int rect_chain(Ctx* c, T* a, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma, cudaEvent_t* marks);
+template <typename T> int transpose(Ctx* c, const T* src, size_t rows, size_t cols, T* dst);        // rect.cu
 template <typename T> int stage1_tile_order(Ctx* c, T* a, size_t n, size_t band);
 template <typename T> int gemm_tn(Ctx* c, const T* v, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, T* w);
 template <typename T> int gemm_nn(Ctx* c, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, const T* ut, T* w);

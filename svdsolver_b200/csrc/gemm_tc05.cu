@@ -692,12 +692,7 @@ static int make_map(Ctx* c, CUtensorMap* m, const float* ptr, size_t rows, size_
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-static int ensure_scratch(Ctx* c) {
-    if (c->tcsplit) return 0;
-    c->tcsplit_elems = 4 * (c->max_n + 64) * c->band + 1024;
-    SVDB_CHECK(c, cudaMalloc(&c->tcsplit, sizeof(float) * c->tcsplit_elems));
-    return 0;
-}
+static int ensure_scratch(Ctx* c) { return reserve(c, c->tcsplit, sizeof(float) * (4 * (c->max_n + 64) * c->band + 1024)); }
 
 static int launch_split(Ctx* c, const float* src, size_t ld_src, int rows, int cols, float* hi, float* lo, size_t ld_dst) {
     const size_t total = (size_t)rows * cols;
@@ -733,11 +728,11 @@ int rank_update_tc05<float>(Ctx* c, float* cm, size_t ldc, int M, int N, int K, 
     if (!wanted(c, M, N, K) || !aligned16(cm) || (ldc & 3)) return 1;
     SVDB_TRY(ensure_scratch(c));
     const size_t ldn = ((size_t)N + 3) & ~(size_t)3;
-    float* ph = reinterpret_cast<float*>(c->tcsplit);
+    float* ph = reinterpret_cast<float*>(c->tcsplit.p);
     float* pl = ph + (size_t)M * K;
     float* qh = pl + (size_t)M * K;
     float* ql = qh + (size_t)K * ldn;
-    if ((size_t)(ql + (size_t)K * ldn - ph) > c->tcsplit_elems) return 1;
+    if ((size_t)(ql + (size_t)K * ldn - ph) > c->tcsplit.bytes / sizeof(float)) return 1;
     SVDB_TRY(launch_split(c, p, (size_t)K, M, K, ph, pl, (size_t)K));
     SVDB_TRY(launch_split(c, q, ldq, K, N, qh, ql, ldn));
     CUtensorMap tC, tPh, tPl, tQh, tQl;
@@ -785,9 +780,9 @@ static int gemm_common(Ctx* c, int mode, const float* cm, size_t ldc, int M, int
     if (!wanted(c, M, N, B) || !aligned16(cm) || (ldc & 3)) return 1;
     SVDB_TRY(ensure_scratch(c));
     const int xrows = mode == 0 ? N : M;
-    float* xh = reinterpret_cast<float*>(c->tcsplit);
+    float* xh = reinterpret_cast<float*>(c->tcsplit.p);
     float* xl = xh + (size_t)xrows * B;
-    if ((size_t)2 * xrows * B > c->tcsplit_elems) return 1;
+    if ((size_t)2 * xrows * B > c->tcsplit.bytes / sizeof(float)) return 1;
     SVDB_TRY(launch_split(c, x, (size_t)B, xrows, B, xh, xl, (size_t)B));
     const int ktot = mode == 0 ? N : M;
     const int tiles = ((mode == 0 ? M : N) + 127) / 128;

@@ -241,14 +241,8 @@ int stage2_run(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
     const long long grid = groups * G;
     int* prog = c->prog;
     if (count > 1) {
-        const size_t need = (size_t)count * n;
-        if (c->batch_prog_elems < need) {
-            if (c->batch_prog) cudaFree(c->batch_prog);
-            c->batch_prog = nullptr; c->batch_prog_elems = 0;
-            SVDB_CHECK(c, cudaMalloc(&c->batch_prog, sizeof(int) * need));
-            c->batch_prog_elems = need;
-        }
-        prog = c->batch_prog;
+        SVDB_TRY(reserve(c, c->batch_prog, sizeof(int) * count * n));
+        prog = reinterpret_cast<int*>(c->batch_prog.p);
     }
     SVDB_CHECK(c, cudaMemsetAsync(prog, 0, sizeof(int) * n * (size_t)count, c->stream));
     int ni = (int)n, bi = cb, cnt = count, gi = (int)G, complete = c->cfg.stage2_complete;
@@ -281,8 +275,8 @@ template <typename T>
 int stage2_chase_packed(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e) {
     if (n < 2 || band < 1) return SVDB200_E_SHAPE;
     if (n > c->max_n || band > c->band) return SVDB200_E_CAPACITY;
-    if (!c->band_ws) SVDB_CHECK(c, cudaMalloc(&c->band_ws, c->esz * c->max_n * 3 * c->band));
-    T* w = reinterpret_cast<T*>(c->band_ws);
+    SVDB_TRY(reserve(c, c->band_ws, c->esz * c->max_n * 3 * c->band));
+    T* w = reinterpret_cast<T*>(c->band_ws.p);
     const size_t total = n * 3 * band;
     const unsigned blocks = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)c->num_sms * 16);
     pack_band_kernel<T><<<blocks, 256, 0, c->stream>>>(ab, (int)n, (int)band, w);
