@@ -202,6 +202,29 @@ int svdb200_svdvals_batched_dev_f64(svdb200_handle h, double* a_dev, size_t coun
  * n <= 1024, band <= 64 (the range of the one-launch-per-step batched kernels). */
 int svdb200_chain_batched_dev_f32(svdb200_handle h, float* a_dev, size_t count, size_t n, size_t band, int what, float* d_dev, float* e_dev, float* sigma_dev);
 int svdb200_chain_batched_dev_f64(svdb200_handle h, double* a_dev, size_t count, size_t n, size_t band, int what, double* d_dev, double* e_dev, double* sigma_dev);
+
+/* Batched rectangular matrices: `count` m x n row-major matrices back to back (stride m * n); with k = min(m, n), sigma
+ * is count x k (each row descending), d and e are count x k (rows of length k; the last entry of an e row is unused).
+ * `a` is overwritten as by the single-matrix _mn calls (LAPACK gebrd's convention: upper band / bidiagonal in the top
+ * n x n block for m >= n, lower band / bidiagonal in the left m x m block for m < n, e then the sub-diagonal).  With m == n
+ * the results are byte for byte those of svdb200_svdvals_batched_* / svdb200_chain_batched_dev_*.
+ * The one-launch-per-step batched kernels take k <= 1024, band <= 64 and a tallest panel (max(m, n) rows) that fits the
+ * batched panel's cluster shared memory (about 2500 rows in f64 at band 64, 5800 at band 32); this is decided before
+ * anything is enqueued.  Outside that range svdvals_batched_mn runs the single-matrix chain once per matrix, one after
+ * the other, with the bytes and the handle settings of svdb200_svdvals_mn_dev_*; chain_batched_mn_dev returns
+ * SVDB200_E_CAPACITY and leaves `a` untouched.  what (chain call): 1 stage 1, 2 stage 2, 4 singular values, each bit its
+ * own stage only (stage 2 alone of a wide batch takes the lower band stage 1 left).
+ * Statuses: SVDB200_E_ARG for a null pointer, a dtype mismatch, what outside 1..7 or bit 4 without sigma; the shape and
+ * capacity rules of the _mn calls; count == 0 returns 0 and does nothing.  The host variant allocates its device buffers
+ * per call. */
+int svdb200_svdvals_batched_mn_f32(svdb200_handle h, float* a, size_t count, size_t m, size_t n, size_t band, float* sigma);
+int svdb200_svdvals_batched_mn_f64(svdb200_handle h, double* a, size_t count, size_t m, size_t n, size_t band, double* sigma);
+int svdb200_svdvals_batched_mn_dev_f32(svdb200_handle h, float* a_dev, size_t count, size_t m, size_t n, size_t band, float* sigma_dev);
+int svdb200_svdvals_batched_mn_dev_f64(svdb200_handle h, double* a_dev, size_t count, size_t m, size_t n, size_t band, double* sigma_dev);
+int svdb200_chain_batched_mn_dev_f32(svdb200_handle h, float* a_dev, size_t count, size_t m, size_t n, size_t band, int what,
+                                     float* d_dev, float* e_dev, float* sigma_dev);
+int svdb200_chain_batched_mn_dev_f64(svdb200_handle h, double* a_dev, size_t count, size_t m, size_t n, size_t band, int what,
+                                     double* d_dev, double* e_dev, double* sigma_dev);
 /* Test hook for svdb200_bidiagonalize_many_*: dev_bufs[i] (device, n[i] x n[i] elements, or NULL) receives the band
  * matrix with which matrix i of the NEXT many-call enters stage 2; cleared by that call. */
 int svdb200_set_band_capture(svdb200_handle h, void* const* dev_bufs, size_t count);
@@ -210,7 +233,7 @@ int svdb200_set_band_capture(svdb200_handle h, void* const* dev_bufs, size_t cou
  * Device time (CUDA events on the handle's stream) of the stages of the LAST host-pointer compute call
  * (not the list calls), ms: h2d, d2h and every stage the call ran (stage 1 includes the transposes of a
  * wide matrix and the one-stage reduction); a stage the call did not run reports exactly 0.
- * svdvals_batched interleaves the stages of its matrices and reports only h2d and d2h.
+ * svdvals_batched and svdvals_batched_mn interleave the stages of their matrices and report only h2d and d2h.
  * stage-1 sub-times: panel factorisations vs trailing updates are reported by svdb200_stage1_profile. */
 int svdb200_last_timings(svdb200_handle h, double* ms_stage1, double* ms_stage2, double* ms_qr, double* ms_h2d, double* ms_d2h);
 /* Per-kernel-class profiling.  When on, every launch of the hot-path kernels is bracketed by CUDA

@@ -255,6 +255,14 @@ class Handle:
         self._check(self._fn("svdvals_batched")(self.h, _p(a), Z(count), Z(n), Z(band), _p(sigma)))
         return sigma
 
+    def svdvals_batched_mn(self, a, band):
+        """singular values of count m x n matrices (a: count x m x n): returns sigma, count x min(m, n), rows descending"""
+        a = np.ascontiguousarray(a, dtype=self.dtype).copy()
+        count, m, n = a.shape
+        sigma = np.zeros((count, min(m, n)), self.dtype)
+        self._check(self._fn("svdvals_batched_mn")(self.h, _p(a), Z(count), Z(m), Z(n), Z(band), _p(sigma)))
+        return sigma
+
     def mse(self, a, b, band):
         a = np.ascontiguousarray(a, dtype=self.dtype)
         b = np.ascontiguousarray(b, dtype=self.dtype)
@@ -302,6 +310,15 @@ class Handle:
     def chain_batched_dev(self, a_ptr, count, n, band, what, d_ptr=None, e_ptr=None, sigma_ptr=None):
         """stages of the batched path: what = 1 stage 1 | 2 stage 2 | 4 singular values"""
         self._check(self._fn("chain_batched_dev")(self.h, _p(a_ptr), Z(count), Z(n), Z(band), ctypes.c_int(what), _p(d_ptr), _p(e_ptr), _p(sigma_ptr)))
+
+    def svdvals_batched_mn_dev(self, a_ptr, count, m, n, band, sigma_ptr):
+        self._check(self._fn("svdvals_batched_mn_dev")(self.h, _p(a_ptr), Z(count), Z(m), Z(n), Z(band), _p(sigma_ptr)))
+
+    def chain_batched_mn_dev(self, a_ptr, count, m, n, band, what, d_ptr=None, e_ptr=None, sigma_ptr=None):
+        """stages of the batched path on count m x n matrices: what = 1 stage 1 | 2 stage 2 | 4 singular values; d, e, sigma
+        count x min(m, n)"""
+        self._check(self._fn("chain_batched_mn_dev")(self.h, _p(a_ptr), Z(count), Z(m), Z(n), Z(band), ctypes.c_int(what),
+                                                     _p(d_ptr), _p(e_ptr), _p(sigma_ptr)))
 
     def set_band_capture(self, dev_ptrs):
         """test hook: device buffers that receive the band of matrix i of the next bidiagonalize_many_* call"""

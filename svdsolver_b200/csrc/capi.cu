@@ -190,65 +190,83 @@ constexpr int kBatchPool = 16;
 // not only those set after the sub-handle was created.
 static void inherit_settings(const Ctx* c, Ctx* s) { s->cfg = c->cfg; }
 
-// Small matrices (n <= 1024, band <= 64): every kernel of the path runs ONCE PER STEP FOR THE WHOLE BATCH -- a
+// Small matrices (min(m, n) <= 1024, band <= 64): every kernel of the path runs ONCE PER STEP FOR THE WHOLE BATCH -- a
 // thread-block cluster per matrix for the panels (panel resident in cluster shared memory), one grid slice per
 // matrix for the three update GEMMs, groups of CTAs that pipeline the sweeps of one matrix each for stage 2, one
 // thread per singular value for the bisection -- instead of ~80 launches per matrix.  The matrices of a chunk stay
-// L2 / HBM resident; workspace is (5 n b + 2 n) elements per matrix of the chunk.
+// L2 / HBM resident.  `a` holds count m x n matrices back to back; with k = min(m, n), the rows of d, e and sigma have
+// length k.  Tall (m >= n): the QR panels of step j span rows j .. m-1 (as in stage1_panel_order), and stage 2 and sigma
+// run on the top k x k block, which is upper band.  Wide (m < n): each A^T is reduced as tall in the chunk's workspace and
+// transposed back, so `a` ends in gebrd's lower form (as in run_chain).  Workspace per matrix of a chunk: 5 max(m, n) b
+// + 2 k elements, plus m n for A^T when m < n.
+static bool batched_in_range(const Ctx* c, size_t m, size_t n, size_t band) {
+    const size_t k = std::min(m, n);
+    return k >= 2 && k <= 1024 && band <= 64 && c->cluster_ok >= 8 && panel_batched_fits((int)std::max(m, n), (int)band, c->esz);
+}
+
 template <typename T>
-int batched_small(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma, int what = 7, T* d_out = nullptr, T* e_out = nullptr) {
+int batched_small(Ctx* c, T* a, size_t count, size_t m, size_t n, size_t band, T* sigma, int what = 7, T* d_out = nullptr,
+                  T* e_out = nullptr) {
+    if ((what & 4) && !(what & 2) && (!d_out || !e_out)) return SVDB200_E_ARG;
     const int b = (int)band;
-    const size_t per_mat = 5 * n * band + 2 * n;
+    const bool wide = m < n && (what & 3);
+    const size_t N = std::min(m, n), M = std::max(m, n);       // the tall matrices reduced: M x N, ld = N
+    const size_t sA = m * n, sV = M * band;
+    const size_t per_mat = 5 * sV + 2 * N + (wide ? sA : 0);
     size_t chunk = std::min<size_t>(count, 8192);
     while (chunk > 1 && chunk * per_mat * sizeof(T) > ((size_t)2 << 30)) chunk = (chunk + 1) / 2;
     SVDB_TRY(reserve(c, c->batch_ws, chunk * per_mat * sizeof(T)));
-    const size_t sV = n * band, sA = n * n;
     T* Vq = reinterpret_cast<T*>(c->batch_ws.p);
     T* V2q = Vq + chunk * sV;
     T* Vl = V2q + chunk * sV;
     T* V2l = Vl + chunk * sV;
     T* W = V2l + chunk * sV;
     T* dall = W + chunk * sV;
-    T* eall = dall + chunk * n;
+    T* eall = dall + chunk * N;
+    T* xt = eall + chunk * N;                                  // wide: the chunk's A^T
     for (size_t z0 = 0; z0 < count; z0 += chunk) {
         const int cnt = (int)std::min(chunk, count - z0);
-        T* a0 = a + z0 * sA;
-        for (size_t k = 0; (what & 1) && k < n; k += band) {   // same panel sequence as stage1_panel_order (svd_cpu.h:382-423)
-            const int m = (int)(n - k), nc = (int)(n - k - band);
-            const bool has_lq = (k + band < n - 1);
-            SVDB_TRY((panel_batched<T, false>(c, a0 + k * n + k, n, sA, m, b, Vq, V2q, sV, cnt)));
+        T* x0 = a + z0 * sA;
+        if (wide) {
+            SVDB_TRY(transpose_batched<T>(c, x0, sA, m, n, xt, sA, cnt));
+            x0 = xt;
+        }
+        for (size_t j = 0; (what & 1) && j < N; j += band) {   // same panel sequence as stage1_panel_order (svd_cpu.h:382-423)
+            const int mh = (int)(M - j), nc = (int)(N - j - band);
+            const bool has_lq = (j + band < N - 1);
+            SVDB_TRY((panel_batched<T, false>(c, x0 + j * N + j, N, sA, mh, b, Vq, V2q, sV, cnt)));
             if (nc > 0) {
-                T* A2 = a0 + k * n + k + band;
-                SVDB_TRY(gemm_tn_batched<T>(c, Vq, sV, A2, n, sA, m, nc, b, W, sV, cnt));                     // W = V^T A2
-                SVDB_TRY(rank_update_batched<T>(c, A2, n, sA, m, nc, b, V2q, sV, W, (size_t)nc, sV, cnt));     // A2 += (V S^T) W
+                T* A2 = x0 + j * N + j + band;
+                SVDB_TRY(gemm_tn_batched<T>(c, Vq, sV, A2, N, sA, mh, nc, b, W, sV, cnt));                    // W = V^T A2
+                SVDB_TRY(rank_update_batched<T>(c, A2, N, sA, mh, nc, b, V2q, sV, W, (size_t)nc, sV, cnt));    // A2 += (V S^T) W
                 if (has_lq) {
-                    SVDB_TRY((panel_batched<T, true>(c, A2, n, sA, nc, b, Vl, V2l, sV, cnt)));                // LQ of the row panel
-                    const int mr = m - b;
+                    SVDB_TRY((panel_batched<T, true>(c, A2, N, sA, nc, b, Vl, V2l, sV, cnt)));               // LQ of the row panel
+                    const int mr = mh - b;
                     if (mr > 0) {
-                        T* A3 = a0 + (k + band) * n + k + band;
-                        SVDB_TRY(gemm_nn_batched<T>(c, A3, n, sA, mr, nc, b, Vl, sV, W, sV, cnt));             // W = A3 U^T
-                        SVDB_TRY(rank_update_batched<T>(c, A3, n, sA, mr, nc, b, W, sV, V2l, (size_t)nc, sV, cnt));
+                        T* A3 = x0 + (j + band) * N + j + band;
+                        SVDB_TRY(gemm_nn_batched<T>(c, A3, N, sA, mr, nc, b, Vl, sV, W, sV, cnt));            // W = A3 U^T
+                        SVDB_TRY(rank_update_batched<T>(c, A3, N, sA, mr, nc, b, W, sV, V2l, (size_t)nc, sV, cnt));
                     }
                 }
             }
         }
         if (what & 2) {
-            SVDB_TRY(stage2_chase_batched<T>(c, a0, n, band, dall, eall, cnt));
-            if (d_out) SVDB_CHECK(c, cudaMemcpyAsync(d_out + z0 * n, dall, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
-            if (e_out) SVDB_CHECK(c, cudaMemcpyAsync(e_out + z0 * n, eall, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
+            SVDB_TRY(stage2_chase_batched<T>(c, x0, sA, N, band, dall, eall, cnt));
+            if (d_out) SVDB_CHECK(c, cudaMemcpyAsync(d_out + z0 * N, dall, sizeof(T) * N * cnt, cudaMemcpyDeviceToDevice, c->stream));
+            if (e_out) SVDB_CHECK(c, cudaMemcpyAsync(e_out + z0 * N, eall, sizeof(T) * N * cnt, cudaMemcpyDeviceToDevice, c->stream));
         }
+        if (wide) SVDB_TRY(transpose_batched<T>(c, xt, sA, n, m, a + z0 * sA, sA, cnt));
         if (!(what & 4)) continue;
         if (!(what & 2)) {                                // sigma of caller-provided bidiagonals
-            if (!d_out || !e_out) return SVDB200_E_ARG;
-            SVDB_CHECK(c, cudaMemcpyAsync(dall, d_out + z0 * n, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
-            SVDB_CHECK(c, cudaMemcpyAsync(eall, e_out + z0 * n, sizeof(T) * n * cnt, cudaMemcpyDeviceToDevice, c->stream));
+            SVDB_CHECK(c, cudaMemcpyAsync(dall, d_out + z0 * N, sizeof(T) * N * cnt, cudaMemcpyDeviceToDevice, c->stream));
+            SVDB_CHECK(c, cudaMemcpyAsync(eall, e_out + z0 * N, sizeof(T) * N * cnt, cudaMemcpyDeviceToDevice, c->stream));
         }
         if (c->cfg.qr_method == 1) {                      // the reference's zero-shift QR sweeps, one CTA per matrix
-            for (int i = 0; i < cnt; ++i) SVDB_TRY(bidiag_qr<T>(c, dall + (size_t)i * n, eall + (size_t)i * n, n, sigma + (z0 + i) * n));
+            for (int i = 0; i < cnt; ++i) SVDB_TRY(bidiag_qr<T>(c, dall + (size_t)i * N, eall + (size_t)i * N, N, sigma + (z0 + i) * N));
         } else {
             for (int i0 = 0; i0 < cnt; i0 += 32768) {
                 const int ic = std::min(32768, cnt - i0);
-                SVDB_TRY(bidiag_bisect_batched<T>(c, dall + (size_t)i0 * n, eall + (size_t)i0 * n, n, sigma + (z0 + i0) * n, ic));
+                SVDB_TRY(bidiag_bisect_batched<T>(c, dall + (size_t)i0 * N, eall + (size_t)i0 * N, N, sigma + (z0 + i0) * N, ic));
             }
         }
     }
@@ -258,7 +276,7 @@ int batched_small(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma, i
 template <typename T>
 int batched_svdvals(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma) {
     if (count == 0) return 0;
-    if (n <= 1024 && band <= 64 && c->cluster_ok >= 8 && n >= 2) return batched_small<T>(c, a, count, n, band, sigma);
+    if (batched_in_range(c, n, n, band)) return batched_small<T>(c, a, count, n, n, band, sigma);
     if (c->pool_n != n || c->pool_band != band) {
         for (auto& h : c->pool) if (h) { svdb200_destroy(reinterpret_cast<svdb200_handle>(h)); h = nullptr; }
         c->pool.clear();
@@ -298,14 +316,16 @@ int batched_svdvals(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma)
     }
     return 0;
 }
+// The stages of the batched path (m x n matrices, m == n for the square call); outside the range of its kernels there is
+// no other batched path: SVDB200_E_CAPACITY, with nothing enqueued
 template <typename T>
-int batched_chain(Ctx* c, T* a, size_t count, size_t n, size_t band, int what, T* d, T* e, T* sigma) {
+int batched_chain(Ctx* c, T* a, size_t count, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma) {
     if (count == 0) return 0;
-    if (!(n <= 1024 && band <= 64 && c->cluster_ok >= 8 && n >= 2)) return SVDB200_E_CAPACITY;
-    return batched_small<T>(c, a, count, n, band, sigma, what, d, e);
+    if (!batched_in_range(c, m, n, band)) return SVDB200_E_CAPACITY;
+    return batched_small<T>(c, a, count, m, n, band, sigma, what, d, e);
 }
-template int batched_chain<float>(Ctx*, float*, size_t, size_t, size_t, int, float*, float*, float*);
-template int batched_chain<double>(Ctx*, double*, size_t, size_t, size_t, int, double*, double*, double*);
+template int batched_chain<float>(Ctx*, float*, size_t, size_t, size_t, size_t, int, float*, float*, float*);
+template int batched_chain<double>(Ctx*, double*, size_t, size_t, size_t, size_t, int, double*, double*, double*);
 template int batched_svdvals<float>(Ctx*, float*, size_t, size_t, size_t, float*);
 template int batched_svdvals<double>(Ctx*, double*, size_t, size_t, size_t, double*);
 
@@ -626,6 +646,20 @@ int run_chain(Ctx* c, T* a, size_t m, size_t n, size_t band, int order, int what
     SVDB_TRY(mark(c, marks, 2));
     if (wide) SVDB_TRY(transpose<T>(c, x, n, m, a));
     return mark(c, marks, 3);
+}
+
+// Singular values of count m x n matrices (back to back; sigma count x min(m, n)): the batched kernels where they apply,
+// otherwise one run_chain per matrix on the handle -- the bytes of svdb200_svdvals_mn_dev_* with the handle's settings
+template <typename T>
+int batched_svdvals_mn(Ctx* c, T* a, size_t count, size_t m, size_t n, size_t band, T* sigma) {
+    if (count == 0) return 0;
+    if (batched_in_range(c, m, n, band)) return batched_small<T>(c, a, count, m, n, band, sigma);
+    const size_t k = std::min(m, n);
+    T* d = reinterpret_cast<T*>(c->d);
+    T* e = reinterpret_cast<T*>(c->e);
+    for (size_t i = 0; i < count; ++i)
+        SVDB_TRY(run_chain<T>(c, a + i * m * n, m, n, band, SVDB200_ORDER_PANEL, 7, d, e, sigma + i * k, nullptr));
+    return 0;
 }
 
 // One-stage Golub-Kahan bidiagonalisation: the stage-1 panel driver with band 1 in the one-stage order, then d, e (optional)
@@ -1076,7 +1110,35 @@ int svdb200_synchronize(svdb200_handle h) {
         SVDB_ENTER(T)                                                                                                    \
         if (!a || what <= 0 || what > 7 || ((what & 4) && !sigma)) return SVDB200_E_ARG;                                 \
         SVDB_TRY(check_square(c, n, n, band, dtype_of<T>()));                                                            \
-        return batched_chain<T>(c, a, count, n, band, what, d, e, sigma);                                                \
+        return batched_chain<T>(c, a, count, n, n, band, what, d, e, sigma);                                             \
+    }                                                                                                                    \
+    int svdb200_svdvals_batched_mn_dev_##S(svdb200_handle h, T* a, size_t count, size_t m, size_t n, size_t band, T* sigma) { \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return batched_svdvals_mn<T>(c, a, count, m, n, band, sigma);                                                    \
+    }                                                                                                                    \
+    int svdb200_svdvals_batched_mn_##S(svdb200_handle h, T* a, size_t count, size_t m, size_t n, size_t band, T* sigma) { \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || !sigma) return SVDB200_E_ARG;                                                                          \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        DevBuf ad, sd;                                     /* per call, as svdb200_svdvals_batched_* */                  \
+        SVDB_TRY(reserve(c, ad, sizeof(T) * count * m * n));                                                             \
+        SVDB_TRY(reserve(c, sd, sizeof(T) * count * std::min(m, n)));                                                    \
+        return host_call(c, {{ad.p, a, ad.bytes}},                                                                       \
+                         [&](cudaEvent_t* mk) {                                                                          \
+                             SVDB_TRY(batched_svdvals_mn<T>(c, (T*)ad.p, count, m, n, band, (T*)sd.p));                  \
+                             for (int k = 0; k < 4; ++k) SVDB_TRY(mark(c, mk, k));                                       \
+                             return 0;                                                                                   \
+                         },                                                                                              \
+                         {{sigma, sd.p, sd.bytes}, {a, ad.p, ad.bytes}}, 0);                                             \
+    }                                                                                                                    \
+    int svdb200_chain_batched_mn_dev_##S(svdb200_handle h, T* a, size_t count, size_t m, size_t n, size_t band, int what, \
+                                         T* d, T* e, T* sigma) {                                                         \
+        SVDB_ENTER(T)                                                                                                    \
+        if (!a || what <= 0 || what > 7 || ((what & 4) && !sigma)) return SVDB200_E_ARG;                                 \
+        SVDB_TRY(check_mn(c, m, n, band));                                                                               \
+        return batched_chain<T>(c, a, count, m, n, band, what, d, e, sigma);                                             \
     }                                                                                                                    \
     int svdb200_panel_factor_dev_##S(svdb200_handle h, T* a, size_t lda, size_t m, size_t b, int trans, T* v, T* v2) {   \
         SVDB_ENTER(T)                                                                                                    \

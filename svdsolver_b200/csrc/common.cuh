@@ -235,6 +235,7 @@ template <typename T> int bidiag_bisect(Ctx* c, const T* d, const T* e, size_t n
 template <typename T> int bidiag_sqr(Ctx* c, T* d, T* e, size_t n, T* sigma);
 template <typename T> int stage1_panel_order(Ctx* c, T* a, size_t rows, size_t n, size_t band);   // a: rows x n, rows >= n
 template <typename T> int transpose(Ctx* c, const T* src, size_t rows, size_t cols, T* dst);        // rect.cu
+template <typename T> int transpose_batched(Ctx* c, const T* src, size_t sS, size_t rows, size_t cols, T* dst, size_t sD, size_t count);
 template <typename T> int stage1_tile_order(Ctx* c, T* a, size_t n, size_t band);
 template <typename T> int gemm_tn(Ctx* c, const T* v, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, T* w);
 template <typename T> int gemm_nn(Ctx* c, const T* cm, size_t ldc, size_t mrows, size_t ncols, size_t b, const T* ut, T* w);
@@ -244,12 +245,13 @@ template <typename T> int rank_update_batched(Ctx* c, T* cm, size_t ldc, size_t 
 template <typename T> int gemm_tn_batched(Ctx* c, const T* v, size_t sV, const T* cm, size_t ldc, size_t sC, int M, int N, int B, T* w, size_t sW, int count);
 template <typename T> int gemm_nn_batched(Ctx* c, const T* cm, size_t ldc, size_t sC, int M, int N, int B, const T* ut, size_t sU, T* w, size_t sW, int count);
 template <typename T, bool kTrans> int panel_batched(Ctx* c, T* a, size_t lda, size_t sA, int m, int b, T* V, T* V2, size_t sV, int count);
-template <typename T> int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count);
+bool panel_batched_fits(int m, int b, size_t esz);   // panel_batched takes panels of height (or length) m at width b
+template <typename T> int stage2_chase_batched(Ctx* c, T* a, size_t sA, size_t n, size_t band, T* d, T* e, int count);
 template <typename T> int bidiag_bisect_batched(Ctx* c, const T* d, const T* e, size_t n, T* sigma, int count);
 template <typename T> int fill_uniform(Ctx* c, T* a, size_t count, unsigned long long seed, double lo, double hi);
 template <typename T> int mse_metric(Ctx* c, const T* a, const T* b, size_t n, size_t band, T* out_host);
 template <typename T> int batched_svdvals(Ctx* c, T* a, size_t count, size_t n, size_t band, T* sigma);
-template <typename T> int batched_chain(Ctx* c, T* a, size_t count, size_t n, size_t band, int what, T* d, T* e, T* sigma);
+template <typename T> int batched_chain(Ctx* c, T* a, size_t count, size_t m, size_t n, size_t band, int what, T* d, T* e, T* sigma);
 int probe_peak(Ctx* c, int kind, double* tflops);
 int probe_tc05_tf32(Ctx* c, double* tflops);
 int panel_reg_debug_read(long long* out16);

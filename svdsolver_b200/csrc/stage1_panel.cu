@@ -357,15 +357,29 @@ template int launch_panel_public<double, true>(Ctx*, double*, size_t, int, int, 
 
 // Batched panels (uniform shape): one thread-block cluster per matrix, panel resident in the cluster's shared
 // memory, all-reduce over DSMEM.  Used by the small-matrix batched driver (BASELINE configs[4]).
+// Cluster size and shared memory of a batched panel of height (QR) or length (LQ) m: <= 128 rows per CTA, few, fat CTAs
+// (many matrices share the GPU), at most 8 CTAs per cluster.
+struct PanelBatchedShape { int G, rows; size_t smem; };
+static PanelBatchedShape panel_batched_shape(int m, int b, size_t esz) {
+    int G = (m + 127) / 128;
+    if (G > 8) G = 8;
+    const int rows = (m + G - 1) / G;
+    G = (m + rows - 1) / rows;
+    return {G, rows, panel_smem_bytes(rows, b, esz)};
+}
+
+// The batched driver decides with this, before it enqueues anything, whether its tallest panel (height max(m, n) at
+// step 0) can run: the cluster's shared memory holds the panel.
+constexpr size_t kPanelBatchedSmem = 200 * 1024;
+bool panel_batched_fits(int m, int b, size_t esz) { return panel_batched_shape(m, b, esz).smem <= kPanelBatchedSmem; }
+
 template <typename T, bool kTrans>
 int panel_batched(Ctx* c, T* a, size_t lda, size_t sA, int m, int b, T* V, T* V2, size_t sV, int count) {
     if (count <= 0 || m <= 0) return 0;
-    int G = (m + 127) / 128;                       // <= 128 rows per CTA: few, fat CTAs (many matrices share the GPU)
-    if (G > 8) G = 8;
-    int rows = (m + G - 1) / G;
-    G = (m + rows - 1) / rows;
-    const size_t smem = panel_smem_bytes(rows, b, sizeof(T));
-    if (smem > 200 * 1024) return SVDB200_E_CAPACITY;
+    const PanelBatchedShape ps = panel_batched_shape(m, b, sizeof(T));
+    if (ps.smem > kPanelBatchedSmem) return SVDB200_E_CAPACITY;
+    const int G = ps.G, rows = ps.rows;
+    const size_t smem = ps.smem;
     auto kern = panel_factor_kernel<T, kTrans, true>;
     SVDB_CHECK(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     T* S = nullptr;

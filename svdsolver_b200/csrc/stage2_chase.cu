@@ -43,7 +43,7 @@ using namespace s2;
 // kC: the band as a compile-time constant (32 / 64: the sizes the configs use), 0 = any band at run time
 // kPacked: the matrix is held in the packed 3c-diagonal layout (Layout, stage2_common.cuh); single matrix only
 template <typename T, int kMaxThreads, int kMinBlocks, int kC, bool kPacked>
-__global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T* __restrict__ A0, int n, int band, int* __restrict__ prog0,
+__global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T* __restrict__ A0, size_t sA, int n, int band, int* __restrict__ prog0,
                                                                       int count, int G, int complete) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int c = kC > 0 ? kC : band, w = c + 1;
@@ -58,12 +58,12 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks) stage2_chase_kernel(T
     const int tx = tid % c, ty = tid / c, tys = nt / c;   // 2-D view of the CTA: c columns x tys rows (nt >= c)
 
     // Batched use: the grid is split into groups of G CTAs; a group pipelines the sweeps of one matrix at a time
-    // (matrices group, group + #groups, ...).  Progress counters are per matrix and pre-zeroed, so a CTA that runs
+    // (matrices group, group + #groups, ..., sA elements apart).  Progress counters are per matrix and pre-zeroed, so a CTA that runs
     // ahead into its group's next matrix only ever waits on counters of that matrix.  Single matrix: count = 1,
     // G = gridDim.x.
     const int grp = blockIdx.x / G, rank = blockIdx.x - grp * G, ngroups = gridDim.x / G;
     for (int mat = grp; mat < count; mat += ngroups) {
-    T* __restrict__ A = A0 + (size_t)mat * N * N;
+    T* __restrict__ A = A0 + (size_t)mat * sA;
     int* __restrict__ prog = prog0 + (size_t)mat * N;
     long long tick = SVDB_S2_TIMING ? clock64() : 0;
     (void)tick;
@@ -182,10 +182,10 @@ int stage2_debug_read(long long* out16) {
 namespace {
 
 template <typename T, bool kPacked>
-__global__ void extract_bidiagonal_kernel(const T* __restrict__ A, int n, int band, T* __restrict__ d, T* __restrict__ e) {
+__global__ void extract_bidiagonal_kernel(const T* __restrict__ A, size_t sA, int n, int band, T* __restrict__ d, T* __restrict__ e) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     const Layout<kPacked> at = make_layout<kPacked>(n, band);
-    A += (size_t)blockIdx.y * n * n;                 // batched (dense only): one matrix per blockIdx.y, d/e rows of length n
+    A += (size_t)blockIdx.y * sA;                    // batched (dense only): one matrix per blockIdx.y, d/e rows of length n
     if (d) d += (size_t)blockIdx.y * n;
     if (e) e += (size_t)blockIdx.y * n;
     if (i < n) {
@@ -206,9 +206,9 @@ __global__ void pack_band_kernel(const T* __restrict__ ab, int n, int b, T* __re
     }
 }
 
-// Stage 2 of `count` dense matrices (count > 1: back to back, n x n each), or of ONE matrix in the packed layout
+// Stage 2 of `count` dense matrices (count > 1: n x n each, ld = n, sA elements apart), or of ONE matrix in the packed layout
 template <typename T, bool kPacked>
-int stage2_run(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
+int stage2_run(Ctx* c, T* a, size_t sA, size_t n, size_t band, T* d, T* e, int count) {
     if (n < 2 || band < 1 || count < 1) return SVDB200_E_SHAPE;
     if (n > (size_t)INT_MAX / 4) return SVDB200_E_CAPACITY;
     const int cb = (int)band;
@@ -252,12 +252,12 @@ int stage2_run(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
         if (fast != 0 && fast != 1) return fast;
     }
     if (fast != 0) {
-        void* args[] = {&a, &ni, &bi, &prog, &cnt, &gi, &complete};
+        void* args[] = {&a, &sA, &ni, &bi, &prog, &cnt, &gi, &complete};
         SVDB_CHECK(c, cudaLaunchCooperativeKernel((void*)kern, dim3((unsigned)grid), dim3(nt), args, smem, c->stream));
         c->launches++;
     }
     if (d || e) {
-        extract_bidiagonal_kernel<T, kPacked><<<dim3((unsigned)((n + 255) / 256), (unsigned)count), 256, 0, c->stream>>>(a, ni, cb, d, e);
+        extract_bidiagonal_kernel<T, kPacked><<<dim3((unsigned)((n + 255) / 256), (unsigned)count), 256, 0, c->stream>>>(a, sA, ni, cb, d, e);
         SVDB_CHECK(c, cudaGetLastError());
         c->launches++;
     }
@@ -267,7 +267,9 @@ int stage2_run(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) {
 }  // namespace
 
 template <typename T>
-int stage2_chase_batched(Ctx* c, T* a, size_t n, size_t band, T* d, T* e, int count) { return stage2_run<T, false>(c, a, n, band, d, e, count); }
+int stage2_chase_batched(Ctx* c, T* a, size_t sA, size_t n, size_t band, T* d, T* e, int count) {
+    return stage2_run<T, false>(c, a, sA, n, band, d, e, count);
+}
 
 // Stage 2 of a band matrix given in LAPACK upper band storage: packed into the handle's working buffer (max_n x 3 band,
 // allocated on first use) and chased there; `ab` is not modified.
@@ -282,17 +284,17 @@ int stage2_chase_packed(Ctx* c, const T* ab, size_t n, size_t band, T* d, T* e) 
     pack_band_kernel<T><<<blocks, 256, 0, c->stream>>>(ab, (int)n, (int)band, w);
     SVDB_CHECK(c, cudaGetLastError());
     c->launches++;
-    return stage2_run<T, true>(c, w, n, band, d, e, 1);
+    return stage2_run<T, true>(c, w, n * 3 * band, n, band, d, e, 1);
 }
 
 template <typename T>
-int stage2_chase(Ctx* c, T* a, size_t n, size_t band, T* d, T* e) { return stage2_chase_batched<T>(c, a, n, band, d, e, 1); }
+int stage2_chase(Ctx* c, T* a, size_t n, size_t band, T* d, T* e) { return stage2_chase_batched<T>(c, a, n * n, n, band, d, e, 1); }
 
 // d = diag(A), e = diag(A, 1) of a device matrix (what Bidiagonal{A.diag(), A.diag(1)} returns, svd_serial.h:264)
 template <typename T>
 int extract_bidiagonal(Ctx* c, const T* a, size_t n, T* d, T* e) {
     if (!d && !e) return 0;
-    extract_bidiagonal_kernel<T, false><<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(a, (int)n, 1, d, e);
+    extract_bidiagonal_kernel<T, false><<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(a, n * n, (int)n, 1, d, e);
     SVDB_CHECK(c, cudaGetLastError());
     c->launches++;
     return 0;
@@ -300,8 +302,8 @@ int extract_bidiagonal(Ctx* c, const T* a, size_t n, T* d, T* e) {
 template int extract_bidiagonal<float>(Ctx*, const float*, size_t, float*, float*);
 template int extract_bidiagonal<double>(Ctx*, const double*, size_t, double*, double*);
 
-template int stage2_chase_batched<float>(Ctx*, float*, size_t, size_t, float*, float*, int);
-template int stage2_chase_batched<double>(Ctx*, double*, size_t, size_t, double*, double*, int);
+template int stage2_chase_batched<float>(Ctx*, float*, size_t, size_t, size_t, float*, float*, int);
+template int stage2_chase_batched<double>(Ctx*, double*, size_t, size_t, size_t, double*, double*, int);
 template int stage2_chase<float>(Ctx*, float*, size_t, size_t, float*, float*);
 template int stage2_chase<double>(Ctx*, double*, size_t, size_t, double*, double*);
 template int stage2_chase_packed<float>(Ctx*, const float*, size_t, size_t, float*, float*);
